@@ -5,6 +5,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--model res15] [--precision bf16|bf16x3|fp32]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's logits as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of synthetic waveforms per GPU.
   value     whole-job utterances/s with the waveforms already resident in HBM (device-timed, CUDA events, max over
@@ -23,7 +24,7 @@ One "step" = one pass of the hot path over one batch of synthetic waveforms per 
   parity_mode  the same measurements for the other tensor-core precision (bf16x3 when the headline runs bf16): the
             mode that meets the fp32 tolerance, driver-visible next to the headline.
   other_configs  the other BASELINE.json configurations (res8, res26, res15-narrow, cnn-trad-fpool3, res15 in fp32, res15
-            on 9 s clips), five device-resident steps each with their own roofline object, so that one driver run sees them.
+            on 9 s clips), --steps device-resident steps each with their own roofline object, so that one driver run sees them.
   e2e_pcm16 the e2e path fed with int16 PCM host buffers (the wav files' own sample format; bit-identical logits).
   cpu_baseline  the oracle port (oracle/: the reference algorithm in numpy / PyTorch-CPU fp32) timed on this host's
             cores on a bounded sample.
@@ -74,6 +75,20 @@ def committed_traffic(kernel_path, batch, precision):
                 d.get("precision", "bf16") == precision:
             best = d
     return None if best is None else {"dram_bytes_per_launch": best["dram_bytes_per_launch"], "source": best.get("source")}
+
+
+def dump_outputs(path, arrays, limit=64 << 20):
+    """Write each array (name -> tensor) as float32 `path/<name>.npy`, so that two builds can be compared output for output.
+    An array larger than its share of `limit` bytes is cut to a fixed, seeded sample of its rows (the same rows on every
+    run with the same arguments)."""
+    os.makedirs(path, exist_ok=True)
+    share = limit // len(arrays)
+    for name, t in arrays.items():
+        a = torch.as_tensor(t).detach().float().cpu().numpy()
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def peaks():
@@ -168,9 +183,11 @@ def run_reference_arm(args):
     t_fe = t_model = 0.0
     t0 = time.perf_counter()
     for i in range(args.steps):
-        a, b, _ = ref.step(waves[args.warmup + i])
+        a, b, logits = ref.step(waves[args.warmup + i])
         t_fe += a; t_model += b
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": logits})
     value = batch * args.steps / dt
     sample = (f"each step is a bounded sample of the workload: {batch} of its {args.batch} synthetic {N_SAMPLES / 16000:g} s clips "
               f"(the reference's own configured batch size), {args.steps} steps: numpy restatement of compute_mfccs per "
@@ -252,7 +269,12 @@ def main():
                     help="skip the short device-resident runs of the other BASELINE.json configurations (`other_configs`)")
     ap.add_argument("--gpu-eager-bar", action="store_true",
                     help="also time the PyTorch-eager (cuDNN) forward of the reference architecture on this GPU (SURVEY 8d)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logits of the last timed step as DIR/<name>.npy (float32; rank 0): logits (device-"
+                         "resident path), e2e_logits and e2e_pcm16_logits (host-buffer paths); --impl reference: logits")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     global N_SAMPLES
     N_SAMPLES = args.clip_samples
@@ -312,7 +334,8 @@ def main():
 
     def timed_device(per_gpu, steps, warm):
         """`steps` device-resident steps of `per_gpu` utterances per GPU: forward_wave straight into the gather buffer,
-        accuracy counted on the device into the same buffer, one collective.  -> (ms max over ranks, launches)."""
+        accuracy counted on the device into the same buffer, one collective.
+        -> (ms max over ranks, launches, host time window, logits of the last step)."""
         gather = kdist.LogitsGather(per_gpu * world, model.n_labels, dev)
         acc = Acc(counts=gather.counts)
         tg = targets[:per_gpu]
@@ -336,11 +359,12 @@ def main():
         e1.record()
         barrier()
         th1 = time.perf_counter()
-        return max_over_ranks(e0.elapsed_time(e1)), launches, (th0, th1)
+        return max_over_ranks(e0.elapsed_time(e1)), launches, (th0, th1), gather.logits
 
     def timed_e2e(per_gpu, steps, hosts=None):
         """pinned host waveforms -> H2D -> forward_wave -> logits D2H, pipelined; every step's result is complete (event)
-        before its host buffer is handed out again.  `hosts`: other pinned host batches (the int16 PCM form)."""
+        before its host buffer is handed out again.  `hosts`: other pinned host batches (the int16 PCM form).
+        -> (ms max over ranks, host logits of the last step)."""
         host_sets = hosts if hosts is not None else host_f32
         pipe = HostPipeline(model, fe, N_SAMPLES, sub_batch=min(args.e2e_sub_batch, per_gpu), device=dev,
                             slots=args.e2e_slots, dtype=host_sets[0].dtype)
@@ -366,21 +390,24 @@ def main():
         for ev in pending:
             ev.synchronize()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1))
+        return max_over_ranks(e0.elapsed_time(e1)), outs[(steps - 1) & 1]
 
     with torch.no_grad():
         sampler = ClockSampler(local)
         if rank == 0:
             sampler.start()
-        ms, launches, window = timed_device(B, K, W)
+        ms, launches, window, logits = timed_device(B, K, W)
         clocks = sampler.stop(window) if rank == 0 else None
         value = B * world * K / (ms / 1e3)
-        ms_e2e = timed_e2e(B, K)
+        ms_e2e, logits_e2e = timed_e2e(B, K)
         e2e_value = B * world * K / (ms_e2e / 1e3)
         # the same end-to-end path fed with 16-bit PCM samples, the format of the wav files behind the reference's
         # datasets (librosa returns float32(s / 32768) for them): half the host->device bytes, bit-identical logits
         host_pcm = [(h * 32768.0).round().clamp(-32768, 32767).to(torch.int16).pin_memory() for h in host_f32]
-        ms_e2e_pcm = timed_e2e(B, K, hosts=host_pcm)
+        ms_e2e_pcm, logits_e2e_pcm = timed_e2e(B, K, hosts=host_pcm)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"logits": logits, "e2e_logits": logits_e2e,
+                                             "e2e_pcm16_logits": logits_e2e_pcm})
         # (the clips are 16-bit PCM already, see pcm_round: the two paths must agree bit for bit)
         n_chk = min(B, 1024)
         pcm_same = bool(torch.equal(model.forward_wave(host_pcm[0][:n_chk].to(dev), fe),
@@ -390,8 +417,8 @@ def main():
         strong = None
         if world > 1 and args.scaling == "weak":
             per = -(-B_cfg // world)
-            ms_s, _, _ = timed_device(per, K, W)
-            ms_s_e2e = timed_e2e(per, K)
+            ms_s = timed_device(per, K, W)[0]
+            ms_s_e2e = timed_e2e(per, K)[0]
             strong = {"total_batch": per * world, "batch_per_gpu": per, "value": per * world * K / (ms_s / 1e3),
                       "ms_per_step": ms_s / K, "e2e_value": per * world * K / (ms_s_e2e / 1e3), "unit": UNIT,
                       "note": "the 8192-utterance batch of the headline configuration split over the ranks "
@@ -423,8 +450,8 @@ def main():
             if other is not None and world == 1 and not args.no_second_mode:
                 model.precision = other
                 try:
-                    ms2, _, _ = timed_device(B, K, W)
-                    ms2_e2e = timed_e2e(B, K)
+                    ms2 = timed_device(B, K, W)[0]
+                    ms2_e2e = timed_e2e(B, K)[0]
                     prof2 = honk2_b200.profile_layers(model, fe, [d[:B] for d in dev_sets], K)
                     second = {"precision": other, "value": B * K / (ms2 / 1e3), "unit": UNIT, "ms_per_step": ms2 / K,
                               "e2e": {"value": B * K / (ms2_e2e / 1e3), "unit": UNIT, "ms_per_step": ms2_e2e / K},
@@ -475,17 +502,16 @@ def main():
                         mo.forward_wave(ws[i & 1], fe, out=out)
                     torch.cuda.synchronize()
                     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    ko = 5
                     e0.record()
-                    for i in range(ko):
+                    for i in range(K):
                         mo.forward_wave(ws[i & 1], fe, out=out)
                     e1.record()
                     torch.cuda.synchronize()
                     ms_o = e0.elapsed_time(e1)
-                    pr = honk2_b200.profile_layers(mo, fe, ws, ko)
-                    rf = roofline_for(pr, prec, pk, nb, ko)
+                    pr = honk2_b200.profile_layers(mo, fe, ws, K)
+                    rf = roofline_for(pr, prec, pk, nb, K)
                     others.append({"model": name, "precision": prec, "batch": nb, "clip_samples": ns, "baseline_config": tag,
-                                   "value": nb * ko / (ms_o / 1e3), "unit": UNIT, "ms_per_step": ms_o / ko, "steps": ko,
+                                   "value": nb * K / (ms_o / 1e3), "unit": UNIT, "ms_per_step": ms_o / K, "steps": K,
                                    "roofline": None if rf is None else {k: rf[k] for k in (
                                        "bound", "achieved", "peak", "unit", "frac", "frac_of_burst_peak", "kernel",
                                        "avg_launch_ms", "share_of_step", "frontend_ms_per_step")}})
@@ -525,7 +551,7 @@ def main():
             stream = torch.from_numpy(synth.broadband(1, N=B * 160 + N_SAMPLES, seed=77)[0]).to(dev)
             feats_s = torch.empty((B, fe.n_frames(N_SAMPLES), fe.n_mels), dtype=torch.float32, device=dev)
 
-            def timed(fn, reps=5):
+            def timed(fn, reps=K):
                 for _ in range(2):
                     fn()
                 a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
