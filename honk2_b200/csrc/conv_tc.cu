@@ -1,33 +1,18 @@
-// bf16 tensor-core ResNet path for sm_100a: tcgen05.mma (UMMA) implicit-GEMM 3x3 dilated
-// convolution with TMA-staged halo tiles, TMEM accumulators and a fused
-// ReLU / residual / BatchNorm epilogue (/root/reference/model/resnet.py:48-55), plus the
-// conv_0 and mean+linear kernels for the same activation layout.
+// bf16 tensor-core ResNet path for sm_100a (tcgen05.mma, TMEM accumulators, TMA / bulk copies): the host-side plans
+// and dispatch of the two whole-network kernels, the weight-packing kernels, and the conv_0 pre-pass of the packed
+// strips.
 //
-// Activation layout ("planar-8"): [B][NP][H][W][8] bf16, NP = CP/8 planes of 8 channels,
-// CP = channels padded to a multiple of 16 (45 -> 48).  One plane row is W*16 contiguous bytes,
-// so a TMA box {8 ch, Wp, rows} lands in shared memory as a dense array of 16-byte "positions":
-// exactly the UMMA K-major SWIZZLE_NONE canonical layout (core matrix = 8 positions x 16 B,
-// SBO = 128 B), in which a pixel shift is nothing but a start-address offset.
+//   resnet_tc_sweep_kernel  (resnet_sweep.cuh)   column sweep: the 128 MMA lanes are 128 rows of one map column
+//   resnet_tc_fused_kernel  (resnet_fused.cuh)   position major: halo tiles of a planar-8 map
 //
-// Implicit GEMM per tap (dh, dw) and 16-channel chunk kc:
-//   D[128 positions x CP] += A[128 positions x 16] (shifted view of the staged tile)
-//                          * B[16 x CP]            (weights, resident in shared memory)
-// Positions are flat indices p = r * Wp + c into the zero-padded tile rows (Wp = W + d: the d
-// left-pad columns of row r+1 double as the right padding of row r; TMA out-of-bounds fill
-// supplies every zero).  Outputs at pad positions are computed and discarded.
-//
-// Warp roles (192 threads, 1 CTA per SM, persistent over tiles):
-//   warp 0     TMA producer: one stage = one 16-channel chunk of the haloed input tile
-//   warp 1     MMA issuer (one elected lane) + TMEM allocation
-//   warps 2-5  epilogue: tcgen05.ld -> ReLU -> +skip -> BN -> bf16 planar-8 stores
-// TMEM holds two accumulator buffers (up to 5 M-tiles x CP columns each) so the epilogue of
-// tile i overlaps the MMAs of tile i+1.
+// Each runs conv_0 -> every C->C layer -> global mean -> Linear for a whole batch in one launch, in plain bf16 and in
+// the split-bf16 ("bf16x3") mode.  Both precisions pick the kernel by one rule: the sweep plan if it can stage the
+// map, else the position-major plan, else KWS_ERR_UNSUPPORTED.
 #include "tc.cuh"
 #include "ptx.cuh"
 #include <cuda.h>
 #include <cstdlib>
 #include <cstring>
-#include <map>
 #include <tuple>
 #include <vector>
 
@@ -40,7 +25,6 @@ __host__ __device__ constexpr int tc_epi_warps(int NKC) { return 4 * NKC; }
 __host__ __device__ constexpr int tc_threads(int NKC) { return 32 * (1 + kTcIssuers + tc_epi_warps(NKC)); }
 constexpr int kTcMaxMt = 8;       // upper bound of M-tiles per tile (min(8, kAccCols / CP) at run time)
 constexpr int kAccCols = 256;     // TMEM columns per accumulator buffer
-constexpr int kTcMaxLanes = 4;
 constexpr int kMaxStages = 8;
 // ---------------------------------------------------------------------------------------------
 struct TcGeom {
@@ -54,490 +38,10 @@ struct TcGeom {
   int smem_w_off, smem_ring_off, smem_total;
 };
 
-struct TcConvParams {
-  const __nv_bfloat16* wpack;  // [9][NKC][2][CP][8]; input-channel axis pre-multiplied by the previous layer's BN scale
-  const float* kconst;         // [CP] per-channel epilogue constant: (mean of the skip layer, even layers) - mean of this layer
-  const __nv_bfloat16* skip;   // even layers: centred activation z of layer i-2 (conv_0 output for i = 2); may alias y
-  __nv_bfloat16* y;            // centred activation z = x - mean (the 1/sigma factor lives in the next layer's weights)
-  float* pool_sum;             // [B][CP] per-utterance sums of z over H*W (last layer), or nullptr
-  int B, total_tiles;
-  TcGeom g;
-};
-
-// HAS_PREV: even layer (adds and rewrites the skip tensor).  DO_POOL: last layer (accumulates the
-// global mean instead of storing the activation).
-template <int NKC, bool HAS_PREV, bool DO_POOL>
-__global__ void __launch_bounds__(tc_threads(NKC), 1)
-conv3x3_tc_kernel(const __grid_constant__ CUtensorMap tmap, const TcConvParams p) {
-  constexpr int CP = 16 * NKC;       // padded channels = UMMA N
-  constexpr int NP = 2 * NKC;        // 8-channel planes
-  constexpr int W_HALF = CP * 16;    // bytes of one [CP][8] weight half-slab
-  constexpr int W_BYTES = 9 * NKC * 2 * W_HALF;
-  constexpr int MAXMT = (kAccCols / CP) < kTcMaxMt ? (kAccCols / CP) : kTcMaxMt;
-  constexpr int MAXU = (MAXMT + kTcIssuers - 1) / kTcIssuers;   // M-tiles per issuer warp
-  extern __shared__ __align__(1024) unsigned char smem[];
-  const TcGeom& g = p.g;
-
-  // ---- shared memory carve-up
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem);   // full[8], empty[8], tfull[2], tempty[2], wfull
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 8 * 24);
-  float* s_kconst = reinterpret_cast<float*>(smem + 256);         // [CP]
-  unsigned char* s_w = smem + g.smem_w_off;
-  unsigned char* s_ring = smem + g.smem_ring_off;
-  const uint32_t bar0 = smem_u32(bars);
-  auto full_bar = [&](int s) { return bar0 + 8u * s; };
-  auto empty_bar = [&](int s) { return bar0 + 8u * (kMaxStages + s); };
-  auto tfull_bar = [&](int a) { return bar0 + 8u * (2 * kMaxStages + a); };
-  auto tempty_bar = [&](int a) { return bar0 + 8u * (2 * kMaxStages + 2 + a); };
-  const uint32_t wfull_bar = bar0 + 8u * (2 * kMaxStages + 4);
-
-  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);   // warp-uniform for the compiler
-  const int lane = threadIdx.x & 31;
-
-  // ---- one-time setup
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < g.n_stages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), kTcIssuers); }
-    for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), kTcIssuers); mbar_init(tempty_bar(a), tc_epi_warps(NKC)); }
-    mbar_init(wfull_bar, 1);
-    fence_barrier_init();
-    tma_prefetch_desc(&tmap);
-    // weights: one asynchronous bulk copy global -> shared, completion on wfull_bar
-    mbar_expect_tx(wfull_bar, W_BYTES);
-    bulk_load(smem_u32(s_w), p.wpack, W_BYTES, wfull_bar);
-  }
-  if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 512);
-  for (int i = threadIdx.x; i < CP; i += tc_threads(NKC)) s_kconst[i] = p.kconst[i];
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  // Programmatic dependent launch: everything above (barriers, TMEM, weights) overlapped the tail of the
-  // previous layer's kernel; the activations it wrote are only touched after this wait.  The next
-  // layer's kernel may be scheduled as soon as SMs free up.
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-
-  const int tiles_per_utt = g.tiles_per_utt;
-  // Each CTA takes a contiguous range of tiles: consecutive tiles of one utterance stay on one SM (L2/TLB
-  // locality, and the fused pooling flushes once per utterance instead of once per tile).
-  const int t_begin = (int)(((int64_t)blockIdx.x * p.total_tiles) / gridDim.x);
-  const int t_end = (int)(((int64_t)(blockIdx.x + 1) * p.total_tiles) / gridDim.x);
-  // tile index inside an utterance -> (phase p, first row r0 in phase-row units, number of rows).
-  // Row r of the tile is image row (r0 + r) * hstep + p, hstep = d in phase mode and 1 otherwise.
-  auto tile_decode = [&](int tix, int& ph, int& r0, int& rows) {
-    if (g.phase) {
-      ph = tix / g.chunks_per_phase;
-      r0 = (tix - ph * g.chunks_per_phase) * g.R;
-      rows = min(g.R, (g.H - ph + g.d - 1) / g.d - r0);
-    } else {
-      ph = 0;
-      r0 = tix * g.R;
-      rows = min(g.R, g.H - r0);
-    }
-  };
-
-  if (warp == 0) {
-    // ================================ TMA producer ================================
-    if (elect_one()) {
-      int stage = 0;
-      uint32_t phase = 0;
-      const uint32_t tx = (uint32_t)(2 * g.n_boxes * g.rows_box * g.Wp * 16);
-      for (int t = t_begin; t < t_end; ++t) {
-        const int b = t / tiles_per_utt, tix = t - b * tiles_per_utt;
-        int ph, r0, rows;
-        tile_decode(tix, ph, r0, rows);
-        if (rows <= 0) continue;
-        for (int kc = 0; kc < NKC; ++kc) {
-          mbar_wait(empty_bar(stage), phase ^ 1);
-          mbar_expect_tx(full_bar(stage), tx);
-          const uint32_t sbase = smem_u32(s_ring + (size_t)stage * g.stage_bytes);
-          for (int half = 0; half < 2; ++half)
-            for (int bx = 0; bx < g.n_boxes; ++bx)
-              tma_load_5d(sbase + half * g.slab_bytes + bx * g.box_stride, &tmap, full_bar(stage), 0, -g.dpad,
-                          r0 + g.h_start[bx], ph, b * NP + 2 * kc + half);
-          if (++stage == g.n_stages) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp <= kTcIssuers) {
-    // ================================ MMA issuers (3 warps) ================================
-    // A 128 x CP x 16 MMA lasts ~CP/2 tensor-pipe cycles, less than one thread needs to set up and
-    // issue it, so the M-tiles of a tile are dealt round-robin to kTcIssuers warps (disjoint TMEM
-    // accumulators, hence no ordering between them); every issuer commits to the same barriers.
-    // All operands are warp-uniform.  A descriptor = {lo: addr>>4 | (LBO>>4)<<16, hi: SBO>>4 | version};
-    // per MMA only the 14-bit address field of `lo` changes, by a precomputed 16-byte-unit offset.
-    const int me = warp - 1;
-    int stage = 0, acc = 0;
-    uint32_t phase = 0, acc_phase = 0;
-    constexpr uint32_t idesc = umma_idesc(128, CP);
-    constexpr uint32_t desc_hi = (128u >> 4) | (1u << 14);
-    const uint32_t a_lo_fields = ((uint32_t)(g.slab_bytes >> 4) & 0x3FFFu) << 16;
-    const uint32_t b_lo_base = ((smem_u32(s_w) >> 4) & 0x3FFFu) | (((uint32_t)(W_HALF >> 4) & 0x3FFFu) << 16);
-    int tap16[9];   // start offset of tap (dh,dw) inside a stage, in 16-byte units (may be negative)
-#pragma unroll
-    for (int dh = 0; dh < 3; ++dh)
-#pragma unroll
-      for (int dw = 0; dw < 3; ++dw) tap16[dh * 3 + dw] = (g.tap_off[dh] >> 4) + (dw - 1) * g.d;
-    const bool side = g.side_taps != 0;
-    const int first_tap = side ? 0 : 1;
-    const bool leader = elect_one();
-    mbar_wait(wfull_bar, 0);   // weights have landed
-    for (int t = t_begin; t < t_end; ++t) {
-      int ph, r0, rows;
-      tile_decode(t % tiles_per_utt, ph, r0, rows);
-      if (rows <= 0) continue;
-      const int n_mt = (rows * g.Wp + 127) >> 7;
-      mbar_wait(tempty_bar(acc), acc_phase ^ 1);
-      tc_fence_after();
-      const uint32_t d_base = tmem_base + acc * kAccCols + me * CP;
-#pragma unroll
-      for (int kc = 0; kc < NKC; ++kc) {
-        mbar_wait(full_bar(stage), phase);
-        tc_fence_after();
-        if (leader) {
-          const uint32_t a_lo_stage =
-              (((smem_u32(s_ring + (size_t)stage * g.stage_bytes) >> 4) + me * 128) & 0x3FFFu) | a_lo_fields;
-#pragma unroll
-          for (int tap = 0; tap < 9; ++tap) {
-            if ((tap % 3) != 1 && !side) continue;
-            const uint32_t a_lo = a_lo_stage + (uint32_t)tap16[tap];
-            const uint32_t b_lo = b_lo_base + (uint32_t)(((tap * NKC + kc) * 2 * W_HALF) >> 4);
-            if (kc == 0 && tap <= 1) {
-              // the first tap of a tile overwrites the accumulators (tap 0, or tap 1 when d >= W)
-              const uint32_t accum = (tap == first_tap) ? 0u : 1u;
-#pragma unroll
-              for (int u = 0; u < MAXU; ++u)
-                if (me + u * kTcIssuers < n_mt)
-                  umma_f16_lohi_rt(d_base + u * kTcIssuers * CP, a_lo + u * kTcIssuers * 128, b_lo, desc_hi, idesc, accum);
-            } else {
-#pragma unroll
-              for (int u = 0; u < MAXU; ++u)
-                if (me + u * kTcIssuers < n_mt)
-                  umma_f16_lohi<true>(d_base + u * kTcIssuers * CP, a_lo + u * kTcIssuers * 128, b_lo, desc_hi, idesc);
-            }
-          }
-          umma_commit(empty_bar(stage));                       // stage reusable once these MMAs retire
-          if (kc == NKC - 1) umma_commit(tfull_bar(acc));      // accumulators complete
-        }
-        __syncwarp();
-        if (++stage == g.n_stages) { stage = 0; phase ^= 1; }
-      }
-      acc ^= 1;
-      if (acc == 0) acc_phase ^= 1;
-    }
-  } else {
-    // ================================ epilogue (4*NKC warps) ================================
-    // Warp e reads TMEM lane quarter q = warp % 4 (fixed by hardware) and the 16 accumulator columns of
-    // channel group j = e / 4, for every M-tile of the tile: z = ReLU(acc) (+ skip) + kconst, two 16-byte
-    // planar-8 stores per position.  The 16 per-channel constants live in registers.
-    const int q = warp & 3;
-    const int j = (warp - (1 + kTcIssuers)) >> 2;
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    const int64_t plane_stride = (int64_t)g.Hpad * g.W;   // in 16-byte (8-channel) units
-    const int hstep = g.phase ? g.d : 1;
-    const uint4* skip_in = reinterpret_cast<const uint4*>(p.skip) + (int64_t)(2 * j) * plane_stride;
-    uint4* y_out = reinterpret_cast<uint4*>(p.y) + (int64_t)(2 * j) * plane_stride;
-    float kc_reg[16];
-#pragma unroll
-    for (int c = 0; c < 16; ++c) kc_reg[c] = s_kconst[16 * j + c];
-    float psum[DO_POOL ? 16 : 1];   // this thread's share of sum_{h,w} z of the current utterance (resnet.py:57-58)
-    int pool_b = -1;
-    auto pool_flush = [&]() {
-      if constexpr (DO_POOL) {
-        if (pool_b >= 0) {   // warp-reduce the 32 positions, one atomic per channel
-#pragma unroll
-          for (int c = 0; c < 16; ++c) {
-            float sum = psum[c];
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-            if (lane == c) atomicAdd(p.pool_sum + (int64_t)pool_b * CP + 16 * j + c, sum);
-          }
-        }
-#pragma unroll
-        for (int c = 0; c < 16; ++c) psum[c] = 0.f;
-      }
-    };
-    pool_flush();
-    for (int t = t_begin; t < t_end; ++t) {
-      const int b = t / tiles_per_utt, tix = t - b * tiles_per_utt;
-      if (DO_POOL && b != pool_b) { pool_flush(); pool_b = b; }
-      int ph, r0, rows;
-      tile_decode(tix, ph, r0, rows);
-      if (rows <= 0) continue;
-      const int n_mt = (rows * g.Wp + 127) >> 7;
-      const int64_t utt_base = ((int64_t)b * NP) * plane_stride + (int64_t)(r0 * hstep + ph) * g.W;
-      // position of this thread in M-tile `mt`: valid flag and offset (16-byte units) inside a plane
-      auto locate = [&](int mt, bool& valid) -> int64_t {
-        const int pos = mt * 128 + q * 32 + lane;
-        const int r = pos / g.Wp;
-        const int w = pos - r * g.Wp - g.dpad;
-        valid = (w >= 0) && (r < rows) && (mt < n_mt);
-        return utt_base + (int64_t)(r * hstep) * g.W + w;
-      };
-      // The skip tensor is fetched one M-tile ahead; the first fetch is issued BEFORE waiting for
-      // the accumulators, so its latency hides behind the MMAs of this tile.
-      uint4 pv_next[2];
-      if constexpr (HAS_PREV) {
-        bool v0;
-        const int64_t b0 = locate(0, v0);
-        if (v0) { pv_next[0] = skip_in[b0]; pv_next[1] = skip_in[b0 + plane_stride]; }
-      }
-      mbar_wait(tfull_bar(acc), acc_phase);
-      tc_fence_after();
-      for (int mt = 0; mt < n_mt; ++mt) {
-        bool valid;
-        const int64_t base = locate(mt, valid);
-        uint4 pv[2];
-        if constexpr (HAS_PREV) {
-          pv[0] = pv_next[0]; pv[1] = pv_next[1];
-          bool v2;
-          const int64_t b2 = locate(mt + 1, v2);
-          if (v2) { pv_next[0] = skip_in[b2]; pv_next[1] = skip_in[b2 + plane_stride]; }
-        }
-        uint32_t v[16];
-        tmem_ld16(tmem_base + ((uint32_t)(q * 32) << 16) + acc * kAccCols + mt * CP + 16 * j, v);
-        tmem_ld_wait();
-        if (valid) {
-#pragma unroll
-          for (int hf = 0; hf < 2; ++hf) {
-            float x[8];
-#pragma unroll
-            for (int e = 0; e < 8; ++e) x[e] = fmaxf(__uint_as_float(v[8 * hf + e]), 0.f) + kc_reg[8 * hf + e];
-            if constexpr (HAS_PREV) {
-              const __nv_bfloat162* pb = reinterpret_cast<const __nv_bfloat162*>(&pv[hf]);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                const float2 f = __bfloat1622float2(pb[e]);
-                x[2 * e] += f.x;
-                x[2 * e + 1] += f.y;
-              }
-            }
-            if constexpr (DO_POOL) {
-#pragma unroll
-              for (int e = 0; e < 8; ++e) psum[8 * hf + e] += x[e];
-            } else {
-              uint4 yo;
-              __nv_bfloat162* yb = reinterpret_cast<__nv_bfloat162*>(&yo);
-#pragma unroll
-              for (int e = 0; e < 4; ++e) yb[e] = __floats2bfloat162_rn(x[2 * e], x[2 * e + 1]);
-              y_out[base + hf * plane_stride] = yo;
-            }
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(acc));
-      acc ^= 1;
-      if (acc == 0) acc_phase ^= 1;
-    }
-    pool_flush();
-  }
-
-  // ---- teardown
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
 }  // namespace kws
 #include "resnet_fused.cuh"
 #include "resnet_sweep.cuh"
 namespace kws {
-
-// ---------------------------------------------------------------------------------------------
-// conv_0 (1 -> C, 3x3, pad 1) + ReLU + AvgPool -> planar-8 bf16 (resnet.py:40-44).
-// One thread per output pixel; channels in groups of 8 -> one 16-byte store per plane.
-__global__ void __launch_bounds__(256)
-conv0_p8_kernel(const float* __restrict__ feat, const float* __restrict__ w0, __nv_bfloat16* __restrict__ out,
-                float* __restrict__ pool_sum, int T, int F, int C, int NP, int ph, int pw, int Ho, int Wo,
-                int rows_per_tile, int Hpad) {
-  if (pool_sum != nullptr && blockIdx.x == 0 && threadIdx.x < NP * 8)
-    pool_sum[(int64_t)blockIdx.y * NP * 8 + threadIdx.x] = 0.f;
-  extern __shared__ __align__(16) float smem_f[];
-  const int in_rows = rows_per_tile * ph + 2, in_cols = F + 2;
-  float* s_in = smem_f;
-  float* s_w = smem_f + round_up(in_rows * in_cols, 4);   // [NP*8][12], zero for pad channels
-  const int64_t b = blockIdx.y;
-  const int ho0 = blockIdx.x * rows_per_tile;
-  const float* src = feat + b * (int64_t)T * F;
-  for (int i = threadIdx.x; i < in_rows * in_cols; i += blockDim.x) {
-    const int r = i / in_cols, c = i - r * in_cols;
-    const int h = ho0 * ph - 1 + r, w = c - 1;
-    s_in[i] = (h >= 0 && h < T && w >= 0 && w < F) ? __ldg(src + (int64_t)h * F + w) : 0.f;
-  }
-  for (int i = threadIdx.x; i < NP * 8 * 12; i += blockDim.x) {
-    const int c = i / 12, k = i - c * 12;
-    s_w[i] = (k < 9 && c < C) ? __ldg(w0 + c * 9 + k) : 0.f;
-  }
-  __syncthreads();
-  const int r = threadIdx.x / Wo, wo = threadIdx.x - r * Wo;
-  const int ho = ho0 + r;
-  if (r >= rows_per_tile || ho >= Ho) return;
-  const float inv = 1.f / (float)(ph * pw);
-  const int64_t plane_stride = (int64_t)Hpad * Wo;
-  uint4* dst = reinterpret_cast<uint4*>(out) + (b * NP) * plane_stride + (int64_t)ho * Wo + wo;
-  for (int pl = 0; pl < NP; ++pl) {
-    float acc[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) acc[e] = 0.f;
-    for (int i = 0; i < ph; ++i)
-      for (int j = 0; j < pw; ++j) {
-        const float* q = s_in + (r * ph + i) * in_cols + wo * pw + j;
-        float xin[9];
-#pragma unroll
-        for (int a = 0; a < 3; ++a)
-#pragma unroll
-          for (int e = 0; e < 3; ++e) xin[a * 3 + e] = q[a * in_cols + e];
-#pragma unroll
-        for (int e = 0; e < 8; ++e) {
-          const float* wc = s_w + (pl * 8 + e) * 12;
-          const float4 wa = *reinterpret_cast<const float4*>(wc);
-          const float4 wb = *reinterpret_cast<const float4*>(wc + 4);
-          float v = xin[0] * wa.x;
-          v = fmaf(xin[1], wa.y, v); v = fmaf(xin[2], wa.z, v); v = fmaf(xin[3], wa.w, v);
-          v = fmaf(xin[4], wb.x, v); v = fmaf(xin[5], wb.y, v); v = fmaf(xin[6], wb.z, v);
-          v = fmaf(xin[7], wb.w, v); v = fmaf(xin[8], wc[8], v);
-          acc[e] += fmaxf(v, 0.f);
-        }
-      }
-    uint4 o;
-    __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&o);
-#pragma unroll
-    for (int e = 0; e < 4; ++e) ob[e] = __floats2bfloat162_rn(acc[2 * e] * inv, acc[2 * e + 1] * inv);
-    dst[pl * plane_stride] = o;
-  }
-}
-
-// conv_0 without pooling (res15): each thread computes 4 consecutive pixels x all channels, so
-// every weight read from shared memory feeds 4 FMAs; stores are 64 contiguous bytes per plane.
-constexpr int kC0Px = 4;
-__global__ void __launch_bounds__(256)
-conv0_p8_w4_kernel(const float* __restrict__ feat, const float* __restrict__ w0, __nv_bfloat16* __restrict__ out,
-                   float* __restrict__ pool_sum, int T, int F, int C, int NP, int groups_per_row,
-                   int rows_per_tile, int Hpad) {
-  extern __shared__ __align__(16) float smem_f[];
-  const int in_rows = rows_per_tile + 2, in_cols = groups_per_row * kC0Px + 2;
-  float* s_in = smem_f;
-  float* s_w = smem_f + round_up(in_rows * in_cols, 4);   // [NP*8][12]
-  const int64_t b = blockIdx.y;
-  const int h0 = blockIdx.x * rows_per_tile;
-  if (pool_sum != nullptr && blockIdx.x == 0 && threadIdx.x < NP * 8) pool_sum[b * NP * 8 + threadIdx.x] = 0.f;
-  const float* src = feat + b * (int64_t)T * F;
-  for (int i = threadIdx.x; i < in_rows * in_cols; i += blockDim.x) {
-    const int r = i / in_cols, c = i - r * in_cols;
-    const int h = h0 - 1 + r, w = c - 1;
-    s_in[i] = (h >= 0 && h < T && w >= 0 && w < F) ? __ldg(src + (int64_t)h * F + w) : 0.f;
-  }
-  for (int i = threadIdx.x; i < NP * 8 * 12; i += blockDim.x) {
-    const int c = i / 12, k = i - c * 12;
-    s_w[i] = (k < 9 && c < C) ? __ldg(w0 + c * 9 + k) : 0.f;
-  }
-  __syncthreads();
-  const int r = threadIdx.x / groups_per_row, gx = threadIdx.x - r * groups_per_row;
-  const int h = h0 + r;
-  if (r >= rows_per_tile || h >= T) return;
-  const int w0px = gx * kC0Px;
-  float pch[3][kC0Px + 2];
-#pragma unroll
-  for (int a = 0; a < 3; ++a)
-#pragma unroll
-    for (int e = 0; e < kC0Px + 2; ++e) pch[a][e] = s_in[(r + a) * in_cols + w0px + e];
-  const int64_t plane_stride = (int64_t)Hpad * F;
-  uint4* dst = reinterpret_cast<uint4*>(out) + (b * NP) * plane_stride + (int64_t)h * F + w0px;
-  for (int pl = 0; pl < NP; ++pl) {
-    float acc[kC0Px][8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const float* wc = s_w + (pl * 8 + e) * 12;
-      const float4 wa = *reinterpret_cast<const float4*>(wc);
-      const float4 wb = *reinterpret_cast<const float4*>(wc + 4);
-      const float w8 = wc[8];
-#pragma unroll
-      for (int px = 0; px < kC0Px; ++px) {
-        float v = pch[0][px] * wa.x;
-        v = fmaf(pch[0][px + 1], wa.y, v); v = fmaf(pch[0][px + 2], wa.z, v);
-        v = fmaf(pch[1][px], wa.w, v); v = fmaf(pch[1][px + 1], wb.x, v); v = fmaf(pch[1][px + 2], wb.y, v);
-        v = fmaf(pch[2][px], wb.z, v); v = fmaf(pch[2][px + 1], wb.w, v); v = fmaf(pch[2][px + 2], w8, v);
-        acc[px][e] = fmaxf(v, 0.f);
-      }
-    }
-#pragma unroll
-    for (int px = 0; px < kC0Px; ++px) {
-      if (w0px + px < F) {
-        uint4 o;
-        __nv_bfloat162* ob = reinterpret_cast<__nv_bfloat162*>(&o);
-#pragma unroll
-        for (int e = 0; e < 4; ++e) ob[e] = __floats2bfloat162_rn(acc[px][2 * e], acc[px][2 * e + 1]);
-        dst[pl * plane_stride + px] = o;
-      }
-    }
-  }
-}
-
-// Linear on the pooled sums produced by the last convolution's epilogue (resnet.py:57-59).
-__global__ void __launch_bounds__(256)
-tail_pool_kernel(const float* __restrict__ pool_sum, const float* __restrict__ scale, const float* __restrict__ out_w,
-                 const float* __restrict__ out_b, float* __restrict__ logits, int64_t B, int C, int CP, int HW,
-                 int n_labels) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= B * n_labels) return;
-  const int64_t b = i / n_labels;
-  const int l = (int)(i - b * n_labels);
-  const float inv = 1.f / (float)HW;
-  float v = __ldg(out_b + l);
-  // pool_sum holds sums of z = x - mean; BatchNorm output mean = z_mean / sigma (resnet.py:55-58)
-  for (int c = 0; c < C; ++c) v = fmaf(pool_sum[b * CP + c] * inv * __ldg(scale + c), __ldg(out_w + l * C + c), v);
-  logits[i] = v;
-}
-
-// mean over H*W of planar-8 bf16 + Linear (resnet.py:57-59).  One CTA per utterance.
-__global__ void __launch_bounds__(256)
-tail_p8_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ out_w, const float* __restrict__ out_b,
-               float* __restrict__ logits, int C, int NP, int HW, int n_labels) {
-  __shared__ float s_part[8][64];
-  __shared__ float s_mean[64];
-  const int64_t b = blockIdx.x;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int pl = 0; pl < NP; ++pl) {
-    const uint4* src = reinterpret_cast<const uint4*>(y) + (b * NP + pl) * (int64_t)HW;
-    float s[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) s[e] = 0.f;
-    for (int i = threadIdx.x; i < HW; i += 256) {
-      const uint4 v = __ldg(src + i);
-      const __nv_bfloat162* vb = reinterpret_cast<const __nv_bfloat162*>(&v);
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const float2 f = __bfloat1622float2(vb[e]);
-        s[2 * e] += f.x;
-        s[2 * e + 1] += f.y;
-      }
-    }
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) s[e] += __shfl_xor_sync(0xffffffffu, s[e], o);
-      if (lane == 0) s_part[warp][pl * 8 + e] = s[e];
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x < NP * 8) {
-    float t = 0.f;
-    for (int wv = 0; wv < 8; ++wv) t += s_part[wv][threadIdx.x];
-    s_mean[threadIdx.x] = t / (float)HW;
-  }
-  __syncthreads();
-  for (int l = threadIdx.x; l < n_labels; l += 256) {
-    float v = __ldg(out_b + l);
-    for (int c = 0; c < C; ++c) v = fmaf(s_mean[c], __ldg(out_w + l * C + c), v);
-    logits[b * n_labels + l] = v;
-  }
-}
 
 // torch [C][C][3][3] fp32 -> [9][NKC][2][CP][8] bf16 (tap, 16-ch chunk, K half, cout, 8 cin)
 // `in_scale` (nullable): BN scale 1/sigma of the PREVIOUS layer, folded into the input-channel axis
@@ -666,10 +170,8 @@ struct TcResNet {
   __nv_bfloat16* conv0_wb3 = nullptr;       // same for the split-bf16 mode
   float* out_w = nullptr;
   float* out_b = nullptr;
-  std::map<std::tuple<const void*, int64_t, int, int, int>, CUtensorMap> maps;
   // whole-network persistent kernel (resnet_fused.cuh): device copies of the layer table and tensor maps,
   // rebuilt when the input shape or the workspace changes
-  bool fused_enabled = true;
   void* fused_dev = nullptr;   // [TcLayerDesc x n_layers][pad][CUtensorMap x n_layers]
   std::tuple<int, int, const void*, int> fused_key{-1, -1, nullptr, 0};
   TcFusedParams fused_prm{};
@@ -680,11 +182,6 @@ struct TcResNet {
   int l2_policy = 1, wait_polls = 48, sweep_max_stages = 0, sweep_min_pct = 60;
   bool sweep_discard = true;
   bool sweep_pack = true;      // HONK2_TC_SWEEP_PACK=0: short / pooled maps stay on the position-major kernel
-  // chunk pipelining: consecutive chunks run on `lanes` internal streams so that the prologue / tail of one
-  // chunk's layer kernels overlaps the steady state of another's (each lane has its own activation buffers)
-  int lanes = 1;
-  cudaStream_t lane_stream[kTcMaxLanes] = {};
-  cudaEvent_t ev_start = nullptr, ev_done[kTcMaxLanes] = {};
 };
 
 static int tc_max_mt(int CP) {
@@ -709,7 +206,7 @@ static int tc_hpad(const kws_resnet_config& c, int H) {
   return round_up(H, m);
 }
 
-// Tile geometry of one layer launch.  Returns false if the layer cannot be tiled.
+// Tile geometry of one layer of the position-major kernel.  Returns false if the layer cannot be tiled.
 static bool tc_geom(int NKC, int H, int Hpad, int W, int d, TcGeom* g) {
   const int CP = 16 * NKC;
   g->H = H; g->W = W; g->d = d; g->Hpad = Hpad;
@@ -831,7 +328,6 @@ int tc_resnet_create(const kws_resnet_config& cfg, TcResNet** out) {
     p->out_b = reinterpret_cast<float*>(b);
     // every knob is read HERE, once per model handle (DESIGN.md section 4 lists them)
     auto env_int = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
-    p->fused_enabled = env_int("HONK2_TC_FUSED", 1) != 0;
     p->sweep_enabled = env_int("HONK2_TC_SWEEP", 1) != 0;
     p->sweep_k32 = env_int("HONK2_TC_SWEEP_K32", 1) != 0;
     p->sweep_discard = env_int("HONK2_TC_SWEEP_DISCARD", 1) != 0;
@@ -840,16 +336,6 @@ int tc_resnet_create(const kws_resnet_config& cfg, TcResNet** out) {
     p->sweep_min_pct = env_int("HONK2_TC_SWEEP_MINPCT", 60);
     p->l2_policy = env_int("HONK2_TC_L2POLICY", 1);
     p->wait_polls = env_int("HONK2_TC_WAIT_POLLS", 48);
-    p->lanes = std::max(1, std::min(kTcMaxLanes, env_int("HONK2_TC_LANES", 2)));
-    bool ok = cudaEventCreateWithFlags(&p->ev_start, cudaEventDisableTiming) == cudaSuccess;
-    for (int l = 0; l < p->lanes && ok; ++l)
-      ok = cudaStreamCreateWithFlags(&p->lane_stream[l], cudaStreamNonBlocking) == cudaSuccess &&
-           cudaEventCreateWithFlags(&p->ev_done[l], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) {
-      set_error("tc_resnet_create: could not create the chunk-pipelining streams");
-      tc_resnet_destroy(p);
-      return KWS_ERR_CUDA;
-    }
   }
   *out = p;
   return KWS_OK;
@@ -859,11 +345,6 @@ void tc_resnet_destroy(TcResNet* p) {
   if (!p) return;
   if (p->blob) cudaFree(p->blob);
   if (p->fused_dev) cudaFree(p->fused_dev);
-  for (int l = 0; l < kTcMaxLanes; ++l) {
-    if (p->lane_stream[l]) cudaStreamDestroy(p->lane_stream[l]);
-    if (p->ev_done[l]) cudaEventDestroy(p->ev_done[l]);
-  }
-  if (p->ev_start) cudaEventDestroy(p->ev_start);
   delete p;
 }
 
@@ -900,19 +381,6 @@ static void tc_map_hw(const kws_resnet_config& c, int T, int F, int* H, int* W) 
   *W = F / pw;
 }
 
-static int64_t tc_chunk(const TcResNet* p, int64_t B, int H, int W, int chunk) {
-  const int64_t per = (int64_t)p->NP * H * W * 16;
-  int64_t c = chunk > 0 ? chunk : (256ll << 20) / (2 * std::max<int64_t>(per, 1));
-  if (chunk <= 0) {
-    // whole number of CTA waves for the common 7-tile geometry is not knowable here; keep it simple
-    if (c < 16) c = 16;
-    if (c > 2048) c = 2048;
-  }
-  if (c > B) c = B;
-  if (c < 1) c = 1;
-  return c;
-}
-
 static bool tc_layers_ok(const TcResNet* p, int H, int W) {
   TcGeom g;
   const int Hpad = tc_hpad(p->cfg, H);
@@ -923,54 +391,29 @@ static bool tc_layers_ok(const TcResNet* p, int H, int W) {
   return true;
 }
 
-static size_t tc_lane_bytes(const TcResNet* p, int64_t chunk, int H, int W, size_t* buf_out) {
-  const size_t buf = round_up<size_t>((size_t)chunk * p->NP * tc_hpad(p->cfg, H) * W * 16, 1024);
-  if (buf_out) *buf_out = buf;
-  return 2 * buf + round_up<size_t>((size_t)chunk * p->CP * 4, 1024);   // two activation buffers + pooled sums
-}
-
-static int tc_encode_map(const void* base, int64_t planes, int H, int W, const TcGeom& g, CUtensorMap* out);
-
-static int tc_get_map(TcResNet* p, const void* base, int64_t planes, int H, int W, const TcGeom& g, CUtensorMap** out) {
-  auto key = std::make_tuple(base, planes, H, W, (g.d * 1024 + g.rows_box) * 2 + g.phase);
-  auto it = p->maps.find(key);
-  if (it == p->maps.end()) {
-    if (p->maps.size() > 256) p->maps.clear();
-    CUtensorMap m;
-    KWS_TRY(tc_encode_map(base, planes, H, W, g, &m));
-    it = p->maps.emplace(key, m).first;
-  }
-  *out = &it->second;
-  return KWS_OK;
-}
-
+// Input tensor map of one layer: dims 8 channels, W, rows (of one phase), phases, planes.  Plain tiling is the
+// 1-phase case.
 static int tc_encode_map(const void* base, int64_t planes, int H, int W, const TcGeom& g, CUtensorMap* out) {
-  {
-    {
-    CUtensorMap& m = *out;
-    // dims: 8 channels, W, rows (of one phase), phases, planes.  Plain tiling is the 1-phase case.
-    const cuuint64_t row_stride = (cuuint64_t)W * 16, plane_stride = (cuuint64_t)g.Hpad * W * 16;
-    cuuint64_t dims[5], strides[4];
-    dims[0] = 8; dims[1] = (cuuint64_t)W; dims[4] = (cuuint64_t)planes;
-    strides[0] = 16; strides[3] = plane_stride;
-    if (g.phase) {
-      dims[2] = (cuuint64_t)(g.Hpad / g.d); dims[3] = (cuuint64_t)g.d;
-      strides[1] = row_stride * g.d; strides[2] = row_stride;
-    } else {
-      dims[2] = (cuuint64_t)H; dims[3] = 1;
-      strides[1] = row_stride; strides[2] = plane_stride;
-    }
-    const cuuint32_t box[5] = {8, (cuuint32_t)g.Wp, (cuuint32_t)g.rows_box, 1, 1};
-    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = get_encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), dims, strides, box,
-                                 estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled failed (%d) for W=%d H=%d planes=%lld box=%dx%d phase=%d", (int)r, W, H,
-                (long long)planes, g.Wp, g.rows_box, g.phase);
-      return KWS_ERR_CUDA;
-    }
-    }
+  const cuuint64_t row_stride = (cuuint64_t)W * 16, plane_stride = (cuuint64_t)g.Hpad * W * 16;
+  cuuint64_t dims[5], strides[4];
+  dims[0] = 8; dims[1] = (cuuint64_t)W; dims[4] = (cuuint64_t)planes;
+  strides[0] = 16; strides[3] = plane_stride;
+  if (g.phase) {
+    dims[2] = (cuuint64_t)(g.Hpad / g.d); dims[3] = (cuuint64_t)g.d;
+    strides[1] = row_stride * g.d; strides[2] = row_stride;
+  } else {
+    dims[2] = (cuuint64_t)H; dims[3] = 1;
+    strides[1] = row_stride; strides[2] = plane_stride;
+  }
+  const cuuint32_t box[5] = {8, (cuuint32_t)g.Wp, (cuuint32_t)g.rows_box, 1, 1};
+  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  CUresult r = get_encode_fn()(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(base), dims, strides, box,
+                               estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
+                               CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    set_error("cuTensorMapEncodeTiled failed (%d) for W=%d H=%d planes=%lld box=%dx%d phase=%d", (int)r, W, H,
+              (long long)planes, g.Wp, g.rows_box, g.phase);
+    return KWS_ERR_CUDA;
   }
   return KWS_OK;
 }
@@ -986,7 +429,7 @@ struct TcFusedPlan {
 static TcFusedPlan tc_fused_plan(const TcResNet* p, int H, int W, bool split) {
   TcFusedPlan f;
   const kws_resnet_config& c = p->cfg;
-  if ((!p->fused_enabled && !split) || c.n_layers < 1 || c.n_layers > kFusedMaxLayers || c.n_labels > 4096) return f;
+  if (c.n_layers < 1 || c.n_layers > kFusedMaxLayers || c.n_labels > 4096) return f;
   f.Hpad = tc_hpad(c, H);
   f.n_slots = p->n_sms;
   f.split = split;
@@ -997,7 +440,7 @@ static TcFusedPlan tc_fused_plan(const TcResNet* p, int H, int W, bool split) {
   for (int i = 1; i <= c.n_layers; ++i) {
     TcGeom g;
     const int d = c.use_dilation ? (1 << ((i - 1) / 3)) : 1;
-    // (tc_geom sizes its tiles for the layer-per-launch kernel's shared memory; the check below is this kernel's)
+    // (tc_geom picks the tile rows against a budget of one resident weight set; this kernel's ring is sized below)
     if (!tc_geom(p->NKC, H, f.Hpad, W, d, &g)) return f;
     f.slot_bytes = std::max(f.slot_bytes, round_up(g.stage_bytes, 128));
     f.geoms.push_back(g);
@@ -1465,23 +908,17 @@ static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat,
   }
 }
 
+// One rule for both precisions: the column-sweep kernel if its plan can stage the map, else the position-major
+// kernel, else unsupported (workspace 0).
 size_t tc_resnet_workspace_bytes(const TcResNet* p, int64_t B, int T, int F, int chunk, bool split) {
   if (!p || !p->supported) return 0;
   int H, W;
   tc_map_hw(p->cfg, T, F, &H, &W);
   if (H < 1 || W < 1 || W > 256 || !tc_layers_ok(p, H, W)) return 0;
   const TcSweepPlan sp = tc_sweep_plan(p, H, W, split);
+  if (sp.ok) return tc_sweep_ws_bytes(p, sp, H, W, B, chunk, nullptr);
   const TcFusedPlan f = tc_fused_plan(p, H, W, split);
-  if (split) {   // the split-bf16 mode exists in the two whole-network kernels only
-    if (sp.ok) return tc_sweep_ws_bytes(p, sp, H, W, B, chunk, nullptr);
-    return f.ok ? tc_fused_ws_bytes(p, f, W, nullptr) : 0;
-  }
-  const int64_t c = tc_chunk(p, B, H, W, chunk);
-  const size_t layered = p->lanes * tc_lane_bytes(p, c, H, W, nullptr);
-  // the layer-per-launch path stays available (profiling, shapes the fused kernel cannot stage)
-  size_t need = f.ok ? std::max(layered, tc_fused_ws_bytes(p, f, W, nullptr)) : layered;
-  if (sp.ok) need = std::max(need, tc_sweep_ws_bytes(p, sp, H, W, B, chunk, nullptr));
-  return need;
+  return f.ok ? tc_fused_ws_bytes(p, f, W, nullptr) : 0;
 }
 
 const char* tc_resnet_kernel_path(const TcResNet* p, int T, int F, bool split) {
@@ -1491,36 +928,7 @@ const char* tc_resnet_kernel_path(const TcResNet* p, int T, int F, bool split) {
   if (H < 1 || W < 1 || W > 256 || !tc_layers_ok(p, H, W)) return "unsupported";
   if (tc_sweep_plan(p, H, W, split).ok) return "resnet_tc_sweep_kernel";
   if (tc_fused_plan(p, H, W, split).ok) return "resnet_tc_fused_kernel";
-  return split ? "unsupported" : "conv3x3_tc_kernel";
-}
-
-template <int NKC, bool HAS_PREV, bool DO_POOL>
-static int tc_launch_conv3(const CUtensorMap& map, const TcConvParams& prm, int grid, cudaStream_t st) {
-  KWS_CUDA(cudaFuncSetAttribute(conv3x3_tc_kernel<NKC, HAS_PREV, DO_POOL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                prm.g.smem_total));
-  static const bool use_pdl = [] { const char* e = std::getenv("HONK2_TC_PDL"); return e == nullptr || std::atoi(e) != 0; }();
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(tc_threads(NKC));
-  cfg.dynamicSmemBytes = prm.g.smem_total;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = use_pdl ? 1 : 0;
-  KWS_CUDA(cudaLaunchKernelEx(&cfg, conv3x3_tc_kernel<NKC, HAS_PREV, DO_POOL>, map, prm));
-  ++g_launches;
-  return KWS_OK;
-}
-
-template <int NKC>
-static int tc_launch_conv(const CUtensorMap& map, const TcConvParams& prm, int grid, cudaStream_t st) {
-  const bool prev = prm.skip != nullptr, pool = prm.pool_sum != nullptr;
-  if (prev && pool) return tc_launch_conv3<NKC, true, true>(map, prm, grid, st);
-  if (prev) return tc_launch_conv3<NKC, true, false>(map, prm, grid, st);
-  if (pool) return tc_launch_conv3<NKC, false, true>(map, prm, grid, st);
-  return tc_launch_conv3<NKC, false, false>(map, prm, grid, st);
+  return "unsupported";
 }
 
 int tc_resnet_forward(TcResNet* p, const float* feat, int64_t B, int T, int F, float* logits, void* ws,
@@ -1530,9 +938,8 @@ int tc_resnet_forward(TcResNet* p, const float* feat, int64_t B, int T, int F, f
               p->cfg.n_maps);
     return KWS_ERR_UNSUPPORTED;
   }
-  const kws_resnet_config& c = p->cfg;
   int H, W;
-  tc_map_hw(c, T, F, &H, &W);
+  tc_map_hw(p->cfg, T, F, &H, &W);
   KWS_REQUIRE(H >= 1 && W >= 1, "ResNet: input %dx%d is smaller than the pooling window", T, F);
   const size_t need = tc_resnet_workspace_bytes(p, B, T, F, chunk_cfg, split);
   if (need == 0) {
@@ -1543,113 +950,9 @@ int tc_resnet_forward(TcResNet* p, const float* feat, int64_t B, int T, int F, f
     set_error("ResNet bf16 forward needs %zu bytes of workspace, got %zu", need, ws_bytes);
     return KWS_ERR_WORKSPACE;
   }
-  {
-    // whole-network persistent kernel unless per-launch profiling was requested
-    static const bool prof_layered = [] { const char* e = std::getenv("HONK2_TC_PROFILE_LAYERED"); return e && std::atoi(e) != 0; }();
-    const bool layered = prof && prof->enabled && prof_layered && !split;
-    const TcSweepPlan sp = tc_sweep_plan(p, H, W, split);
-    if (sp.ok && !layered) {
-      return tc_sweep_forward(p, sp, feat, B, T, F, H, W, logits, ws, chunk_cfg, prof, st);
-    }
-    const TcFusedPlan f = tc_fused_plan(p, H, W, split);
-    if (f.ok && !layered) {
-      return tc_fused_forward(p, f, feat, B, T, F, H, W, logits, ws, prof, st);
-    }
-    if (split) {
-      set_error("split-bf16 tensor-core path: no whole-network kernel can stage a %dx%d map", H, W);
-      return KWS_ERR_UNSUPPORTED;
-    }
-  }
-  const int64_t chunk = tc_chunk(p, B, H, W, chunk_cfg);
-  const int Hpad = tc_hpad(c, H);
-  size_t buf = 0;
-  const size_t lane_bytes = tc_lane_bytes(p, chunk, H, W, &buf);
-  // per-launch profiling needs one ordered stream; a single chunk has nothing to overlap with
-  const int lanes = (prof && prof->enabled) || B <= chunk ? 1 : p->lanes;
-  cudaStream_t caller = st;
-  if (lanes > 1) {
-    KWS_CUDA(cudaEventRecord(p->ev_start, caller));
-    for (int l = 0; l < lanes; ++l) KWS_CUDA(cudaStreamWaitEvent(p->lane_stream[l], p->ev_start, 0));
-  }
-  const bool fuse_pool = c.n_layers >= 1;
-  const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
-  KWS_REQUIRE(W <= 256, "conv_0: map width %d exceeds 256", W);
-  const bool fast0 = (ph == 1 && pw == 1);
-  const int groups0 = ceil_div(W, kC0Px);
-  const int rows0f = std::max(1, std::min(H, 256 / groups0));
-  const size_t smem0f = sizeof(float) * (round_up((rows0f + 2) * (groups0 * kC0Px + 2), 4) + p->NP * 8 * 12);
-  const int rows0 = std::max(1, std::min(H, 256 / W));
-  const size_t smem0 = sizeof(float) * (round_up((rows0 * ph + 2) * (F + 2), 4) + p->NP * 8 * 12);
-  KWS_REQUIRE(smem0 <= 48 * 1024, "conv_0: tile needs %zu bytes of shared memory", smem0);
-
-  int64_t chunk_idx = 0;
-  for (int64_t b0 = 0; b0 < B; b0 += chunk, ++chunk_idx) {
-    const int64_t nb = std::min(chunk, B - b0);
-    const int lane = (int)(chunk_idx % lanes);
-    if (lanes > 1) st = p->lane_stream[lane];
-    char* lws = static_cast<char*>(ws) + (size_t)lane * lane_bytes;
-    // P: conv_0 output and the even layers' activations (updated in place, it doubles as the skip tensor);
-    // Q: the odd layers' activations
-    __nv_bfloat16* P = reinterpret_cast<__nv_bfloat16*>(lws);
-    __nv_bfloat16* Q = reinterpret_cast<__nv_bfloat16*>(lws + buf);
-    float* pool = reinterpret_cast<float*>(lws + 2 * buf);
-    if (Hpad > H && chunk_idx < lanes) {   // first use of this lane's buffers in this call
-      for (__nv_bfloat16* bp : {P, Q}) {
-        zero_pad_rows_kernel<<<256, 256, 0, st>>>(reinterpret_cast<uint4*>(bp), chunk * p->NP, H, Hpad, W);
-        KWS_CHECK_LAUNCH();
-      }
-    }
-    if (prof) prof->tick(1, st);
-    if (fast0 && smem0f <= 48 * 1024)
-      conv0_p8_w4_kernel<<<dim3(ceil_div(H, rows0f), (unsigned)nb), 256, smem0f, st>>>(
-          feat + b0 * (int64_t)T * F, p->conv0_w, P, fuse_pool ? pool : nullptr, T, F, c.n_maps, p->NP, groups0,
-          rows0f, Hpad);
-    else
-      conv0_p8_kernel<<<dim3(ceil_div(H, rows0), (unsigned)nb), 256, smem0, st>>>(
-          feat + b0 * (int64_t)T * F, p->conv0_w, P, fuse_pool ? pool : nullptr, T, F, c.n_maps, p->NP, ph, pw, H,
-          W, rows0, Hpad);
-    KWS_CHECK_LAUNCH();
-    for (int i = 1; i <= c.n_layers; ++i) {
-      TcConvParams prm;
-      const int d = c.use_dilation ? (1 << ((i - 1) / 3)) : 1;
-      KWS_REQUIRE(tc_geom(p->NKC, H, Hpad, W, d, &prm.g), "bf16 conv: cannot tile H=%d W=%d d=%d", H, W, d);
-      const bool even = (i % 2 == 0), last = (i == c.n_layers);
-      const __nv_bfloat16* x = even ? Q : P;     // input: output of the previous layer
-      CUtensorMap* map = nullptr;
-      KWS_TRY(tc_get_map(p, x, nb * p->NP, H, W, prm.g, &map));
-      prm.wpack = p->wpack[i - 1];
-      prm.kconst = p->shift_p[i - 1];
-      prm.skip = even ? P : nullptr;             // resnet.py:51-53, reconstructed from z_{i-2}
-      prm.y = last ? nullptr : (even ? P : Q);   // even layers overwrite their skip tensor element-wise
-      prm.pool_sum = last ? pool : nullptr;
-      prm.B = (int)nb;
-      prm.total_tiles = (int)nb * prm.g.tiles_per_utt;
-      const int grid = std::min(p->n_sms, prm.total_tiles);
-      if (prof) prof->tick(0, st);
-      switch (p->NKC) {
-        case 1: KWS_TRY(tc_launch_conv<1>(*map, prm, grid, st)); break;
-        case 2: KWS_TRY(tc_launch_conv<2>(*map, prm, grid, st)); break;
-        case 3: KWS_TRY(tc_launch_conv<3>(*map, prm, grid, st)); break;
-        default: KWS_TRY(tc_launch_conv<4>(*map, prm, grid, st)); break;
-      }
-    }
-    if (prof) prof->tick(1, st);
-    if (fuse_pool)
-      tail_pool_kernel<<<(unsigned)ceil_div<int64_t>(nb * c.n_labels, 256), 256, 0, st>>>(
-          pool, p->scale_p[c.n_layers - 1], p->out_w, p->out_b, logits + b0 * c.n_labels, nb, c.n_maps, p->CP, H * W,
-          c.n_labels);
-    else
-      tail_p8_kernel<<<(unsigned)nb, 256, 0, st>>>(P, p->out_w, p->out_b, logits + b0 * c.n_labels, c.n_maps, p->NP,
-                                                   H * W, c.n_labels);   // n_layers == 0: Hpad == H
-    KWS_CHECK_LAUNCH();
-  }
-  if (lanes > 1) {
-    for (int l = 0; l < lanes; ++l) {
-      KWS_CUDA(cudaEventRecord(p->ev_done[l], p->lane_stream[l]));
-      KWS_CUDA(cudaStreamWaitEvent(caller, p->ev_done[l], 0));
-    }
-  }
-  return KWS_OK;
+  const TcSweepPlan sp = tc_sweep_plan(p, H, W, split);
+  if (sp.ok) return tc_sweep_forward(p, sp, feat, B, T, F, H, W, logits, ws, chunk_cfg, prof, st);
+  return tc_fused_forward(p, tc_fused_plan(p, H, W, split), feat, B, T, F, H, W, logits, ws, prof, st);
 }
 
 }  // namespace kws

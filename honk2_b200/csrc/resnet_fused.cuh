@@ -11,11 +11,32 @@
 //                  layer i odd : TMA reads P, epilogue writes Q
 //                  layer i even: TMA reads Q, epilogue adds the skip (read from P) and writes P in place
 //                  last layer  : epilogue accumulates the pooled sums in shared memory -> logits
-// The per-tile pipeline inside a layer is the one of conv3x3_tc_kernel (TMA producer warp, 3 MMA
-// issuer warps, 8 epilogue warps, mbarrier ring, double-buffered TMEM accumulators).  Between
-// layers the CTA drains: epilogue stores -> __threadfence + fence.proxy.async -> __syncthreads ->
-// the producer may issue TMA loads of what was just written.  Weights of layer i+1 are bulk-copied
+// Between layers the CTA drains: epilogue stores -> __threadfence + fence.proxy.async -> __syncthreads
+// -> the producer may issue TMA loads of what was just written.  Weights of layer i+1 are bulk-copied
 // into the second weight buffer while layer i runs.
+//
+// Activation layout ("planar-8"): [slot][NP][Hpad][W][8] bf16, NP = CP/8 planes of 8 channels,
+// CP = channels padded to a multiple of 16 (45 -> 48).  One plane row is W*16 contiguous bytes,
+// so a TMA box {8 ch, Wp, rows} lands in shared memory as a dense array of 16-byte "positions":
+// exactly the UMMA K-major SWIZZLE_NONE canonical layout (core matrix = 8 positions x 16 B,
+// SBO = 128 B), in which a pixel shift is nothing but a start-address offset.
+//
+// Implicit GEMM per tap (dh, dw) and 16-channel chunk kc:
+//   D[128 positions x CP] += A[128 positions x 16] (shifted view of the staged tile)
+//                          * B[16 x CP]            (weights, resident in shared memory)
+// Positions are flat indices p = r * Wp + c into the zero-padded tile rows (Wp = W + d: the d
+// left-pad columns of row r+1 double as the right padding of row r; TMA out-of-bounds fill
+// supplies every zero).  Outputs at pad positions are computed and discarded.  Tile rows and
+// boxes come from tc_geom (conv_tc.cu); large dilations tile by phase (rows p, p+d, p+2d, ...).
+//
+// Warp roles (tc_threads(NKC) threads, 1 CTA per SM; every role walks the same tile sequence):
+//   warp 0             TMA producer: one ring stage = one 16-channel chunk of the haloed input tile
+//   warps 1-3          MMA issuers, one elected lane each; the M-tiles of a tile are dealt round-robin
+//                      (warp 1 also allocates TMEM)
+//   4*NKC warps        epilogue: tcgen05.ld -> ReLU -> +skip -> BN -> bf16 planar-8 stores
+//                      (last layer: pooled sums instead of stores)
+// TMEM holds two accumulator buffers (up to min(8, 256 / CP) M-tiles x CP columns each) so the
+// epilogue of tile i overlaps the MMAs of tile i+1.
 //
 // SPLIT (the "bf16x3" precision): activations and weights are carried as bf16 pairs hi + lo (planes 0 .. NP-1 hold the
 // hi parts, NP .. 2 NP-1 the lo parts; the lo weight set follows the hi set) and every product is three MMAs,

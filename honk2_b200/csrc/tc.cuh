@@ -17,8 +17,8 @@ size_t tc_resnet_workspace_bytes(const TcResNet* p, int64_t B, int T, int F, int
 int tc_resnet_forward(TcResNet* p, const float* feat, int64_t B, int T, int F, float* logits, void* ws,
                       size_t ws_bytes, int chunk, bool split, LaunchProfiler* prof, cudaStream_t st);
 
-// Which kernel a bf16 forward of a [B][T][F] batch runs: "resnet_tc_sweep_kernel", "resnet_tc_fused_kernel",
-// "conv3x3_tc_kernel" (layer per launch) or "unsupported".
+// Which kernel a bf16 / split-bf16 forward of a [B][T][F] batch runs: "resnet_tc_sweep_kernel" if the column-sweep
+// plan can stage the map, else "resnet_tc_fused_kernel" if the position-major plan can, else "unsupported".
 const char* tc_resnet_kernel_path(const TcResNet* p, int T, int F, bool split);
 
 

@@ -153,17 +153,21 @@ int kws_model_forward_wave_pcm16(kws_model_t* m, const kws_frontend_t* fe, const
 /* Number of kernel launches the last forward on this handle issued (bench "gpu_launches"). */
 int64_t kws_model_last_launches(const kws_model_t* m);
 /* Name of the kernel family a forward of a [B][T][F] batch runs in the given precision (bench / profile labels):
- * "resnet_tc_sweep_kernel", "resnet_tc_fused_kernel", "conv3x3_tc_kernel", "fp32 CUDA-core kernels" or
- * "unsupported".  Static string, never freed. */
+ * "resnet_tc_sweep_kernel", "resnet_tc_fused_kernel", "fp32 CUDA-core kernels" or "unsupported".  Static string,
+ * never freed. */
 const char* kws_model_kernel_path(const kws_model_t* m, int T, int F, int precision);
 /* Per-launch timing for the bench roofline: while enabled, kws_model_forward brackets every
- * layer launch with CUDA events and synchronises the stream before returning.
+ * launch with CUDA events and synchronises the stream before returning.
  * kws_model_profile_read returns (and clears) the accumulated milliseconds / launch counts of
- * the C->C convolution launches (the dominant kernel) and of all other launches. */
+ * the dominant kernel's launches and of all other launches.  The dominant kernel is the C->C
+ * convolution on the fp32 paths, the whole-network kernel on the ResNet tensor-core paths and the
+ * fused conv_0 + conv_1 kernel on the CNN tensor-core path. */
 int kws_model_set_profile(kws_model_t* m, int enabled);
 int kws_model_profile_read(kws_model_t* m, double* conv_ms, int64_t* conv_launches, double* other_ms,
                            int64_t* other_launches);
-/* Tuning knob: utterances per L2-resident sub-batch of the tensor-core path (0 = default). */
+/* Tuning knob: utterances per sub-batch (0 = default) of the fp32 paths, of the bf16 CNN path and of the
+ * packed-strip mode of the ResNet column-sweep kernel.  The other ResNet tensor-core paths run the whole
+ * batch in one launch and ignore it. */
 int kws_model_set_chunk(kws_model_t* m, int precision, int chunk);
 
 /* ---- metrics: replaces Acc.accumulate (metric/acc.py:14-24) -------------------------------

@@ -847,6 +847,90 @@ def _kernel_path(m, dev, T=101, F=40):
     return lib.kws_model_kernel_path(st["handle"], T, F, m._precision_id()).decode()
 
 
+def _workspace_bytes(m, dev, B, T=101, F=40):
+    lib, st = m._state(dev)
+    return lib.kws_model_workspace_bytes(st["handle"], B, T, F, m._precision_id())
+
+
+# The whole-network kernel every zoo ResNet runs in the two tensor-core precisions, on 1 s (101 frames) and 9 s (901
+# frames) clips, as measured on a B200.  A change that moves a zoo config to another kernel has to say so here.
+ZOO_KERNEL_PATHS = {
+    ("dev", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("dev", "bf16", 901): "resnet_tc_fused_kernel",
+    ("dev", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("dev", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("hey_snips_res26", "bf16", 101): "resnet_tc_fused_kernel",
+    ("hey_snips_res26", "bf16", 901): "resnet_tc_fused_kernel",
+    ("hey_snips_res26", "bf16x3", 101): "resnet_tc_fused_kernel",
+    ("hey_snips_res26", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res15", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res15", "bf16", 901): "resnet_tc_sweep_kernel",
+    ("res15", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res15", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res15_narrow", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res15_narrow", "bf16", 901): "resnet_tc_sweep_kernel",
+    ("res15_narrow", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res15_narrow", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res26", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res26", "bf16", 901): "resnet_tc_fused_kernel",
+    ("res26", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res26", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res26_narrow", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res26_narrow", "bf16", 901): "resnet_tc_fused_kernel",
+    ("res26_narrow", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res26_narrow", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res8", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res8", "bf16", 901): "resnet_tc_fused_kernel",
+    ("res8", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res8", "bf16x3", 901): "resnet_tc_fused_kernel",
+    ("res8_narrow", "bf16", 101): "resnet_tc_sweep_kernel",
+    ("res8_narrow", "bf16", 901): "resnet_tc_fused_kernel",
+    ("res8_narrow", "bf16x3", 101): "resnet_tc_sweep_kernel",
+    ("res8_narrow", "bf16x3", 901): "resnet_tc_fused_kernel",
+}
+
+
+@pytest.mark.parametrize("name,precision,T", sorted(ZOO_KERNEL_PATHS))
+def test_zoo_resnet_kernel_dispatch(dev, name, precision, T):
+    assert {n for n, _, _ in ZOO_KERNEL_PATHS} == set(RESNETS)
+    m, _ = gpu_model(name, "default", dev, precision=precision)
+    assert _kernel_path(m, dev, T=T) == ZOO_KERNEL_PATHS[name, precision, T]
+
+
+@pytest.mark.parametrize("n_layers", [0, 65])
+def test_resnet_depths_without_a_whole_network_kernel(dev, n_layers):
+    """No C->C layers, or more than the 64 the whole-network kernels hold: the tensor-core precisions refuse the model
+    (no workspace, kernel path "unsupported", NativeError from the forward); the fp32 path still runs it."""
+    from honk2_b200.class_registry import find_cls
+    cfg = {"n_layers": n_layers, "n_feature_maps": 19, "use_dilation": False, "n_labels": 12}
+    torch.manual_seed(n_layers)
+    m = find_cls("model.ResNet")(dict(cfg))
+    m.eval()
+    sd = {k: v.clone() for k, v in m.state_dict().items()}
+    x = torch.randn(3, 101, 40, generator=torch.Generator().manual_seed(n_layers)) * 3.0
+    ref = model_ref.forward("ResNet", sd, cfg, x).numpy()
+    m = m.to(dev)
+    with torch.no_grad():
+        y = m(x.to(dev)).cpu().numpy()
+    assert logit_err(y, ref) <= LOGIT_TOL, logit_err(y, ref)
+    for precision in ("bf16", "bf16x3"):
+        m.precision = precision
+        assert _kernel_path(m, dev) == "unsupported"
+        assert _workspace_bytes(m, dev, 3) == 0
+        with pytest.raises(honk2_b200.NativeError), torch.no_grad():
+            m(x.to(dev))
+
+
+def test_bf16_workspace_is_what_the_sweep_kernel_uses(dev):
+    """res15 at 8192 x 1 s clips in bf16: the workspace is the sweep kernel's two activation buffers per SM slot,
+    [n_sms][NP = 6][101][40][16 B] each, rounded up to 1 KB; nothing is reserved for any other path."""
+    m, _ = gpu_model("res15", "default", dev, precision="bf16")
+    assert _kernel_path(m, dev) == "resnet_tc_sweep_kernel"
+    n_sms = torch.cuda.get_device_properties(dev).multi_processor_count
+    buf = -(-n_sms * 6 * 101 * 40 * 16 // 1024) * 1024
+    assert _workspace_bytes(m, dev, 8192) == 2 * buf
+
+
 @pytest.mark.parametrize("name", ["res8", "res26", "res8_narrow", "res26_narrow"])
 @pytest.mark.parametrize("precision,tol", [("bf16", BF16_TOL), ("bf16x3", LOGIT_TOL)])
 def test_packed_strips_ragged_batches_vs_oracle(dev, name, precision, tol):
