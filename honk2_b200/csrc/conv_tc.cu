@@ -429,7 +429,7 @@ struct TcFusedPlan {
 static TcFusedPlan tc_fused_plan(const TcResNet* p, int H, int W, bool split) {
   TcFusedPlan f;
   const kws_resnet_config& c = p->cfg;
-  if (c.n_layers < 1 || c.n_layers > kFusedMaxLayers || c.n_labels > 4096) return f;
+  if (c.n_layers < 1 || c.n_layers > kFusedMaxLayers) return f;
   f.Hpad = tc_hpad(c, H);
   f.n_slots = p->n_sms;
   f.split = split;
@@ -579,7 +579,8 @@ static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
   const int H_map = H;
   (void)H_map;
   const kws_resnet_config& c = p->cfg;
-  if (!p->sweep_enabled || c.n_layers < 1 || c.n_layers > kFusedMaxLayers || c.n_labels > 4096) return f;
+  // (no label bound: both kernels' tails loop over every label kws_resnet_create accepts, 1..1024)
+  if (!p->sweep_enabled || c.n_layers < 1 || c.n_layers > kFusedMaxLayers) return f;
   if (W < 1 || W > kSwMaxW || H < 1) return f;
   if (p->NKC > 3) return f;   // 64 maps: 640 threads leave 96 registers, the epilogue spills (position-major kernel instead)
   if ((1 + c.n_layers) * p->CP * 4 > kSwKcBytes) return f;   // per-layer epilogue constants live in shared memory

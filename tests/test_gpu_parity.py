@@ -783,13 +783,19 @@ def test_bf16_sweep_kernel_label_counts(dev, n_labels, model_golden):
     assert logit_err(y, ref) <= BF16_TOL, logit_err(y, ref)
 
 
+ODD_MAP_PATHS = {100: "resnet_tc_sweep_kernel", 128: "resnet_tc_sweep_kernel", 129: "resnet_tc_fused_kernel",
+                 97: "resnet_tc_sweep_kernel"}
+
+
 @pytest.mark.parametrize("T,F,B", [(100, 8, 5), (128, 3, 2), (129, 17, 3), (97, 1, 4)])
 def test_bf16_sweep_kernel_odd_map_shapes(dev, T, F, B):
     """Maps narrower than the dilation (every run is a single column: one-block windows, both stand-in arrivals),
-    layers with fewer steps than the weight-prefetch step, a strip boundary at exactly 128 rows and one row more,
-    a single-column map: all against the CPU oracle (res15 topology, 13 layers, dilation up to 16)."""
+    layers with fewer steps than the weight-prefetch step, a map of exactly one 128-row strip, a single-column map: all
+    against the CPU oracle (res15 topology, 13 layers, dilation up to 16).  129 rows fill 50 % of two strips and are too
+    tall to stack, so they run on the position-major kernel; test_tc_shapes.py has the sweep's real strip boundaries."""
     kind, cfg = model_config("res15")
     m, sd = gpu_model("res15", "hardened", dev, precision="bf16")
+    assert _kernel_path(m, dev, T=T, F=F) == ODD_MAP_PATHS[T]
     g = torch.Generator().manual_seed(T * 100 + F)
     x = torch.randn(B, T, F, generator=g) * 3.0 - 8.0
     ref = model_ref.forward(kind, sd, cfg, x).numpy()
@@ -972,14 +978,21 @@ def test_packed_strips_match_position_major_kernel(dev, monkeypatch, name):
     assert float((y_pack - y_pos).abs().max()) <= 1e-2 * float(y_pos.abs().max())
 
 
-@pytest.mark.parametrize("name,T", [("res15", 50), ("res15", 33), ("res15_narrow", 61), ("res8", 57)])
+SHORT_CLIP_PATHS = {("res15", 50): "resnet_tc_sweep_kernel", ("res15", 33): "resnet_tc_sweep_kernel",
+                    ("res15_narrow", 61): "resnet_tc_fused_kernel", ("res8", 57): "resnet_tc_sweep_kernel"}
+
+
+@pytest.mark.parametrize("name,T", list(SHORT_CLIP_PATHS))
 def test_packed_strips_short_clips(dev, name, T):
-    """Short clips: unpooled maps of fewer than 77 rows are stacked with dmax (16 for res15) zero rows between them."""
+    """Short clips: unpooled maps of fewer than 77 rows are stacked with dmax (16 for res15) zero rows between them, as
+    many as fit a 128-row strip (two of 50 or 33 rows; eight of res8's pooled 14).  Two maps of 61 rows do not fit, and a
+    single map that fills less than 60 % of its strip stays on the position-major kernel."""
     kind, cfg = model_config(name)
     rng = np.random.default_rng(T)
     feats = torch.from_numpy((rng.standard_normal((37, T, 40)) * 4 - 6).astype(np.float32))
     for precision, tol in (("bf16", BF16_TOL), ("bf16x3", LOGIT_TOL)):
         m, sd = gpu_model(name, "hardened", dev, precision=precision)
+        assert _kernel_path(m, dev, T=T) == SHORT_CLIP_PATHS[name, T], precision
         with torch.no_grad():
             y = m(feats.to(dev)).cpu().numpy()
         ref = model_ref.forward(kind, sd, cfg, feats).numpy()
