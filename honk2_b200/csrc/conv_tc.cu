@@ -611,8 +611,8 @@ static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
   f.n_slots = p->n_sms;
   f.dmax = dmax;
   f.split = split;
-  // 16 channels per row: [K chunk][w][h][32 B] in HBM, swizzle-32B operand in shared memory, one bulk copy per chunk
-  // and step (single-strip maps; HONK2_TC_SWEEP_K32=0 keeps them on the planar layout of the multi-strip maps)
+  // 16 channels per row: [w][K chunk][h][32 B] in HBM, swizzle-32B operand in shared memory, one bulk copy per step
+  // (single-strip maps; HONK2_TC_SWEEP_K32=0 keeps them on the planar layout of the multi-strip maps)
   f.k32 = f.n_strips == 1 && (p->sweep_k32 || split);
   if (split && !f.k32) return f;   // the split-bf16 mode is built on the 32-byte-row layout
   const int set_bytes = 9 * p->NKC * 2 * p->CP * 16;           // one weight set
@@ -621,14 +621,25 @@ static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
   f.w_off[0] = f.c0w_off + round_up(3 * 2 * 3 * p->CP * 16, 128);
   f.w_off[1] = split ? f.w_off[0] : f.w_off[0] + round_up(w_bytes, 128);   // (split: one buffer, see the kernel)
   f.skip_off = round_up(f.w_off[1] + w_bytes, 1024);
-  f.pool_off = f.skip_off + (split ? 0 : sw_groups(p->NKC) * p->NP * 2048);   // one skip slot per epilogue warp group
+  // one skip slot per epilogue warp group: a planar strip column, [NP][128 rows][16 B], or a k32 column, NKC x H rows x 32 B
+  f.pool_off = f.skip_off + (split ? 0 : sw_groups(p->NKC) * p->NP * 2048);
   f.ring_off = f.pool_off + (f.packed ? round_up(f.pack_n * sw_epi_warps(p->NKC) * p->CP * 4, 1024) : 0);   // packed: pooled sums per stacked utterance
-  // rows per chunk of a staged column.  The split mode stages twice the chunks: its chunks are cut down to the rows
-  // the map's own lanes read (H + 2 dmax); the lanes past the map then read into the next chunk / the slack.
-  const int full_rows = (128 + 2 * dmax + 7) & ~7;
-  f.chunk_rows = (split && f.n_strips == 1) ? std::min(full_rows, round_up(H + 2 * dmax, 8)) : full_rows;
-  f.slot_bytes = (split ? 2 : 1) * p->NP * f.chunk_rows * 16;
-  f.slack_bytes = (full_rows - f.chunk_rows) * 32;
+  if (f.k32) {
+    // a stage is [dmax guard rows][NA chunks x H rows][to a multiple of 8 rows: stages stay 256-byte aligned, the phase
+    // of the 32-byte swizzle].  The MMA of chunk kc, tap dh reads 128 rows from dmax + kc H + (dh - 1) d: the last
+    // chunk's lanes past the map read up to dmax + (NA - 1) H + dmax + 128 rows, into the next stage or, behind the
+    // last stage, into the slack.
+    const int na = (split ? 2 : 1) * p->NKC;
+    const int slot_rows = round_up(dmax + na * H, 8);
+    f.chunk_rows = H;
+    f.slot_bytes = slot_rows * 32;
+    f.slack_bytes = round_up(std::max(0, dmax + (na - 1) * H + dmax + 128 - slot_rows), 8) * 32;
+  } else {
+    // planar: dmax zero rows above and below the strip's 128 rows, in every plane
+    f.chunk_rows = (128 + 2 * dmax + 7) & ~7;
+    f.slot_bytes = p->NP * f.chunk_rows * 16;
+    f.slack_bytes = 0;
+  }
   const int max_stages = std::min(kSwMaxStages, p->sweep_max_stages > 0 ? p->sweep_max_stages : kSwMaxStages);
   f.n_stages = std::min(max_stages, (227 * 1024 - f.slack_bytes - f.ring_off) / f.slot_bytes);
   if (f.n_stages < 3) return f;
@@ -660,8 +671,8 @@ static size_t tc_sweep_ws_bytes(const TcResNet* p, const TcSweepPlan& f, int H, 
 
 // conv_0 (1 -> C, 3x3, pad 1) + ReLU + AvgPool(PH, PW) (resnet.py:40-44) for the packed-strip mode of the sweep kernel:
 // writes the bf16 activations of a group of `pack_n` stacked utterances exactly as the sweep kernel's epilogue would
-// ([K chunk][w][stacked row][16 ch = 32 B], halves swapped where ((dmax + row) >> 2) & 1, zero rows between the
-// utterances; split: the lo parts in chunks NKC .. 2 NKC-1).  One thread = one (column, stacked row) position of a group;
+// ([w][K chunk][stacked row][16 ch = 32 B], halves of chunk kc swapped where ((dmax + kc Hst + row) >> 2) & 1, zero rows
+// between the utterances; split: the lo parts in chunks NKC .. 2 NKC-1).  One thread = one (column, stacked row) position of a group;
 // a group's W * Hst positions are dealt to blocks of 128 threads column by column (rows fastest: 32-byte stores coalesce).
 template <int PH, int PW>
 __global__ void __launch_bounds__(128)
@@ -692,7 +703,8 @@ conv0_pool_pack_kernel(const float* __restrict__ feat, const float* __restrict__
       patch[a][e] = (live && hh >= 0 && hh < T && ww >= 0 && ww < F) ? __ldg(feat + (b * T + hh) * (int64_t)F + ww) : 0.f;
     }
   constexpr float inv = 1.f / (float)(PH * PW);
-  const int swl = ((dmax + row) >> 2) & 1;
+  const int NA = split ? 2 * NKC : NKC;
+  auto swl_of = [&](int kc) { return ((dmax + kc * Hst + row) >> 2) & 1; };
   // (a warp whose 32 items are all gap rows / past the batch only stores zeros; the pad channels C .. CP-1 are zeros too)
   const bool warp_live = __any_sync(0xffffffffu, live);
   for (int kc = 0; kc < NKC; ++kc) {
@@ -730,13 +742,15 @@ conv0_pool_pack_kernel(const float* __restrict__ feat, const float* __restrict__
         lb[e] = __floats2bfloat162_rn(a - fh.x, c2 - fh.y);
       }
     }
-    uint4* dst = ext + g * ext_stride + ((int64_t)(kc * W + wo) * Hst + row) * 2;
+    uint4* dst = ext + g * ext_stride + ((int64_t)(wo * NA + kc) * Hst + row) * 2;
+    const int swl = swl_of(kc);
     dst[swl] = hi[0];
     dst[swl ^ 1] = hi[1];
     if (split) {
-      uint4* dl = ext + g * ext_stride + ((int64_t)((NKC + kc) * W + wo) * Hst + row) * 2;
-      dl[swl] = lo[0];
-      dl[swl ^ 1] = lo[1];
+      uint4* dl = ext + g * ext_stride + ((int64_t)(wo * NA + NKC + kc) * Hst + row) * 2;
+      const int swl_lo = swl_of(NKC + kc);
+      dl[swl_lo] = lo[0];
+      dl[swl_lo ^ 1] = lo[1];
     }
   }
 }

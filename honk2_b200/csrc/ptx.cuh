@@ -230,6 +230,18 @@ __device__ __forceinline__ void umma_f16_lohi2(uint32_t d_tmem, uint32_t a_lo, u
       ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "n"(kAccumulate ? 1 : 0)
       : "memory");
 }
+// Same, accumulating, with a disable-output-lane mask: bit i of the 128-bit {m.x, m.y, m.z, m.w} (word j = lanes
+// 32 j .. 32 j + 31) set = accumulator lane i is left unchanged (tools/umma_bench6: bit-exact, no cost at the pipe rate).
+__device__ __forceinline__ void umma_f16_lohi2_mask(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
+                                                    uint32_t idesc, const uint4& m) {
+  asm volatile(
+      "{\n\t.reg .b64 da, db;\n\t"
+      "mov.b64 da, {%1, %2};\n\t"
+      "mov.b64 db, {%3, %4};\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, {%6, %7, %8, %9}, 1;\n\t}"
+      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(m.x), "r"(m.y), "r"(m.z), "r"(m.w)
+      : "memory");
+}
 __device__ __forceinline__ void umma_f16_lohi2_rt(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
                                                   uint32_t idesc, uint32_t accumulate) {
   asm volatile(

@@ -18,14 +18,18 @@
 // ring is issued as two narrower MMAs (N = 96 + 48).
 //
 // Activation layouts, one slot (buffers P and Q) per CTA, staged by 1-D bulk copies (cp.async.bulk):
-//   single-strip maps (H <= 128): [slot][K chunk][W][H][16 ch = 32 B] bf16; a staged column is [chunk][pad | H rows |
-//     pad][32 B] in shared memory, read as a SWIZZLE_32B K-major operand, one copy of H*32 contiguous bytes per chunk
-//     into a slot whose pad rows were zeroed once;
+//   single-strip maps (H <= 128): [slot][W][K chunk][H][16 ch = 32 B] bf16, so that a column is NA * H * 32 contiguous
+//     bytes and lands with ONE copy per step in a stage laid out as [dmax guard rows][NA chunks x H rows][slack], read
+//     as a SWIZZLE_32B K-major operand (chunk pitch H rows).  Nothing in the stage is zero: the reference's zero
+//     padding (resnet.py:22-24, padding = dilation) is the MMA's disable-output-lane mask instead -- the height tap that
+//     reads row h - d leaves lanes 0 .. d-1 alone, the one that reads row h + d lanes H-d .. H-1 (tools/umma_bench6:
+//     bit-exact, and free at the pipe rate).  The guard and the slack, and the neighbouring chunk's rows, only ever
+//     feed masked lanes: lanes >= H are masked in every MMA too (their results are dropped anyway, and a disabled lane
+//     saves tensor-pipe power, which under the power cap is clock);
 //   taller maps ("column planar-8"): [slot][NP][W][H][8] bf16; a staged column is [NP planes][rows -d .. 128+d][8 ch]
 //     = the K-major SWIZZLE_NONE canonical layout (row pitch 16 B, plane pitch = LBO), one copy per plane of the rows
-//     of the strip's window that lie inside the map.
-// Rows outside the map are zero, which is exactly the reference's zero padding (resnet.py:22-24, padding =
-// dilation), and the +-d row shift of a height tap is a descriptor start-address offset.
+//     of the strip's window that lie inside the map; rows outside the map are zero rows of the stage.
+// The +-d row shift of a height tap is a descriptor start-address offset.
 //
 // SPLIT (the "bf16x3" precision, single-strip maps): every activation and weight is carried as a bf16 pair hi + lo
 // (hi = bf16(v), lo = bf16(v - hi): 16 mantissa bits) -- chunks 0 .. NKC-1 hold the hi parts, NKC .. 2 NKC-1 the lo
@@ -111,17 +115,17 @@ struct SwParams {
   int smem_c0w_off;             // conv_0 weight slabs (3 * 2 * 3*CP*16 bytes), resident for the whole kernel
   int smem_w_off[2], smem_ring_off, ring_slot_bytes, n_stages;
   int smem_skip_off;            // skip staging: one slot of NP * 2048 bytes per epilogue warp group (unused by SPLIT)
-  int ring_slack_bytes;         // zeroed bytes behind the last stage (see chunk_rows)
+  int ring_slack_bytes;         // bytes behind the last stage that its lanes past the map read (planar: zeroed)
   int l2_policy;
-  int chunk_rows;               // rows per plane / chunk of a staged column (a multiple of 8): data row h of the strip sits at
+  int chunk_rows;               // planar: rows per plane of a staged column (a multiple of 8): data row h of the strip sits at
                                 //   slot row dmax + h, the pad rows above and below are zero (single strip: zeroed once and
                                 //   never written; several strips: re-zeroed by the producer for the strips that touch the
-                                //   map's top / bottom).  128 + 2 dmax, or H + 2 dmax rounded up when the map is shorter than
-                                //   a strip (the lanes past the map then read into the next chunk: their results are unused)
-  int dmax;                     // largest dilation of the network
-  int k32;                      // 1 = activations as [K chunk][w][h][16 channels = 32 B] (single strip): one copy per chunk and
-                                //     step, swizzle-32B A operand; the two 16-byte halves of a row are stored swapped where
-                                //     ((dmax + h) >> 2) & 1, i.e. exactly as the linear copy must land them in the slot
+                                //   map's top / bottom), 128 + 2 dmax.  (k32: the chunk pitch is H)
+  int dmax;                     // largest dilation of the network = the guard rows in front of a k32 stage's first chunk
+  int k32;                      // 1 = activations as [w][K chunk][h][16 channels = 32 B] (single strip): one copy per step,
+                                //     swizzle-32B A operand, edge lanes masked; the two 16-byte halves of row h of chunk kc are
+                                //     stored swapped where ((dmax + kc H + h) >> 2) & 1, i.e. exactly as the linear copy must
+                                //     land them in the stage (stages are 256-byte aligned: the swizzle works on absolute addresses)
   int wait_polls;               // barrier polls before a wait falls back to the suspending try_wait (HONK2_TC_WAIT_POLLS)
   int discard_q;                // 1 = Q columns are discarded from L2 (no write-back) once the layer that reads them has consumed them
   int diag;                     // diagnostics (wrong results!): 1 = epilogue skips math and stores, 2 = skips the skip-tensor loads
@@ -132,7 +136,7 @@ struct SwParams {
   // neighbours).  H is then the stacked height, B counts GROUPS of pack_n utterances, and conv_0 (+ ReLU + AvgPool,
   // resnet.py:40-44) has been computed by conv0_pool_pack_kernel into `ext_in`, which the first layer reads instead of P
   // and the second layer adds as its skip tensor.
-  const uint4* ext_in;          // [groups][NA chunks][W][H][32 B] (nullptr: conv_0 runs in this kernel as a pseudo-layer)
+  const uint4* ext_in;          // [groups][W][NA chunks][H][32 B] (nullptr: conv_0 runs in this kernel as a pseudo-layer)
   int64_t ext_stride;           // 16-byte units per group
   int pack_n, pack_h, pack_pitch;
   int smem_pool_off;            // pack_n > 1: [pack_n][epilogue warps][CP] f32 pooled sums
@@ -183,10 +187,11 @@ resnet_tc_sweep_kernel(const SwParams p) {
   constexpr int ll0 = ext ? 1 : 0;
 
   // Activation layout in HBM (16-byte units = 8 bf16 channels of one position), one slot per CTA:
-  //   k32     [K chunk][w][h][2]      (single-strip maps; SPLIT: 2 NKC chunks, the lo parts after the hi parts)
+  //   k32     [w][K chunk][h][2]      (single-strip maps; SPLIT: 2 NKC chunks, the lo parts after the hi parts)
   //   planar  [plane][w][h]           (multi-strip maps)
   constexpr bool k32 = K32;   // (compile time: the two layouts' address arithmetic would not fit the epilogue's registers together)
-  const int64_t kc_stride = (int64_t)W * H * 2;   // k32: 16-byte units between K chunks
+  const int kc_stride = H * 2;                     // k32: 16-byte units between K chunks
+  const int64_t col_stride = (int64_t)NA * H * 2;  // k32: 16-byte units between columns
   const int64_t plane_stride = (int64_t)W * H;    // planar: 16-byte units between planes
   const int64_t slot_base = (int64_t)blockIdx.x * ((int64_t)(SPLIT ? 2 : 1) * NP * W * H);   // this CTA's utterance slot
   auto wait_lean = [&](uint32_t bar, uint32_t parity) { mbar_wait_lean(bar, parity, p.wait_polls); };
@@ -219,14 +224,13 @@ resnet_tc_sweep_kernel(const SwParams p) {
       s_kc[i] = ll == 0 ? 0.f : reinterpret_cast<const float*>(p.kconst0 + (ll - 1) * p.layer_stride)[c];
     }
   }
-  {
-    // the pad rows above and below the map are never written again and supply the zero padding (the slack behind the
-    // last stage is only ever read by lanes past the map)
+  if constexpr (!K32) {
+    // planar: the pad rows above and below the map are never written again and supply the zero padding
     uint4* ring = reinterpret_cast<uint4*>(smem + p.smem_ring_off);
     const int n16 = (p.n_stages * p.ring_slot_bytes + p.ring_slack_bytes) >> 4;
     for (int i = threadIdx.x; i < n16; i += sw_threads(NKC)) ring[i] = make_uint4(0u, 0u, 0u, 0u);
   }
-  fence_async_smem();   // generic-proxy writes (zeros, conv_0 weights) -> visible to the tensor core's (async proxy) reads
+  fence_async_smem();   // generic-proxy writes (conv_0 weights, planar zeros) -> visible to the tensor core's (async proxy) reads
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -310,9 +314,9 @@ resnet_tc_sweep_kernel(const SwParams p) {
           const uint32_t prev_phase = (uint32_t)(((sq - 1) >> 1) & 1);
           if (is_c0) {
             // conv_0 pseudo-layer: the producer BUILDS the staged columns.  Rows 128 s - 1 .. 128 s + 128 of feature
-            // column w, each as {hi, lo, 0 x 6} bf16 (fp32 feature split into two bf16 parts) in plane 0; the MMA's
-            // second K half reads the same plane (LBO = 0) against zero weights, so nothing an earlier layer left in
-            // the slot can reach this utterance.  Zero outside the map = the reference's padding.  Up to four
+            // column w (k32: rows 0 .. H-1), each as {hi, lo, 0 x 6} bf16 (fp32 feature split into two bf16 parts) in
+            // plane 0; the MMA's second K half reads the same plane (LBO = 0) against zero weights, so nothing an earlier
+            // layer left in the slot can reach this utterance.  Zero outside the map = the reference's padding.  Up to four
             // consecutive columns are built per pass from one 16-byte feature load per row: the MMAs of a conv_0 step
             // are few, so this warp's instruction count is what bounds the pseudo-layer.
             const int r0 = row0_of(1);
@@ -351,7 +355,8 @@ resnet_tc_sweep_kernel(const SwParams p) {
 #pragma unroll
                   for (int k = 0; k < 5; ++k) {
                     const int rr = lane + 32 * k;
-                    if (rr < 130 && r0 + rr < box_rows) {   // (a chunk cut down to the map never needs the rows past it)
+                    // k32: the map's rows only (the lane masks are the padding; a row past the map could be the next stage's)
+                    if (k32 ? (rr >= 1 && rr <= H) : (rr < 130 && r0 + rr < box_rows)) {
                       const float4 f = fr[k];
                       const float fv[4] = {f.x, f.y, f.z, f.w};
 #pragma unroll
@@ -403,15 +408,12 @@ resnet_tc_sweep_kernel(const SwParams p) {
                 pstamp(pd_empty);
                 const uint32_t dst = sbase + p.smem_ring_off + (uint32_t)stage * p.ring_slot_bytes;
                 if (k32) {
-                  // one contiguous H x 32 B run per 16-channel chunk (SPLIT: hi chunks, then lo chunks)
+                  // the whole column, NA chunks x H rows x 32 B (SPLIT: hi chunks, then lo chunks), behind the guard rows
                   if (leader) {
-                    const uint32_t bytes = (uint32_t)H * 32u;
-                    mbar_expect_tx(full_bar(stage), bytes * NA);
-                    const uint4* src = ((ext && l == 0) ? ext_b : in_q ? bufQ : bufP) + (int64_t)w * H * 2;
-                    const uint32_t d0 = dst + (uint32_t)p.dmax * 32u;
-#pragma unroll
-                    for (int kc = 0; kc < NA; ++kc)
-                      bulk_load_hint(d0 + (uint32_t)(kc * box_rows) * 32u, src + kc * kc_stride, bytes, full_bar(stage), pol);
+                    const uint32_t bytes = (uint32_t)(NA * H) * 32u;
+                    mbar_expect_tx(full_bar(stage), bytes);
+                    const uint4* src = ((ext && l == 0) ? ext_b : in_q ? bufQ : bufP) + (int64_t)w * col_stride;
+                    bulk_load_hint(dst + (uint32_t)p.dmax * 32u, src, bytes, full_bar(stage), pol);
                   }
                 } else {
                   // one contiguous H x 16 B run per 8-channel plane (a TMA box with 16-byte rows fetches a whole
@@ -523,12 +525,28 @@ resnet_tc_sweep_kernel(const SwParams p) {
           // (the swizzle is applied to absolute shared-memory addresses, so any row offset works: tools/umma_bench5)
           const uint32_t a_hi = k32 ? ((256u >> 4) | (1u << 14) | (6u << 29)) : desc_hi;
           const uint32_t row_mul = k32 ? 2u : 1u;                                    // 16-byte units per row
-          const uint32_t kc_step = k32 ? (uint32_t)box_rows * 2u : 2u * plane16;     // 16-byte units per K chunk
+          const uint32_t kc_step = k32 ? (uint32_t)H * 2u : 2u * plane16;            // 16-byte units per K chunk
           const uint32_t w16 = ((sbase + (is_c0 ? p.smem_c0w_off : p.smem_w_off[wq & 1])) >> 4);
           const uint32_t row0 = (uint32_t)row0_of(d);
           // SPLIT: the lo chunks of the staged column follow the NKC hi chunks, the lo slabs follow the hi slabs
           const uint32_t a_lo_off = (uint32_t)NKC * kc_step;
           constexpr uint32_t b_lo_off = (uint32_t)(W_PART >> 4);
+          // k32: the zero padding of the map's edge rows.  The tap dh = 0 reads row h - d: lanes 0 .. d-1 get nothing;
+          // dh = 2 reads row h + d: lanes H-d .. H-1 get nothing.  Every tap also leaves the lanes past the map
+          // (>= H, results never used) alone: the tensor pipe then draws less power, and under the power cap that is
+          // clock (res15: 27 of 128 lanes, +3 % end to end on its own, NVIDIA B200 at 1000 W).
+          auto lane_bits = [](int lo, int hi, int j) {   // word j of the mask of lanes lo .. hi-1
+            const int a = min(max(lo - 32 * j, 0), 32), b = min(max(hi - 32 * j, 0), 32);
+            return (b >= 32 ? ~0u : (1u << b) - 1u) & ~(a >= 32 ? ~0u : (1u << a) - 1u);
+          };
+          const uint4 m_ge = make_uint4(lane_bits(H, 128, 0), lane_bits(H, 128, 1), lane_bits(H, 128, 2), lane_bits(H, 128, 3));
+          const uint4 m_top = make_uint4(lane_bits(0, d, 0) | m_ge.x, lane_bits(0, d, 1) | m_ge.y, lane_bits(0, d, 2) | m_ge.z, lane_bits(0, d, 3) | m_ge.w);
+          const uint4 m_bot = make_uint4(lane_bits(H - d, 128, 0), lane_bits(H - d, 128, 1), lane_bits(H - d, 128, 2), lane_bits(H - d, 128, 3));
+          // one MMA of height tap dh (compile-time after unrolling)
+          auto mma = [&](int dh, uint32_t dt, uint32_t a, uint32_t b, uint32_t id) {
+            if (k32) umma_f16_lohi2_mask(dt, a, a_hi, b, desc_hi, id, dh == 0 ? m_top : dh == 1 ? m_ge : m_bot);
+            else umma_f16_lohi2<true>(dt, a, a_hi, b, desc_hi, id);
+          };
           stamp(dbg_other);
           if (!is_c0) wait_lean(wfull_bar((int)(wq & 1)), (uint32_t)((wq >> 1) & 1));
           stamp(dbg_w);
@@ -583,23 +601,23 @@ resnet_tc_sweep_kernel(const SwParams p) {
                     // conv_0: one 16-channel chunk (k = 0 .. 2 are its three height taps)
                     if (wrap_at == n) {
 #pragma unroll
-                      for (int k = 0; k < 3; ++k) umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k], desc_hi, id1);
+                      for (int k = 0; k < 3; ++k) mma(k, d1, al[k], bl[k], id1);
                     } else {
                       const uint32_t id2 = idesc0 + (uint32_t)(n - wrap_at) * idesc_blk;
                       const uint32_t bo2 = (uint32_t)wrap_at * blk16;
 #pragma unroll
                       for (int k = 0; k < 3; ++k) {
-                        umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k], desc_hi, id1);
-                        umma_f16_lohi2<true>(tmem_u, al[k], a_hi, bl[k] + bo2, desc_hi, id2);
+                        mma(k, d1, al[k], bl[k], id1);
+                        mma(k, tmem_u, al[k], bl[k] + bo2, id2);
                       }
                     }
                   } else if (wrap_at == n) {
 #pragma unroll
                     for (int k = 0; k < 3 * NKC; ++k) {
-                      umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k], desc_hi, id1);
+                      mma(k % 3, d1, al[k], bl[k], id1);
                       if constexpr (SPLIT) {   // lo x hi, hi x lo (shared memory ends far below 256 KB: no carry out of the address fields)
-                        umma_f16_lohi2<true>(d1, al[k] + a_lo_off, a_hi, bl[k], desc_hi, id1);
-                        umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k] + b_lo_off, desc_hi, id1);
+                        mma(k % 3, d1, al[k] + a_lo_off, bl[k], id1);
+                        mma(k % 3, d1, al[k], bl[k] + b_lo_off, id1);
                       }
                     }
                   } else {
@@ -608,13 +626,13 @@ resnet_tc_sweep_kernel(const SwParams p) {
                     const uint32_t bo2 = (uint32_t)wrap_at * blk16;
 #pragma unroll
                     for (int k = 0; k < 3 * NKC; ++k) {
-                      umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k], desc_hi, id1);
-                      umma_f16_lohi2<true>(tmem_u, al[k], a_hi, bl[k] + bo2, desc_hi, id2);   // (weights end far below 256 KB: no carry out of the address field)
+                      mma(k % 3, d1, al[k], bl[k], id1);
+                      mma(k % 3, tmem_u, al[k], bl[k] + bo2, id2);   // (weights end far below 256 KB: no carry out of the address field)
                       if constexpr (SPLIT) {
-                        umma_f16_lohi2<true>(d1, al[k] + a_lo_off, a_hi, bl[k], desc_hi, id1);
-                        umma_f16_lohi2<true>(tmem_u, al[k] + a_lo_off, a_hi, bl[k] + bo2, desc_hi, id2);
-                        umma_f16_lohi2<true>(d1, al[k], a_hi, bl[k] + b_lo_off, desc_hi, id1);
-                        umma_f16_lohi2<true>(tmem_u, al[k], a_hi, bl[k] + b_lo_off + bo2, desc_hi, id2);
+                        mma(k % 3, d1, al[k] + a_lo_off, bl[k], id1);
+                        mma(k % 3, tmem_u, al[k] + a_lo_off, bl[k] + bo2, id2);
+                        mma(k % 3, d1, al[k], bl[k] + b_lo_off, id1);
+                        mma(k % 3, tmem_u, al[k], bl[k] + b_lo_off + bo2, id2);
                       }
                     }
                   }
@@ -732,7 +750,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
               if (mine) {
                 const int row = it.s * 128 + q * 32 + lane;
                 ob.exists = true; ob.w = it.w; ob.s = it.s; ob.slot = esl; ob.par = epr;
-                ob.off = (row >= H || !row_ok) ? -1 : k32 ? (it.w * H + row) * 2 : it.w * H + row;
+                ob.off = (row >= H || !row_ok) ? -1 : k32 ? ((it.w * NA) * H + row) * 2 : it.w * H + row;
               }
               // step the iterator, the ring slot and the owner
               ++it.o; it.w += d;
@@ -760,24 +778,23 @@ resnet_tc_sweep_kernel(const SwParams p) {
             // this lane's row of the staged skip column: [plane][128 rows][16 B]
             const uint32_t sk_addr = sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT + (uint32_t)(q * 32 + lane) * 16u;
             constexpr uint32_t sk_plane = 2048u;
-            // k32: this lane's row, and whether its two 16-byte halves are stored swapped
-            const uint32_t swl = (uint32_t)((p.dmax + q * 32 + lane) >> 2) & 1u;
+            // k32: this lane's row, and whether the two 16-byte halves of its row of chunk kc are stored swapped
+            auto swl_of = [&](int kc) { return (uint32_t)((p.dmax + kc * H + q * 32 + lane) >> 2) & 1u; };
             const uint32_t sk_addr32 = sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT + (uint32_t)(q * 32 + lane) * 32u;
             if constexpr (HAS_SKIP) {
               // This layer READS Q (the previous layer's output), one column per step, and the MMAs of this block were
               // the last consumers of Q column w.  Nothing reads that column again before the next even layer rewrites
               // it, so its dirty lines need not ever reach HBM: discard the 128-byte lines that lie wholly inside the
-              // column (lines shared with the neighbouring columns stay).  One line per lane, planes 16 lanes apart.
+              // column (lines shared with the neighbouring columns stay).  One line per lane (k32: the column is
+              // contiguous, NKC * H * 32 B <= 96 lines), planes 16 lanes apart.
               if (p.discard_q && k32) {
-                const int t = q * 32 + lane, kc = t >> 5, j = t & 31;   // H * 32 B <= 32 lines per chunk column
-                if (kc < NKC) {
-                  const char* qb = reinterpret_cast<const char*>(bufQ);
-                  const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(qb) & 127u);
-                  const uint32_t o0 = (uint32_t)((kc * W + ob.w) * H) * 32u + mis;
-                  const uint32_t a = ((o0 + 127u) & ~127u) + (uint32_t)j * 128u;
-                  if (a + 128u <= o0 + (uint32_t)H * 32u)
-                    asm volatile("discard.global.L2 [%0], 128;" ::"l"(qb + (a - mis)) : "memory");
-                }
+                const char* qb = reinterpret_cast<const char*>(bufQ);
+                const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(qb) & 127u);
+                const uint32_t col_bytes = (uint32_t)(NKC * H) * 32u;
+                const uint32_t o0 = (uint32_t)ob.w * col_bytes + mis;
+                const uint32_t a = ((o0 + 127u) & ~127u) + (uint32_t)(q * 32 + lane) * 128u;
+                if (a + 128u <= o0 + col_bytes)
+                  asm volatile("discard.global.L2 [%0], 128;" ::"l"(qb + (a - mis)) : "memory");
               } else if (p.discard_q) {
                 const int t = q * 32 + lane, pl = t >> 4, j = t & 15;
                 if (pl < NP) {
@@ -821,6 +838,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
               }
               if (valid && !(DBG && (p.diag & 1))) {
                 uint4 ykeep = make_uint4(0u, 0u, 0u, 0u), ykeep_lo = make_uint4(0u, 0u, 0u, 0u);
+                const uint32_t swl = swl_of(jj), swl_lo = SPLIT ? swl_of(NKC + jj) : 0u;   // (SPLIT: the lo chunk's rows)
 #pragma unroll
                 for (int hf = 0; hf < 2; ++hf) {
                   float x[8], kc8[8];   // constants read at use (volatile: not hoisted into registers for the whole layer)
@@ -831,7 +849,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                   if constexpr (HAS_SKIP && SPLIT) {
                     // logical half hf of a row is stored at 16-byte slot hf ^ swl; skip = hi + lo
                     const uint4 sh = (((uint32_t)hf ^ swl) != 0u) ? skv[1] : skv[0];
-                    const uint4 sl = (((uint32_t)hf ^ swl) != 0u) ? skv[3] : skv[2];
+                    const uint4 sl = (((uint32_t)hf ^ swl_lo) != 0u) ? skv[3] : skv[2];
                     const __nv_bfloat162* ph = reinterpret_cast<const __nv_bfloat162*>(&sh);
                     const __nv_bfloat162* pl2 = reinterpret_cast<const __nv_bfloat162*>(&sl);
 #pragma unroll
@@ -843,7 +861,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                   } else if constexpr (HAS_SKIP) {
                     uint4 sv;   // 8 channels of the skip tensor at this position (plane 2 jj + hf)
                     asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(sv.x), "=r"(sv.y), "=r"(sv.z), "=r"(sv.w)
-                                 : "r"(k32 ? sk_addr32 + (uint32_t)jj * 4096u + (((uint32_t)hf ^ swl) << 4)
+                                 : "r"(k32 ? sk_addr32 + (uint32_t)(jj * H) * 32u + (((uint32_t)hf ^ swl) << 4)
                                            : sk_addr + (uint32_t)(2 * jj + hf) * sk_plane));
                     const __nv_bfloat162* pb = reinterpret_cast<const __nv_bfloat162*>(&sv);
 #pragma unroll
@@ -873,7 +891,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                       if (hf == 0) { ykeep = yo; ykeep_lo = yl; }
                       else {
                         st_hint256(y_out + jj * kc_stride + ob.off, swl ? yo : ykeep, swl ? ykeep : yo, pol_out);
-                        st_hint256(y_out + (NKC + jj) * kc_stride + ob.off, swl ? yl : ykeep_lo, swl ? ykeep_lo : yl, pol_out);
+                        st_hint256(y_out + (NKC + jj) * kc_stride + ob.off, swl_lo ? yl : ykeep_lo, swl_lo ? ykeep_lo : yl, pol_out);
                       }
                     } else if constexpr (k32) {
                       // both halves of this row's 32 bytes in ONE store (16-byte stores at a 32-byte stride would write
@@ -897,21 +915,18 @@ resnet_tc_sweep_kernel(const SwParams p) {
             pending_w = ob.w;
           };
           // Skip layers (odd l, resnet.py:51-53): the block of output column w adds column w of P.  That column is staged
-          // in this group's shared-memory slot by NP bulk copies issued by the group's quarter-0 warp as soon as all four
+          // in this group's shared-memory slot (k32: one bulk copy; planar: NP) issued by the group's quarter-0 warp as soon as all four
           // warps have finished reading the previous one, i.e. two block periods before it is needed: no L2 latency on
           // the epilogue's critical path and no prefetch registers (they hold a second accumulator set instead).
           auto stage_skip = [&](const Own& ob) {
             if constexpr (HAS_SKIP && !SPLIT) {
               asm volatile("bar.sync %0, 128;" ::"r"(2 + g) : "memory");   // the group's four warps are done with the slot
               if (k32) {
-                if (q == 0 && ob.exists && elect_one()) {   // [K chunk][128 rows][32 B]
-                  const uint32_t bytes = (uint32_t)H * 32u;
-                  mbar_expect_tx(skfull_bar(g), bytes * NKC);
-                  const uint4* src = skipP + (int64_t)ob.w * H * 2;
-                  const uint32_t d0 = sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT;
-#pragma unroll
-                  for (int kc = 0; kc < NKC; ++kc)
-                    bulk_load_hint(d0 + (uint32_t)kc * 4096u, src + kc * kc_stride, bytes, skfull_bar(g), pol_keep);
+                if (q == 0 && ob.exists && elect_one()) {   // the whole column, [K chunk][H rows][32 B]
+                  const uint32_t bytes = (uint32_t)(NKC * H) * 32u;
+                  mbar_expect_tx(skfull_bar(g), bytes);
+                  bulk_load_hint(sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT, skipP + (ob.w * NKC) * H * 2, bytes,
+                                 skfull_bar(g), pol_keep);
                 }
               } else if (q == 0 && ob.exists && elect_one()) {
                 const int rows = H - ob.s * 128 < 128 ? H - ob.s * 128 : 128;
