@@ -55,6 +55,12 @@ SIGNATURES = {
                                           C.c_size_t, C.c_void_p]),
     "kws_mfcc_stream_forward_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p,
                                                 C.c_void_p, C.c_size_t, C.c_void_p]),
+    "kws_live_state_bytes": (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "kws_live_create": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "kws_live_destroy": (None, [C.c_void_p]),
+    "kws_live_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "kws_live_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "kws_live_push_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "kws_resnet_create": (C.c_int, [C.POINTER(ResNetConfig), C.POINTER(C.c_void_p)]),
     "kws_resnet_set_weights": (C.c_int, [C.c_void_p, C.POINTER(ResNetWeights), C.c_void_p]),
     "kws_cnn_create": (C.c_int, [C.POINTER(CnnConfig), C.POINTER(C.c_void_p)]),

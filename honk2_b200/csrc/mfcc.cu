@@ -15,6 +15,7 @@
 #include <cmath>
 #include <vector>
 #include <cstring>
+#include <type_traits>
 
 namespace kws {
 
@@ -124,9 +125,8 @@ __device__ __forceinline__ void dft15(const float2 (&y)[15], float2 (&z)[15]) {
   }
 }
 
-// EDGES = false: a CTA computes 16 consecutive frames of one clip; clip b starts at wav + b * wav_stride (wav_stride = N
-// for a dense [B, N] batch, = the shift for overlapping windows of a stream).
-// EDGES = true (streaming front-end): a CTA computes the four frames of four windows that touch the reflect padding
+// EDGES = false: a CTA computes 16 consecutive frames of one clip (SRC says where the clip's samples are).
+// EDGES = true (streaming front-ends): a CTA computes the four frames of four windows that touch the reflect padding
 // (t = 0, 1, T-2, T-1); every other frame of a window is shared with the stream-level frame table.
 //
 // SMP = float: waveforms as the reference's loader hands them over (librosa float32 in [-1, 1)).  SMP = int16_t: the 16-bit
@@ -135,10 +135,95 @@ __device__ __forceinline__ void dft15(const float2 (&y)[15], float2 (&z)[15]) {
 __device__ __forceinline__ float smp_ld(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float smp_ld(const int16_t* p) { return (float)__ldg(p) * (1.f / 32768.f); }
 
-template <bool EDGES, typename SMP>
+// Sample sources of mfcc_kernel's two staging loops: where sample j of clip b comes from and where frame t of clip b
+// goes.  clip(b) is what the loops index from; ptr(w, j) addresses sample j of that clip (EDGES: of window b + wi via
+// edge_ptr).  kReflect: librosa's reflect padding at the clip edges applies in the tile loop, so it needs bounds checks.
+//
+// DenseSource: clip b is wav + b * stride (stride = N for a dense [B, N] batch, = the shift for the overlapping windows
+// of a stream); features are dense [B, T, n_mels].
+template <typename SMP>
+struct DenseSource {
+  static constexpr bool kReflect = true;
+  using Clip = const SMP*;
+  const SMP* __restrict__ wav;
+  int64_t stride;
+  __device__ __forceinline__ Clip clip(int64_t b) const { return wav + b * stride; }
+  __device__ __forceinline__ const SMP* ptr(Clip w, int j) const { return w + j; }
+  __device__ __forceinline__ const SMP* edge_ptr(Clip w, int64_t, int wi, int j) const {
+    return w + (int64_t)wi * stride + j;
+  }
+  __device__ __forceinline__ float* out_row(float* feat, int64_t b, int T, int t, int n_mels) const {
+    return feat + (b * (int64_t)T + t) * n_mels;
+  }
+};
+
+__host__ __device__ __forceinline__ int64_t floor_div(int64_t a, int64_t b) {   // b > 0
+  return a >= 0 ? a / b : -((-a + b - 1) / b);
+}
+__device__ __forceinline__ int64_t pos_mod(int64_t a, int64_t m) { const int64_t r = a % m; return r < 0 ? r + m : r; }
+
+// RingSource (live streams): stream s's samples sit in a float ring of `cap` samples (a multiple of 16, so a 16-byte
+// load at a multiple of 4 samples never straddles the wrap), sample p at ring[s][p mod cap], p counted from the
+// stream's last reset.  count[s] includes the current push of n samples; wpos[s] is the ring position of the start of
+// the push's first window (both written by live_append_kernel).  A span is a ring and the ring position of its sample
+// 0; at() takes j in [-cap, cap).
+//  EDGES = false: clip b is stream b's new frame-table rows r0 = c_old/160 - 1 ...: clip sample j is stream sample
+//                 160 r0 + j, read as is (no padding); frame t goes to frame-ring row (r0 + t) mod fcap of stream b.
+//  EDGES = true:  window slot b = (stream b / K, the push's window b % K of that stream).  A CTA's clip holds the spans
+//                 of its four slots b .. b+3, found once per CTA; features are dense [S K, T, n_mels] like DenseSource's.
+template <bool EDGES>
+struct RingSource {
+  static constexpr bool kReflect = false;
+  struct Span { const float* ring; int start; };
+  struct Slots { Span w[4]; };
+  using Clip = std::conditional_t<EDGES, Slots, Span>;
+  const float* __restrict__ ring;
+  const int64_t* __restrict__ count;
+  const int* __restrict__ wpos;
+  int cap, n, fcap, shift, K, slots;
+  __device__ __forceinline__ const float* addr(const Span& w, int j) const {
+    int p = w.start + j;
+    if (p < 0) p += cap;
+    else if (p >= cap) p -= cap;
+    return w.ring + p;
+  }
+  __device__ __forceinline__ Span slot_span(int slot) const {
+    const int s = slot / K;
+    int start = wpos[s] + (slot - s * K) * shift;   // (< 2 cap: wpos < cap, K shift = n <= cap)
+    if (start >= cap) start -= cap;
+    return {ring + (int64_t)s * cap, start};
+  }
+  __device__ __forceinline__ Clip clip(int64_t b) const {
+    if constexpr (EDGES) {
+      Slots c;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) c.w[q] = slot_span(min((int)b + q, slots - 1));   // (slots past the end: unused)
+      return c;
+    } else {
+      return {ring + b * cap, (int)pos_mod(count[b] - n - kHop, cap)};
+    }
+  }
+  __device__ __forceinline__ const float* ptr(const Span& w, int j) const { return addr(w, j); }
+  __device__ __forceinline__ const float* edge_ptr(const Slots& c, int64_t, int wi, int j) const {
+    Span w = c.w[0];
+#pragma unroll
+    for (int q = 1; q < 4; ++q)
+      if (wi == q) w = c.w[q];   // (a select: the spans stay in registers)
+    return addr(w, j);
+  }
+  __device__ __forceinline__ float* out_row(float* feat, int64_t b, int T, int t, int n_mels) const {
+    if constexpr (EDGES) {
+      return feat + (b * (int64_t)T + t) * n_mels;
+    } else {
+      const int64_t r = (count[b] - n) / kHop - 1 + t;
+      return feat + (b * (int64_t)fcap + pos_mod(r, fcap)) * n_mels;
+    }
+  }
+};
+
+template <bool EDGES, typename SMP, typename SRC = DenseSource<SMP>>
 __global__ void __launch_bounds__(kMfccThreads)
-mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, int64_t B, int N, int T,
-            int tiles_per_utt, float* __restrict__ feat) {
+mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_utt, float* __restrict__ feat) {
   constexpr int kStage = EDGES ? kEdgeStageSamples : kStageSamples;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float2* scratch = reinterpret_cast<float2*>(smem_raw);                 // [16][248]
@@ -154,7 +239,7 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
   const int tid = threadIdx.x;
   const int64_t b = EDGES ? (int64_t)blockIdx.x * 4 : blockIdx.x / tiles_per_utt;   // (EDGES: first of four windows)
   const int t0 = EDGES ? 0 : (blockIdx.x % tiles_per_utt) * kFramesPerCta;
-  const SMP* w = wav + b * wav_stride;
+  const typename SRC::Clip w = src.clip(b);
 
   if constexpr (EDGES) {
     // frame slot s = 4 * (window - b) + e, e -> frame t = 0, 1, T-2, T-1: samples [160 t - 240, +480) of its window
@@ -166,7 +251,7 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
       if (j < 0) j = -j;
       if (j >= N) j = 2 * (N - 1) - j;
       j = max(0, min(j, N - 1));
-      s_wave[i] = b + wi < B ? smp_ld(w + (int64_t)wi * wav_stride + j) : 0.f;
+      s_wave[i] = b + wi < B ? smp_ld(src.edge_ptr(w, b, wi, j)) : 0.f;
     }
   } else {
     // stage: samples [160*t0 - 240, +2880) with librosa 'reflect' padding at the clip edges; only the frames that exist
@@ -174,14 +259,16 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
     const int j0 = t0 * kHop - kNfft / 2;
     const int n_fr = min(kFramesPerCta, T - t0);
     const int n_stage = (n_fr - 1) * kHop + kNfft;
-    const bool vec = ((reinterpret_cast<uintptr_t>(w) & 15) == 0);   // (j0 is a multiple of 16 samples)
+    // (j0 is a multiple of 16 samples; a ring source is always aligned: see RingSource)
+    bool vec = true;
+    if constexpr (SRC::kReflect) vec = ((reinterpret_cast<uintptr_t>(w) & 15) == 0);
     constexpr int V = 16 / (int)sizeof(SMP);   // samples per 16-byte load (n_stage is a multiple of 8)
     if (vec) {
       for (int iv = tid; iv < n_stage / V; iv += kMfccThreads) {
         const int i = iv * V, j = j0 + i;
         float e[V];
-        if (j >= 0 && j + V - 1 < N) {
-          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(w + j));
+        if (!SRC::kReflect || (j >= 0 && j + V - 1 < N)) {
+          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(src.ptr(w, j)));
           if constexpr (sizeof(SMP) == 4) {
             e[0] = __uint_as_float(raw.x); e[1] = __uint_as_float(raw.y); e[2] = __uint_as_float(raw.z); e[3] = __uint_as_float(raw.w);
           } else {
@@ -199,7 +286,7 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
             if (jj < 0) jj = -jj;
             if (jj >= N) jj = 2 * (N - 1) - jj;
             jj = max(0, min(jj, N - 1));  // only reachable for samples of masked frames
-            e[q] = smp_ld(w + jj);
+            e[q] = smp_ld(src.ptr(w, jj));
           }
         }
 #pragma unroll
@@ -212,7 +299,7 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
         if (j < 0) j = -j;
         if (j >= N) j = 2 * (N - 1) - j;
         j = max(0, min(j, N - 1));
-        s_wave[i] = smp_ld(w + j);
+        s_wave[i] = smp_ld(src.ptr(w, j));
       }
     }
   }
@@ -295,7 +382,7 @@ mfcc_kernel(FrontendTables tb, const SMP* __restrict__ wav, int64_t wav_stride, 
 
   // ---- sparse mel filterbank, ln, x2 (reference "DCT" of a length-1 axis)
   if (t < T && b_out < B) {
-    float* out = feat + (b_out * (int64_t)T + t) * tb.n_mels;
+    float* out = src.out_row(feat, b_out, T, t, tb.n_mels);
     for (int m = l; m < tb.n_mels; m += 16) {
       const int lo = s_lo[m], cnt = s_cnt[m], off = s_off[m];
       float acc = 0.f;
@@ -316,6 +403,69 @@ mfcc_stream_gather_kernel(const V* __restrict__ S, int64_t K, int T, int m, int 
     const int64_t k = i / per_win;
     const int64_t r = i - k * per_win;   // (t - 2) * row_v + c
     feat[k * (int64_t)T * row_v + 2 * row_v + r] = __ldg(S + (k * m + 2) * (int64_t)row_v + r);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Live streams (kws_live_*): per stream a sample ring, a frame ring and a sample counter, all on the device.
+
+// Launch 1 of a push: stream s's n new samples (chunk row s) go to its sample ring, converted to float, its counter
+// advances by n, and wpos[s] receives the ring position of the push's first window, k = floor((c_old - W) / H) + 1.
+// One CTA per stream, so the counter is written only after every thread has read it.
+__device__ __forceinline__ float live_sample(float v) { return v; }
+__device__ __forceinline__ float live_sample(int16_t v) { return (float)v * (1.f / 32768.f); }
+
+template <typename SMP>
+__global__ void __launch_bounds__(128)
+live_append_kernel(const SMP* __restrict__ chunk, int n, float* __restrict__ ring, int cap, int window, int shift,
+                   int64_t* __restrict__ count, int* __restrict__ wpos) {
+  const int64_t s = blockIdx.x;
+  const int64_t c = count[s];
+  const int start = (int)(c % cap);
+  const SMP* in = chunk + s * n;
+  float* out = ring + s * cap;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    int p = start + i;
+    if (p >= cap) p -= cap;   // (n <= cap)
+    out[p] = live_sample(__ldg(in + i));
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    count[s] = c + n;
+    wpos[s] = (int)pos_mod((floor_div(c - window, shift) + 1) * shift, cap);
+  }
+}
+
+__global__ void live_reset_kernel(const int64_t* __restrict__ ids, int64_t n_ids, int64_t S, int64_t* __restrict__ count) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_ids; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t id = ids[i];
+    if (id >= 0 && id < S) count[id] = 0;
+  }
+}
+
+// Last launch of a push: window slot `slot` = (stream s, window k).  Interior frames t = 2 .. T-3 are frame-ring rows
+// (k m + t) mod fcap of stream s (m = shift / hop); a slot with k < 0 (the warm-up of a fresh stream) is all zeros.
+// One CTA per slot; the edge frames of valid slots are the edge launch's.
+template <typename V>
+__global__ void __launch_bounds__(256)
+live_gather_kernel(const V* __restrict__ frames, const int64_t* __restrict__ count, int n, int window, int shift, int K,
+                   int T, int fcap, int row_v, V* __restrict__ feat) {
+  const int64_t slot = blockIdx.x;
+  const int64_t s = slot / K;
+  const int64_t k = floor_div(count[s] - n - window, shift) + 1 + (slot - s * K);
+  const int r0 = k >= 0 ? (int)pos_mod(k * (shift / kHop), fcap) : 0;
+  const V* rows = frames + s * fcap * (int64_t)row_v;
+  V* out = feat + slot * T * (int64_t)row_v;
+  for (int i = threadIdx.x; i < T * row_v; i += blockDim.x) {
+    const int t = i / row_v, c = i - t * row_v;
+    V v{};
+    if (k >= 0) {
+      if (t < 2 || t >= T - 2) continue;
+      int r = r0 + t;
+      if (r >= fcap) r -= fcap;   // (T <= fcap)
+      v = __ldg(rows + r * (int64_t)row_v + c);
+    }
+    out[i] = v;
   }
 }
 
@@ -438,6 +588,12 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
     e = cudaFuncSetAttribute(mfcc_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes_edges);
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(mfcc_kernel<true, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes_edges);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(mfcc_kernel<false, float, RingSource<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)fe->smem_bytes);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(mfcc_kernel<true, float, RingSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)fe->smem_bytes_edges);
   if (e != cudaSuccess) {
     set_error("kws_frontend_create: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
     cudaFree(fe->dev_blob);
@@ -475,7 +631,7 @@ static int mfcc_forward_any(const char* who, const kws_frontend_t* fe, const SMP
   const int64_t blocks = B * tiles;
   KWS_REQUIRE(blocks < (int64_t)2147483647, "%s: batch too large for one launch", who);
   mfcc_kernel<false, SMP><<<(unsigned)blocks, kMfccThreads, fe->smem_bytes, as_stream(stream)>>>(
-      fe->t, wav, (int64_t)n_samples, B, n_samples, T, tiles, feat);
+      fe->t, DenseSource<SMP>{wav, (int64_t)n_samples}, B, n_samples, T, tiles, feat);
   KWS_CHECK_LAUNCH();
   return KWS_OK;
 }
@@ -517,7 +673,7 @@ static int mfcc_stream_forward_any(const kws_frontend_t* fe, const SMP* wav, int
     const int64_t blocks = n_windows * tiles;
     KWS_REQUIRE(blocks < (int64_t)2147483647, "kws_mfcc_stream_forward: too many windows for one launch");
     mfcc_kernel<false, SMP><<<(unsigned)blocks, kMfccThreads, fe->smem_bytes, st>>>(
-        fe->t, wav, (int64_t)shift, n_windows, window, T, tiles, feat);
+        fe->t, DenseSource<SMP>{wav, (int64_t)shift}, n_windows, window, T, tiles, feat);
     KWS_CHECK_LAUNCH();
     return KWS_OK;
   }
@@ -530,11 +686,11 @@ static int mfcc_stream_forward_any(const kws_frontend_t* fe, const SMP* wav, int
   float* S = static_cast<float*>(scratch);
   const int J = 1 + (int)(span / kHop);
   mfcc_kernel<false, SMP><<<(unsigned)ceil_div(J, kFramesPerCta), kMfccThreads, fe->smem_bytes, st>>>(
-      fe->t, wav, span, (int64_t)1, (int)span, J, ceil_div(J, kFramesPerCta), S);
+      fe->t, DenseSource<SMP>{wav, span}, (int64_t)1, (int)span, J, ceil_div(J, kFramesPerCta), S);
   KWS_CHECK_LAUNCH();
   // 2) the four frames per window that do (reflect padding at the WINDOW's edges, audio_processor.py:19-26 per window)
   mfcc_kernel<true, SMP><<<(unsigned)ceil_div<int64_t>(n_windows, 4), kMfccThreads, fe->smem_bytes_edges, st>>>(
-      fe->t, wav, (int64_t)shift, n_windows, window, T, 1, feat);
+      fe->t, DenseSource<SMP>{wav, (int64_t)shift}, n_windows, window, T, 1, feat);
   KWS_CHECK_LAUNCH();
   // 3) interior frames: copies of table rows
   const int m = shift / kHop;
@@ -559,4 +715,144 @@ extern "C" int kws_mfcc_stream_forward(const kws_frontend_t* fe, const float* wa
 extern "C" int kws_mfcc_stream_forward_pcm16(const kws_frontend_t* fe, const int16_t* wav, int64_t n_windows, int window,
                                              int shift, float* feat, void* scratch, size_t scratch_bytes, void* stream) {
   return mfcc_stream_forward_any<int16_t>(fe, wav, n_windows, window, shift, feat, scratch, scratch_bytes, stream);
+}
+
+// ---- live streams ---------------------------------------------------------------------------
+// One device allocation per state: sample rings [S][cap] f32, frame rings [S][fcap][n_mels] f32, counters [S] i64,
+// first-window ring positions [S] i32.
+struct kws_live {
+  const kws_frontend* fe;
+  int S, window, shift, max_push, T, cap, fcap;
+  void* dev;
+  float* ring;
+  float* frames;
+  int64_t* count;
+  int* wpos;
+};
+
+namespace {
+struct LiveLayout {
+  int T, cap, fcap;
+  size_t o_frames, o_count, o_wpos, total;
+};
+
+int live_layout(const char* who, const kws_frontend_t* fe, int S, int window, int shift, int max_push, LiveLayout* L) {
+  KWS_REQUIRE(fe != nullptr, "%s: frontend is null", who);
+  KWS_REQUIRE(S >= 1, "%s: need at least one stream (got %d)", who, S);
+  KWS_REQUIRE(shift >= 1 && shift % kHop == 0, "%s: the shift must be a positive multiple of the %d-sample hop (got %d)",
+              who, kHop, shift);
+  KWS_REQUIRE(window >= 1 && 1 + window / kHop >= 5,
+              "%s: a window of %d samples has %d frames; at least 5 are needed so that windows share frames", who,
+              window, window >= 1 ? 1 + window / kHop : 0);
+  KWS_REQUIRE(max_push >= 1 && max_push % shift == 0, "%s: max_push must be a positive multiple of the shift %d (got %d)",
+              who, shift, max_push);
+  const int64_t span = (int64_t)window + max_push;   // the oldest sample a push reads lies < window before it
+  KWS_REQUIRE(span <= (int64_t)1 << 30, "%s: window + max_push = %lld samples is too large", who, (long long)span);
+  L->T = 1 + window / kHop;
+  L->cap = (int)round_up<int64_t>(span, 16);          // 16-byte staging loads never straddle the wrap
+  L->fcap = (int)ceil_div<int64_t>(span, kHop);
+  const size_t ring = round_up<size_t>((size_t)S * L->cap * sizeof(float), 256);
+  const size_t frames = round_up<size_t>((size_t)S * L->fcap * fe->n_mels * sizeof(float), 256);
+  L->o_frames = ring;
+  L->o_count = ring + frames;
+  L->o_wpos = L->o_count + (size_t)S * sizeof(int64_t);
+  L->total = L->o_wpos + (size_t)S * sizeof(int);
+  return KWS_OK;
+}
+}  // namespace
+
+extern "C" size_t kws_live_state_bytes(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push) {
+  LiveLayout L;
+  return live_layout("kws_live_state_bytes", fe, n_streams, window, shift, max_push, &L) == KWS_OK ? L.total : 0;
+}
+
+extern "C" int kws_live_create(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push,
+                               kws_live_t** out) {
+  KWS_REQUIRE(out != nullptr, "kws_live_create: out is null");
+  *out = nullptr;
+  LiveLayout L;
+  KWS_TRY(live_layout("kws_live_create", fe, n_streams, window, shift, max_push, &L));
+  void* dev = nullptr;
+  cudaError_t e = cudaMalloc(&dev, L.total);
+  if (e == cudaSuccess) e = cudaMemset(dev, 0, L.total);   // counters start at 0; the rings' contents are never read stale
+  if (e != cudaSuccess) {                                   // by a valid window, zeroing only keeps them finite
+    set_error("kws_live_create: %zu bytes of device state: %s", L.total, cudaGetErrorString(e));
+    if (dev) cudaFree(dev);
+    return KWS_ERR_CUDA;
+  }
+  unsigned char* d = static_cast<unsigned char*>(dev);
+  *out = new kws_live{fe, n_streams, window, shift, max_push, L.T, L.cap, L.fcap, dev, reinterpret_cast<float*>(d),
+                      reinterpret_cast<float*>(d + L.o_frames), reinterpret_cast<int64_t*>(d + L.o_count),
+                      reinterpret_cast<int*>(d + L.o_wpos)};
+  return KWS_OK;
+}
+
+extern "C" void kws_live_destroy(kws_live_t* live) {
+  if (!live) return;
+  cudaFree(live->dev);
+  delete live;
+}
+
+extern "C" int kws_live_reset(kws_live_t* live, const int64_t* stream_ids, int64_t count, void* stream) {
+  KWS_REQUIRE(live != nullptr, "kws_live_reset: live state is null");
+  KWS_REQUIRE(count >= 0, "kws_live_reset: negative count");
+  if (count == 0) return KWS_OK;
+  KWS_REQUIRE(stream_ids != nullptr, "kws_live_reset: stream_ids is null");
+  const unsigned grid = (unsigned)std::min<int64_t>(ceil_div<int64_t>(count, 256), 1024);
+  live_reset_kernel<<<grid, 256, 0, as_stream(stream)>>>(stream_ids, count, live->S, live->count);
+  KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+
+template <typename SMP>
+static int live_push_any(const char* who, kws_live_t* L, const SMP* chunk, int n, float* feat, void* stream) {
+  KWS_REQUIRE(L != nullptr, "%s: live state is null", who);
+  KWS_REQUIRE(n >= 1 && n <= L->max_push && n % L->shift == 0,
+              "%s: a push of %d samples per stream: need a multiple of the shift %d in [%d, %d]", who, n, L->shift,
+              L->shift, L->max_push);
+  KWS_REQUIRE(chunk != nullptr && feat != nullptr, "%s: null buffer", who);
+  const kws_frontend* fe = L->fe;
+  cudaStream_t st = as_stream(stream);
+  const int K = n / L->shift;
+  const int64_t slots = (int64_t)L->S * K;
+  const int rows = n / kHop;
+  const int tiles = ceil_div(rows, kFramesPerCta);
+  KWS_REQUIRE(slots < (int64_t)2147483647 && (int64_t)L->S * tiles < (int64_t)2147483647,
+              "%s: too many streams for one launch", who);
+  // 1) the new samples into the sample rings; counters and first-window positions
+  live_append_kernel<SMP><<<(unsigned)L->S, 128, 0, st>>>(chunk, n, L->ring, L->cap, L->window, L->shift, L->count,
+                                                         L->wpos);
+  KWS_CHECK_LAUNCH();
+  // 2) the n / 160 frame-table rows per stream the push completes, r = c_old/160 - 1 .. c_new/160 - 2 (no padding: N
+  //    is not read)
+  mfcc_kernel<false, float, RingSource<false>><<<(unsigned)(L->S * tiles), kMfccThreads, fe->smem_bytes, st>>>(
+      fe->t, RingSource<false>{L->ring, L->count, L->wpos, L->cap, n, L->fcap, L->shift, K, (int)slots}, (int64_t)L->S, 0,
+      rows, tiles, L->frames);
+  KWS_CHECK_LAUNCH();
+  // 3) the four reflect-padded edge frames of each of the S K new windows
+  mfcc_kernel<true, float, RingSource<true>><<<(unsigned)ceil_div<int64_t>(slots, 4), kMfccThreads, fe->smem_bytes_edges,
+                                               st>>>(
+      fe->t, RingSource<true>{L->ring, L->count, L->wpos, L->cap, n, L->fcap, L->shift, K, (int)slots}, slots, L->window,
+      L->T, 1, feat);
+  KWS_CHECK_LAUNCH();
+  // 4) interior frames from the frame rings; warm-up slots zeroed
+  const bool vec = fe->n_mels % 4 == 0 && (reinterpret_cast<uintptr_t>(feat) & 15) == 0;
+  const int row_v = vec ? fe->n_mels / 4 : fe->n_mels;
+  if (vec)
+    live_gather_kernel<float4><<<(unsigned)slots, 256, 0, st>>>(reinterpret_cast<const float4*>(L->frames), L->count, n,
+                                                                L->window, L->shift, K, L->T, L->fcap, row_v,
+                                                                reinterpret_cast<float4*>(feat));
+  else
+    live_gather_kernel<float><<<(unsigned)slots, 256, 0, st>>>(L->frames, L->count, n, L->window, L->shift, K, L->T,
+                                                               L->fcap, row_v, feat);
+  KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+
+extern "C" int kws_live_push(kws_live_t* live, const float* chunk, int n, float* feat, void* stream) {
+  return live_push_any<float>("kws_live_push", live, chunk, n, feat, stream);
+}
+
+extern "C" int kws_live_push_pcm16(kws_live_t* live, const int16_t* chunk, int n, float* feat, void* stream) {
+  return live_push_any<int16_t>("kws_live_push_pcm16", live, chunk, n, feat, stream);
 }

@@ -1,10 +1,14 @@
 """Host side of the streaming-window path (SURVEY 8f-1): what ``StreamingDataset`` (dataset/dataset_utils.py:20-95)
 does around the audio, restated for a stream that is already one array -- window count, window targets -- plus
-``evaluate_stream``: features of all sliding windows from the shared-frame front-end, then the model, batch by batch.
+``evaluate_stream``: features of all sliding windows from the shared-frame front-end, then the model, batch by batch;
+and ``LiveStreams``, the same windows for many streams whose audio arrives a chunk at a time.
 """
+import ctypes as C
+
 import numpy as np
 import torch
 
+from . import _native
 from .audio_processor import AudioProcessor
 
 
@@ -84,3 +88,142 @@ def evaluate_stream(model, audio_processor, stream, window_size=16000, shift_siz
     if tgt is None:
         return out
     return out, {"correct": acc.counts()[0], "total": n}
+
+
+class LiveStreams(object):
+    """Live keyword-spotting front-end for ``n_streams`` microphones, fed a chunk at a time (``kws_live_*``).
+
+    Each stream keeps a device-resident sample ring, frame ring and sample counter.  ``push(chunk)`` hands every stream
+    the same number n of new samples (a CUDA ``[S, n]`` float32 or int16 PCM tensor; n a multiple of ``shift_size`` in
+    ``[shift_size, max_push]``) and returns the features of the K = n / shift_size window indices the push completes per
+    stream, ``[S, K, T, n_mels]``, with a host-side bool mask ``valid [S, K]``.  Window k of a stream is its samples
+    ``[k * shift_size, k * shift_size + window_size)`` since its last reset -- the windows of ``StreamingDataset`` and
+    ``compute_mfccs_stream``.  Slot j is window ``floor((c - window_size) / shift_size) + 1 + j`` for the sample count
+    c before the push, so the last slot is the newest complete window; a slot is valid iff its window index is >= 0,
+    and the features of invalid slots (the warm-up of a fresh stream) are exactly zero.  Valid features are
+    bit-identical to ``compute_mfccs_batch`` on the materialised windows.  Only the new frames are computed: n / 160
+    frame-table rows per stream and the four reflect-padded edge frames of each window.
+
+    ``samples_seen`` is the host's copy of the counters, so building the mask never synchronises with the device.
+    ``reset`` takes host ids, checks them and updates that copy; it stages them through buffers allocated with the
+    state, so neither ``push`` nor ``reset`` allocates device memory or waits for the device.  A copy made by pickling
+    holds no device state and starts every stream afresh."""
+
+    def __init__(self, audio_processor, n_streams, window_size=16000, shift_size=160, max_push=1600, device=None):
+        self.audio_processor = audio_processor   # owns the front-end tables the state reads
+        self.n_streams = int(n_streams)
+        self.window_size = int(window_size)
+        self.shift_size = int(shift_size)
+        self.max_push = int(max_push)
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev.type != "cuda":
+            raise _native.NativeError("LiveStreams needs a CUDA device: there is no CPU path")
+        self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
+        self.n_frames = audio_processor.n_frames(self.window_size)
+        self._handle = None
+        self._seen = np.zeros(self.n_streams, dtype=np.int64)
+        self._state()
+
+    def _state(self):
+        if self._handle is None:
+            lib = _native.load()
+            fe = self.audio_processor._frontend(self.device)
+            out = C.c_void_p()
+            with torch.cuda.device(self.device):
+                _native.check(lib.kws_live_create(fe, self.n_streams, self.window_size, self.shift_size, self.max_push,
+                                                  C.byref(out)), "kws_live_create")
+            self._handle = out
+            self._seen[:] = 0
+            # reset's stream ids: pinned staging buffer, device copy, and the event that marks the staging buffer free
+            self._ids_host = torch.empty(self.n_streams, dtype=torch.int64, pin_memory=True)
+            self._ids_dev = torch.empty(self.n_streams, dtype=torch.int64, device=self.device)
+            self._ids_copied = torch.cuda.Event()
+        return self._handle
+
+    @property
+    def samples_seen(self):
+        """Samples pushed into each stream since its last reset: CPU int64 [S]."""
+        return torch.from_numpy(self._seen.copy())
+
+    def state_bytes(self):
+        """Device bytes the state holds (kws_live_state_bytes)."""
+        lib = _native.load()
+        return int(lib.kws_live_state_bytes(self.audio_processor._frontend(self.device), self.n_streams,
+                                            self.window_size, self.shift_size, self.max_push))
+
+    def push(self, chunk, model=None, out=None):
+        """chunk: CUDA [S, n] float32 or int16 PCM.  Returns (features [S, K, T, n_mels], valid [S, K] CPU bool); with
+        a model, (logits [S, K, n_labels], valid) where the logits are model(features.view(S * K, T, n_mels)) on the
+        current stream.  ``out``: optional preallocated features buffer."""
+        if not (isinstance(chunk, torch.Tensor) and chunk.is_cuda):
+            raise _native.NativeError("LiveStreams.push needs a CUDA tensor: there is no CPU path")
+        if chunk.dim() != 2 or chunk.shape[0] != self.n_streams:
+            raise ValueError(f"expected a chunk shaped [{self.n_streams}, n], got {tuple(chunk.shape)}")
+        if chunk.device != self.device:
+            raise ValueError(f"the chunk is on {chunk.device}, the live state on {self.device}")
+        pcm16 = chunk.dtype == torch.int16
+        if not pcm16 and chunk.dtype != torch.float32:
+            chunk = chunk.float()
+        chunk = chunk.contiguous()
+        n = chunk.shape[1]
+        K = n // self.shift_size
+        shape = (self.n_streams, K, self.n_frames, self.audio_processor.n_mels)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        elif out.shape != shape or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 {list(shape)} tensor on {self.device}")
+        lib = _native.load()
+        handle = self._state()
+        fn = lib.kws_live_push_pcm16 if pcm16 else lib.kws_live_push
+        with torch.cuda.device(self.device):
+            _native.check(fn(handle, C.c_void_p(chunk.data_ptr()), n, C.c_void_p(out.data_ptr()),
+                             C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
+                          "kws_live_push_pcm16" if pcm16 else "kws_live_push")
+        # window index of slot j: floor((c - W) / H) + 1 + j, c = samples before this push
+        first = (self._seen - self.window_size) // self.shift_size + 1
+        valid = torch.from_numpy(first[:, None] + np.arange(K)[None, :] >= 0)
+        self._seen += n
+        if model is None:
+            return out, valid
+        logits = model(out.view(self.n_streams * K, self.n_frames, self.audio_processor.n_mels))
+        return logits.view(self.n_streams, K, -1), valid
+
+    def reset(self, stream_ids):
+        """Restart the given streams at sample 0; the others are not affected.  stream_ids: host integers (a list, a
+        numpy array or a CPU tensor) in [0, S); repeats are allowed."""
+        if isinstance(stream_ids, torch.Tensor) and stream_ids.is_cuda:
+            raise ValueError("reset takes host stream ids: the host checks them and keeps samples_seen")
+        ids = np.unique(np.asarray(stream_ids, dtype=np.int64).reshape(-1))
+        if ((ids < 0) | (ids >= self.n_streams)).any():
+            raise ValueError(f"stream ids must lie in [0, {self.n_streams})")
+        if ids.size == 0:
+            return
+        lib = _native.load()
+        handle = self._state()
+        m = ids.size
+        st = torch.cuda.current_stream(self.device)
+        self._ids_copied.synchronize()   # the previous reset's copy out of the staging buffer (long done, in practice)
+        self._ids_host[:m].copy_(torch.from_numpy(ids))
+        with torch.cuda.device(self.device):
+            self._ids_dev[:m].copy_(self._ids_host[:m], non_blocking=True)
+            self._ids_copied.record(st)
+            _native.check(lib.kws_live_reset(handle, C.c_void_p(self._ids_dev.data_ptr()), m,
+                                             C.c_void_p(st.cuda_stream)), "kws_live_reset")
+        self._seen[ids] = 0
+
+    def __del__(self):
+        try:
+            lib = _native.loaded()   # (never dlopen from a destructor)
+            if lib is not None and self._handle is not None:
+                lib.kws_live_destroy(self._handle)
+                self._handle = None
+        except Exception:
+            pass
+
+    def __getstate__(self):  # device state never crosses a process boundary
+        d = dict(self.__dict__)
+        d["_handle"] = None
+        d["_seen"] = np.zeros_like(self._seen)
+        for k in ("_ids_host", "_ids_dev", "_ids_copied"):
+            d.pop(k, None)
+        return d

@@ -82,6 +82,35 @@ int kws_mfcc_stream_forward(const kws_frontend_t* fe, const float* wav, int64_t 
 int kws_mfcc_stream_forward_pcm16(const kws_frontend_t* fe, const int16_t* wav, int64_t n_windows, int window, int shift,
                                   float* feat, void* scratch, size_t scratch_bytes, void* stream);
 
+/* Live streams: the streaming-window front-end above for S streams whose audio arrives a few milliseconds at a time.
+ * There is no reference interface: this replaces the caller's own per-stream ring buffer around compute_mfccs.
+ * A state holds, per stream, a device-resident sample ring, a ring of frame-table rows and a sample counter c_s
+ * (samples pushed since the stream's last reset).  Window k of stream s is samples [k*shift, k*shift + window) of it,
+ * the windows of StreamingDataset.__getitem__ (dataset/dataset_utils.py:72).
+ *   kws_live_state_bytes  device bytes kws_live_create allocates (0 on invalid arguments).
+ *   kws_live_create       refuses (KWS_ERR_INVALID) a shift that is not a multiple of the 160-sample hop, windows of
+ *                         fewer than 5 frames, a max_push that is not a multiple of the shift, and n_streams < 1.  The
+ *                         front-end must outlive the state.
+ *   kws_live_push         chunk [S, n] f32 holds n new samples of every stream, n a multiple of the shift in
+ *                         [shift, max_push].  It completes K = n / shift window indices per stream: slot j of stream s
+ *                         is window k = floor((c_s - window) / shift) + 1 + j, c_s counted before the push; the last
+ *                         slot is the newest complete window.  feat [S, K, T, n_mels] receives their features,
+ *                         bit-identical to kws_mfcc_forward on the materialised windows; slots with k < 0 (the warm-up
+ *                         of a fresh stream) are all zeros.  Only the n / 160 new frame-table rows per stream and the
+ *                         four reflect-padded edge frames per window are computed.
+ *   kws_live_push_pcm16   the same on int16 PCM (see kws_mfcc_forward_pcm16): bit-identical to a float push of s/32768.
+ *   kws_live_reset        stream_ids: DEVICE int64[count]; those streams restart at sample 0 (ids outside [0, S) are
+ *                         ignored).  Other streams are unaffected.
+ * Push and reset allocate nothing and do not synchronise the host; counters live on the device, so a caller that
+ * needs the validity of each slot keeps its own copy of c_s (honk2_b200.LiveStreams does). */
+typedef struct kws_live kws_live_t;
+size_t kws_live_state_bytes(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push);
+int kws_live_create(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push, kws_live_t** out);
+void kws_live_destroy(kws_live_t* live);
+int kws_live_reset(kws_live_t* live, const int64_t* stream_ids, int64_t count, void* stream);
+int kws_live_push(kws_live_t* live, const float* chunk, int n, float* feat, void* stream);
+int kws_live_push_pcm16(kws_live_t* live, const int16_t* chunk, int n, float* feat, void* stream);
+
 /* ---- models: replace model.ResNet / model.CNN ---------------------------------------------
  * kws_resnet_create <- ResNet.__init__ (model/resnet.py:11-36); pool_h = pool_w = 0 when the
  *                      config has no "pool" key.
