@@ -61,6 +61,11 @@ SIGNATURES = {
     "kws_live_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "kws_live_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "kws_live_push_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "kws_live_ragged_workspace_bytes": (C.c_size_t, [C.c_void_p]),
+    "kws_live_push_ragged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "kws_live_push_ragged_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "kws_resnet_create": (C.c_int, [C.POINTER(ResNetConfig), C.POINTER(C.c_void_p)]),
     "kws_resnet_set_weights": (C.c_int, [C.c_void_p, C.POINTER(ResNetWeights), C.c_void_p]),
     "kws_cnn_create": (C.c_int, [C.POINTER(CnnConfig), C.POINTER(C.c_void_p)]),

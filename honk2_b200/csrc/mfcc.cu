@@ -12,6 +12,7 @@
 // A warp works on two frames at a time (one per half-warp); a CTA stages the 2880 samples its
 // 16 frames cover once (coalesced loads, reflect indexing at the clip edges).
 #include "common.cuh"
+#include <cub/device/device_scan.cuh>
 #include <cmath>
 #include <vector>
 #include <cstring>
@@ -138,12 +139,14 @@ __device__ __forceinline__ float smp_ld(const int16_t* p) { return (float)__ldg(
 // Sample sources of mfcc_kernel's two staging loops: where sample j of clip b comes from and where frame t of clip b
 // goes.  clip(b) is what the loops index from; ptr(w, j) addresses sample j of that clip (EDGES: of window b + wi via
 // edge_ptr).  kReflect: librosa's reflect padding at the clip edges applies in the tile loop, so it needs bounds checks.
+// kRagged: the number of entries lives on the device (entries()), and CTAs past it exit.  kPacked: a CTA computes 16
+// single frames from anywhere (frame_ptr / frame_out), each staged from its own 480 samples like the edge frames.
 //
 // DenseSource: clip b is wav + b * stride (stride = N for a dense [B, N] batch, = the shift for the overlapping windows
 // of a stream); features are dense [B, T, n_mels].
 template <typename SMP>
 struct DenseSource {
-  static constexpr bool kReflect = true;
+  static constexpr bool kReflect = true, kRagged = false, kPacked = false;
   using Clip = const SMP*;
   const SMP* __restrict__ wav;
   int64_t stride;
@@ -161,6 +164,14 @@ __host__ __device__ __forceinline__ int64_t floor_div(int64_t a, int64_t b) {   
   return a >= 0 ? a / b : -((-a + b - 1) / b);
 }
 __device__ __forceinline__ int64_t pos_mod(int64_t a, int64_t m) { const int64_t r = a % m; return r < 0 ? r + m : r; }
+// At sample count c of a live stream: the last complete frame-table row (row r covers samples [160 r - 240, +480)),
+// and the number of complete windows (window k covers [k shift, k shift + window)).  A push from c to c' completes rows
+// ragged_rows(c) + 1 .. ragged_rows(c') and windows ragged_wins(c) .. ragged_wins(c') - 1.
+__device__ __forceinline__ int64_t ragged_rows(int64_t c) { return floor_div(c - kNfft / 2, kHop); }
+__device__ __forceinline__ int64_t ragged_wins(int64_t c, int window, int shift) {
+  const int64_t k = floor_div(c - window, shift) + 1;
+  return k > 0 ? k : 0;
+}
 
 // RingSource (live streams): stream s's samples sit in a float ring of `cap` samples (a multiple of 16, so a 16-byte
 // load at a multiple of 4 samples never straddles the wrap), sample p at ring[s][p mod cap], p counted from the
@@ -173,7 +184,7 @@ __device__ __forceinline__ int64_t pos_mod(int64_t a, int64_t m) { const int64_t
 //                 of its four slots b .. b+3, found once per CTA; features are dense [S K, T, n_mels] like DenseSource's.
 template <bool EDGES>
 struct RingSource {
-  static constexpr bool kReflect = false;
+  static constexpr bool kReflect = false, kRagged = false, kPacked = false;
   struct Span { const float* ring; int start; };
   struct Slots { Span w[4]; };
   using Clip = std::conditional_t<EDGES, Slots, Span>;
@@ -221,10 +232,95 @@ struct RingSource {
   }
 };
 
+// RaggedSource (ragged pushes): entries of two compacted lists ordered by stream, each stream with its own count.
+// plan[s] (s = 0 .. S) is the exclusive scan of the per-stream counts of the push, new frame-table rows in the high 32
+// bits and completed windows in the low 32 bits (both totals < 2^31, checked on the host): plan[S] holds the totals.  An
+// entry's stream is a binary search over plan, done once per entry by the first threads of the CTA into a shared table
+// (clip() holds one barrier, so every thread calls it).  count[s] already includes the push's len[s] samples.
+//  EDGES = false (kPacked): row entry e = (stream s, row r = floor((c_old - 240) / 160) + 1 + e - plan_rows[s]); frame t
+//                 of the CTA is entry 16 b + t: ring samples 160 r - 240 + [0, 480) (a multiple of 16 samples from the
+//                 ring start, so 16-byte loads), written to row r mod fcap of stream s's frame ring.
+//  EDGES = true:  window entry b = (stream s, window k = max(0, floor((c_old - W) / H) + 1) + b - plan_wins[s]): the
+//                 spans of RingSource<true>, features dense [M, T, n_mels].
+template <bool EDGES>
+struct RaggedSource {
+  static constexpr bool kReflect = false, kRagged = true, kPacked = !EDGES;
+  using Span = RingSource<true>::Span;
+  using Slots = RingSource<true>::Slots;
+  struct Row { Span in; float* out; };
+  using Clip = std::conditional_t<EDGES, Slots, const Row*>;
+  const float* __restrict__ ring;
+  float* frames;
+  const int64_t* __restrict__ count;
+  const int* __restrict__ len;
+  const int64_t* __restrict__ plan;
+  int S, cap, fcap, n_mels, window, shift;
+  __device__ __forceinline__ int64_t field(int64_t p) const { return EDGES ? (p & 0xffffffffll) : (p >> 32); }
+  __device__ __forceinline__ int64_t entries() const { return field(__ldg(plan + S)); }
+  // stream of entry e (< entries()) and the entries of the streams before it
+  __device__ __forceinline__ int stream_of(int64_t e, int64_t* before) const {
+    int lo = 0, hi = S;   // field(plan[lo]) <= e < field(plan[hi])
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (field(__ldg(plan + mid)) <= e) lo = mid;
+      else hi = mid;
+    }
+    *before = field(__ldg(plan + lo));
+    return lo;
+  }
+  __device__ __forceinline__ const float* addr(const Span& w, int j) const {
+    int p = w.start + j;
+    if (p < 0) p += cap;
+    else if (p >= cap) p -= cap;
+    return w.ring + p;
+  }
+  __device__ __forceinline__ Clip clip(int64_t b) const {
+    const int64_t last = entries() - 1;
+    constexpr int kEntries = EDGES ? 4 : kFramesPerCta;
+    __shared__ std::conditional_t<EDGES, Span, Row> tab[kEntries];
+    if (threadIdx.x < kEntries) {
+      const int64_t e = min(b + (int64_t)threadIdx.x, last);   // (entries past the end: unused)
+      int64_t before;
+      const int s = stream_of(e, &before);
+      const int64_t c_old = __ldg(count + s) - __ldg(len + s);
+      if constexpr (EDGES) {
+        const int64_t k = ragged_wins(c_old, window, shift) + (e - before);
+        tab[threadIdx.x] = Span{ring + (int64_t)s * cap, (int)pos_mod(k * shift, cap)};
+      } else {
+        const int64_t r = ragged_rows(c_old) + 1 + (e - before);
+        tab[threadIdx.x] = Row{Span{ring + (int64_t)s * cap, (int)pos_mod(r * kHop - kNfft / 2, cap)},
+                               frames + ((int64_t)s * fcap + pos_mod(r, fcap)) * n_mels};
+      }
+    }
+    __syncthreads();
+    if constexpr (EDGES) {
+      Slots c;
+#pragma unroll
+      for (int q = 0; q < 4; ++q) c.w[q] = tab[q];
+      return c;
+    } else {
+      return tab;
+    }
+  }
+  __device__ __forceinline__ const float* edge_ptr(const Slots& c, int64_t, int wi, int j) const {
+    Span w = c.w[0];
+#pragma unroll
+    for (int q = 1; q < 4; ++q)
+      if (wi == q) w = c.w[q];
+    return addr(w, j);
+  }
+  __device__ __forceinline__ const float* frame_ptr(const Row* c, int slot, int j) const { return addr(c[slot].in, j); }
+  __device__ __forceinline__ float* frame_out(const Row* c, int slot) const { return c[slot].out; }
+  __device__ __forceinline__ float* out_row(float* feat, int64_t b, int T, int t, int n_mels) const {
+    return feat + (b * (int64_t)T + t) * n_mels;
+  }
+};
+
 template <bool EDGES, typename SMP, typename SRC = DenseSource<SMP>>
 __global__ void __launch_bounds__(kMfccThreads)
 mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_utt, float* __restrict__ feat) {
-  constexpr int kStage = EDGES ? kEdgeStageSamples : kStageSamples;
+  constexpr bool kPacked = SRC::kPacked;   // (T = 16: frame t of the CTA is entry 16 b + t)
+  constexpr int kStage = EDGES || kPacked ? kEdgeStageSamples : kStageSamples;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float2* scratch = reinterpret_cast<float2*>(smem_raw);                 // [16][248]
   float2* s_tw240 = scratch + kFramesPerCta * kScStride;                 // [16][16]
@@ -237,11 +333,24 @@ mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_u
   float* s_w = reinterpret_cast<float*>(s_off + kMaxMels);               // [nnz]
 
   const int tid = threadIdx.x;
-  const int64_t b = EDGES ? (int64_t)blockIdx.x * 4 : blockIdx.x / tiles_per_utt;   // (EDGES: first of four windows)
-  const int t0 = EDGES ? 0 : (blockIdx.x % tiles_per_utt) * kFramesPerCta;
+  const int64_t b = EDGES ? (int64_t)blockIdx.x * 4                                  // (EDGES: first of four windows)
+                          : kPacked ? (int64_t)blockIdx.x * kFramesPerCta : blockIdx.x / tiles_per_utt;
+  const int t0 = EDGES || kPacked ? 0 : (blockIdx.x % tiles_per_utt) * kFramesPerCta;
+  if constexpr (SRC::kRagged) {
+    B = src.entries();   // (the grid covers the host's bound)
+    if (b >= B) return;
+  }
   const typename SRC::Clip w = src.clip(b);
 
-  if constexpr (EDGES) {
+  if constexpr (kPacked) {
+    // frame slot s: samples [0, 480) of entry b + s's span, 16 bytes at a time (span starts are multiples of 16 samples)
+    for (int iv = tid; iv < kEdgeStageSamples / 4; iv += kMfccThreads) {
+      const int slot = iv / (kNfft / 4), n = (iv - slot * (kNfft / 4)) * 4;
+      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (b + slot < B) v = __ldg(reinterpret_cast<const float4*>(src.frame_ptr(w, slot, n)));
+      *reinterpret_cast<float4*>(s_wave + slot * kNfft + n) = v;
+    }
+  } else if constexpr (EDGES) {
     // frame slot s = 4 * (window - b) + e, e -> frame t = 0, 1, T-2, T-1: samples [160 t - 240, +480) of its window
     for (int i = tid; i < kEdgeStageSamples; i += kMfccThreads) {
       const int slot = i / kNfft, n = i - slot * kNfft;
@@ -320,7 +429,7 @@ mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_u
   // (whole warps without a frame -- the tail of a clip's last tile -- are done: only __syncwarp from here on)
   if (!EDGES && t0 + 2 * warp >= T) return;
   float2* sc = scratch + t_local * kScStride;
-  const float* fr = s_wave + (EDGES ? kNfft : kHop) * t_local;
+  const float* fr = s_wave + (EDGES || kPacked ? kNfft : kHop) * t_local;
 
   // ---- stage A: 15 radix-16 FFTs over n1 (lane = n2), twiddle by W240^(n2 k1)
   if (l < 15) {
@@ -381,8 +490,10 @@ mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_u
   __syncwarp();
 
   // ---- sparse mel filterbank, ln, x2 (reference "DCT" of a length-1 axis)
-  if (t < T && b_out < B) {
-    float* out = src.out_row(feat, b_out, T, t, tb.n_mels);
+  if (kPacked ? b + t_local < B : t < T && b_out < B) {
+    float* out;
+    if constexpr (kPacked) out = src.frame_out(w, t_local);
+    else out = src.out_row(feat, b_out, T, t, tb.n_mels);
     for (int m = l; m < tb.n_mels; m += 16) {
       const int lo = s_lo[m], cnt = s_cnt[m], off = s_off[m];
       float acc = 0.f;
@@ -466,6 +577,72 @@ live_gather_kernel(const V* __restrict__ frames, const int64_t* __restrict__ cou
       v = __ldg(rows + r * (int64_t)row_v + c);
     }
     out[i] = v;
+  }
+}
+
+// Ragged pushes.  Launch 1: stream s's len[s] new samples (samples + off[s]) go to its ring, its counter advances, and
+// counts[s] receives the push's plan for s: new frame-table rows (high word) and completed windows (low word), from the
+// counts before and after.  counts[S] = 0, so that the exclusive scan of counts[0 .. S] ends in the totals.
+
+template <typename SMP>
+__global__ void __launch_bounds__(128)
+live_ragged_append_kernel(const SMP* __restrict__ samples, const int64_t* __restrict__ off, const int* __restrict__ len,
+                          float* __restrict__ ring, int cap, int window, int shift, int S, int64_t* __restrict__ count,
+                          int64_t* __restrict__ counts) {
+  const int64_t s = blockIdx.x;
+  const int n = len[s];
+  const int64_t c = count[s];
+  const int start = (int)(c % cap);
+  const SMP* in = samples + off[s];
+  float* out = ring + s * cap;
+  for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    int p = start + i;
+    if (p >= cap) p -= cap;   // (n <= max_push < cap)
+    out[p] = live_sample(__ldg(in + i));
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    count[s] = c + n;
+    const int64_t rows = ragged_rows(c + n) - ragged_rows(c);
+    const int64_t wins = ragged_wins(c + n, window, shift) - ragged_wins(c, window, shift);
+    counts[s] = rows << 32 | wins;
+    if (s == 0) counts[S] = 0;
+  }
+}
+
+// Last launch: window entry i (stream s, window k; see RaggedSource<true>): interior frames t = 2 .. T-3 are frame-ring
+// rows (k m + t) mod fcap of stream s.  One CTA per entry of the host's bound; CTAs past the device's count exit.
+template <typename V>
+__global__ void __launch_bounds__(256)
+live_ragged_gather_kernel(const V* __restrict__ frames, const int64_t* __restrict__ count, const int* __restrict__ len,
+                          const int64_t* __restrict__ plan, int S, int window, int shift, int T, int fcap, int row_v,
+                          V* __restrict__ feat, int64_t* __restrict__ win_stream, int64_t* __restrict__ win_index,
+                          int64_t* __restrict__ n_windows) {
+  const int64_t i = blockIdx.x;
+  const int64_t M = __ldg(plan + S) & 0xffffffffll;
+  if (i == 0 && threadIdx.x == 0 && n_windows) *n_windows = M;
+  if (i >= M) return;
+  int lo = 0, hi = S;   // (plan[lo] <= i < plan[hi] in the low words)
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if ((__ldg(plan + mid) & 0xffffffffll) <= i) lo = mid;
+    else hi = mid;
+  }
+  const int64_t s = lo;
+  const int64_t k = ragged_wins(__ldg(count + s) - __ldg(len + s), window, shift) + i -
+                    (__ldg(plan + s) & 0xffffffffll);
+  if (threadIdx.x == 0) {
+    if (win_stream) win_stream[i] = s;
+    if (win_index) win_index[i] = k;
+  }
+  const int r0 = (int)pos_mod(k * (shift / kHop), fcap);
+  const V* rows = frames + s * fcap * (int64_t)row_v;
+  V* out = feat + i * T * (int64_t)row_v;
+  for (int j = threadIdx.x; j < (T - 4) * row_v; j += blockDim.x) {
+    const int t = 2 + j / row_v, c = j - (t - 2) * row_v;
+    int r = r0 + t;
+    if (r >= fcap) r -= fcap;   // (T <= fcap)
+    out[t * row_v + c] = __ldg(rows + r * (int64_t)row_v + c);
   }
 }
 
@@ -594,6 +771,12 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
   if (e == cudaSuccess)
     e = cudaFuncSetAttribute(mfcc_kernel<true, float, RingSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)fe->smem_bytes_edges);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(mfcc_kernel<false, float, RaggedSource<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)fe->smem_bytes_edges);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(mfcc_kernel<true, float, RaggedSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)fe->smem_bytes_edges);
   if (e != cudaSuccess) {
     set_error("kws_frontend_create: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
     cudaFree(fe->dev_blob);
@@ -719,7 +902,8 @@ extern "C" int kws_mfcc_stream_forward_pcm16(const kws_frontend_t* fe, const int
 
 // ---- live streams ---------------------------------------------------------------------------
 // One device allocation per state: sample rings [S][cap] f32, frame rings [S][fcap][n_mels] f32, counters [S] i64,
-// first-window ring positions [S] i32.
+// first-window ring positions [S] i32.  Ragged pushes add a pinned host staging buffer for their per-stream sample
+// offsets and lengths and the event that marks its last copy done; both are created by the first ragged push.
 struct kws_live {
   const kws_frontend* fe;
   int S, window, shift, max_push, T, cap, fcap;
@@ -728,6 +912,8 @@ struct kws_live {
   float* frames;
   int64_t* count;
   int* wpos;
+  void* ragged_host = nullptr;
+  cudaEvent_t ragged_copied = nullptr;
 };
 
 namespace {
@@ -790,6 +976,8 @@ extern "C" int kws_live_create(const kws_frontend_t* fe, int n_streams, int wind
 extern "C" void kws_live_destroy(kws_live_t* live) {
   if (!live) return;
   cudaFree(live->dev);
+  if (live->ragged_copied) cudaEventDestroy(live->ragged_copied);
+  if (live->ragged_host) cudaFreeHost(live->ragged_host);
   delete live;
 }
 
@@ -855,4 +1043,138 @@ extern "C" int kws_live_push(kws_live_t* live, const float* chunk, int n, float*
 
 extern "C" int kws_live_push_pcm16(kws_live_t* live, const int16_t* chunk, int n, float* feat, void* stream) {
   return live_push_any<int16_t>("kws_live_push_pcm16", live, chunk, n, feat, stream);
+}
+
+// ---- ragged pushes --------------------------------------------------------------------------
+// Workspace: per-stream sample offsets i64[S] and lengths i32[S] (one copy from the pinned staging buffer), the plan
+// counts i64[S+1], their exclusive scan i64[S+1], and CUB's scan scratch.
+namespace {
+struct RaggedLayout {
+  size_t o_len, o_counts, o_plan, o_temp, total;
+};
+
+int ragged_layout(const char* who, const kws_live* L, RaggedLayout* R) {
+  const size_t S = (size_t)L->S;
+  R->o_len = S * sizeof(int64_t);
+  R->o_counts = round_up<size_t>(R->o_len + S * sizeof(int32_t), 256);
+  R->o_plan = R->o_counts + round_up<size_t>((S + 1) * sizeof(int64_t), 256);
+  R->o_temp = R->o_plan + round_up<size_t>((S + 1) * sizeof(int64_t), 256);
+  size_t temp = 0;
+  const cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, temp, static_cast<int64_t*>(nullptr),
+                                                      static_cast<int64_t*>(nullptr), L->S + 1);
+  if (e != cudaSuccess) {
+    set_error("%s: scan size query failed: %s", who, cudaGetErrorString(e));
+    return KWS_ERR_CUDA;
+  }
+  R->total = R->o_temp + temp;
+  return KWS_OK;
+}
+}  // namespace
+
+extern "C" size_t kws_live_ragged_workspace_bytes(const kws_live_t* live) {
+  RaggedLayout R;
+  return live && ragged_layout("kws_live_ragged_workspace_bytes", live, &R) == KWS_OK ? R.total : 0;
+}
+
+template <typename SMP>
+static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* samples, const int32_t* lengths, float* feat,
+                                int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                void* workspace, size_t ws_bytes, void* stream) {
+  KWS_REQUIRE(L != nullptr, "%s: live state is null", who);
+  KWS_REQUIRE(lengths != nullptr, "%s: lengths is null", who);
+  // the whole plan is checked on the host, before anything is staged or launched
+  int64_t n_samples = 0, row_bound = 0, win_bound = 0;
+  for (int s = 0; s < L->S; ++s) {
+    const int n = lengths[s];
+    KWS_REQUIRE(n >= 0 && n <= L->max_push, "%s: stream %d brings %d samples; a push takes 0 to max_push = %d", who, s,
+                n, L->max_push);
+    n_samples += n;
+    row_bound += ceil_div(n, kHop);
+    win_bound += ceil_div(n, L->shift);
+  }
+  KWS_REQUIRE(row_bound < INT32_MAX && win_bound < INT32_MAX, "%s: too many new rows or windows for one launch", who);
+  KWS_REQUIRE(capacity >= win_bound,
+              "%s: the push can complete up to %lld windows (sum of ceil(length / shift)); capacity is %lld", who,
+              (long long)win_bound, (long long)capacity);
+  KWS_REQUIRE(n_samples == 0 || samples != nullptr, "%s: samples is null", who);
+  KWS_REQUIRE(win_bound == 0 || feat != nullptr, "%s: feat is null", who);
+  RaggedLayout R;
+  KWS_TRY(ragged_layout(who, L, &R));
+  KWS_REQUIRE(workspace != nullptr && ws_bytes >= R.total, "%s: needs %zu bytes of workspace, got %zu", who, R.total,
+              workspace ? ws_bytes : (size_t)0);
+  cudaStream_t st = as_stream(stream);
+  const size_t stage_bytes = R.o_len + (size_t)L->S * sizeof(int32_t);
+  if (!L->ragged_host) {
+    KWS_CUDA(cudaMallocHost(&L->ragged_host, stage_bytes));
+    KWS_CUDA(cudaEventCreateWithFlags(&L->ragged_copied, cudaEventDisableTiming));
+  } else {
+    KWS_CUDA(cudaEventSynchronize(L->ragged_copied));   // the previous ragged push's copy out of the staging buffer
+  }
+  int64_t* off_h = static_cast<int64_t*>(L->ragged_host);
+  int32_t* len_h = reinterpret_cast<int32_t*>(off_h + L->S);
+  for (int64_t s = 0, o = 0; s < L->S; o += lengths[s], ++s) {
+    off_h[s] = o;
+    len_h[s] = lengths[s];
+  }
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  const int64_t* off = reinterpret_cast<const int64_t*>(ws);
+  const int* len = reinterpret_cast<const int*>(ws + R.o_len);
+  int64_t* counts = reinterpret_cast<int64_t*>(ws + R.o_counts);
+  int64_t* plan = reinterpret_cast<int64_t*>(ws + R.o_plan);
+  KWS_CUDA(cudaMemcpyAsync(ws, L->ragged_host, stage_bytes, cudaMemcpyHostToDevice, st));
+  KWS_CUDA(cudaEventRecord(L->ragged_copied, st));
+  const kws_frontend* fe = L->fe;
+  // 1) the new samples into the sample rings; counters; per-stream counts of new rows and windows
+  live_ragged_append_kernel<SMP><<<(unsigned)L->S, 128, 0, st>>>(samples, off, len, L->ring, L->cap, L->window,
+                                                                 L->shift, L->S, L->count, counts);
+  KWS_CHECK_LAUNCH();
+  // the plan: where each stream's rows and windows start in the compacted lists, and the totals
+  size_t temp = R.total - R.o_temp;
+  KWS_CUDA(cub::DeviceScan::ExclusiveSum(ws + R.o_temp, temp, counts, plan, L->S + 1, st));
+  // 2) the new frame-table rows, 16 entries of the compacted list per CTA, from any streams
+  const RaggedSource<false> rows{L->ring, L->frames, L->count, len, plan, L->S, L->cap, L->fcap, fe->n_mels, L->window,
+                                 L->shift};
+  if (row_bound > 0) {
+    mfcc_kernel<false, float, RaggedSource<false>><<<(unsigned)ceil_div<int64_t>(row_bound, kFramesPerCta),
+                                                     kMfccThreads, fe->smem_bytes_edges, st>>>(
+        fe->t, rows, row_bound, 0, kFramesPerCta, 1, nullptr);
+    KWS_CHECK_LAUNCH();
+  }
+  // 3) the four reflect-padded edge frames of each completed window, four windows per CTA
+  if (win_bound > 0) {
+    const RaggedSource<true> edges{L->ring, L->frames, L->count, len, plan, L->S, L->cap, L->fcap, fe->n_mels,
+                                   L->window, L->shift};
+    mfcc_kernel<true, float, RaggedSource<true>><<<(unsigned)ceil_div<int64_t>(win_bound, 4), kMfccThreads,
+                                                   fe->smem_bytes_edges, st>>>(fe->t, edges, win_bound, L->window,
+                                                                               L->T, 1, feat);
+    KWS_CHECK_LAUNCH();
+  }
+  // 4) interior frames from the frame rings, the window ids, and the count (one CTA even when no window completes)
+  const bool vec = fe->n_mels % 4 == 0 && (reinterpret_cast<uintptr_t>(feat) & 15) == 0;
+  const int row_v = vec ? fe->n_mels / 4 : fe->n_mels;
+  const unsigned grid = (unsigned)std::max<int64_t>(win_bound, 1);
+  if (vec)
+    live_ragged_gather_kernel<float4><<<grid, 256, 0, st>>>(reinterpret_cast<const float4*>(L->frames), L->count, len,
+                                                            plan, L->S, L->window, L->shift, L->T, L->fcap, row_v,
+                                                            reinterpret_cast<float4*>(feat), win_stream, win_index,
+                                                            n_windows);
+  else
+    live_ragged_gather_kernel<float><<<grid, 256, 0, st>>>(L->frames, L->count, len, plan, L->S, L->window, L->shift,
+                                                           L->T, L->fcap, row_v, feat, win_stream, win_index, n_windows);
+  KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+
+extern "C" int kws_live_push_ragged(kws_live_t* live, const float* samples, const int32_t* lengths, float* feat,
+                                    int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                    void* workspace, size_t ws_bytes, void* stream) {
+  return live_push_ragged_any<float>("kws_live_push_ragged", live, samples, lengths, feat, win_stream, win_index,
+                                     capacity, n_windows, workspace, ws_bytes, stream);
+}
+
+extern "C" int kws_live_push_ragged_pcm16(kws_live_t* live, const int16_t* samples, const int32_t* lengths, float* feat,
+                                          int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                          void* workspace, size_t ws_bytes, void* stream) {
+  return live_push_ragged_any<int16_t>("kws_live_push_ragged_pcm16", live, samples, lengths, feat, win_stream,
+                                       win_index, capacity, n_windows, workspace, ws_bytes, stream);
 }

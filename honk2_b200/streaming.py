@@ -3,6 +3,7 @@ does around the audio, restated for a stream that is already one array -- window
 ``evaluate_stream``: features of all sliding windows from the shared-frame front-end, then the model, batch by batch;
 and ``LiveStreams``, the same windows for many streams whose audio arrives a chunk at a time.
 """
+import collections
 import ctypes as C
 
 import numpy as np
@@ -90,6 +91,25 @@ def evaluate_stream(model, audio_processor, stream, window_size=16000, shift_siz
     return out, {"correct": acc.counts()[0], "total": n}
 
 
+RaggedPlan = collections.namedtuple("RaggedPlan", "stream_ids window_ids row_bound window_bound")
+
+
+def ragged_push_plan(seen, lengths, window_size, shift_size):
+    """Host plan of a ragged push (``LiveStreams.push_ragged``, ``kws_live_push_ragged``): stream s has seen ``seen[s]``
+    samples and brings ``lengths[s]`` more.  It completes windows k with
+    ``max(0, floor((seen - W) / H) + 1) <= k <= floor((seen + n - W) / H)``; returns their ``stream_ids`` and
+    ``window_ids`` (int64, ordered by stream, then window), and the bounds the library sizes its launches with:
+    ``row_bound = sum(ceil(n / 160))`` new frame-table rows and ``window_bound = sum(ceil(n / H))`` windows."""
+    seen = np.asarray(seen, dtype=np.int64)
+    n = np.asarray(lengths, dtype=np.int64)
+    first = np.maximum(0, (seen - window_size) // shift_size + 1)
+    count = np.maximum(0, (seen + n - window_size) // shift_size + 1 - first)
+    stream_ids = np.repeat(np.arange(seen.size, dtype=np.int64), count)
+    starts = np.cumsum(count) - count                   # each stream's first row in the compacted list
+    window_ids = np.arange(stream_ids.size, dtype=np.int64) - np.repeat(starts - first, count)
+    return RaggedPlan(stream_ids, window_ids, int((-(-n // 160)).sum()), int((-(-n // shift_size)).sum()))
+
+
 class LiveStreams(object):
     """Live keyword-spotting front-end for ``n_streams`` microphones, fed a chunk at a time (``kws_live_*``).
 
@@ -107,7 +127,10 @@ class LiveStreams(object):
     ``samples_seen`` is the host's copy of the counters, so building the mask never synchronises with the device.
     ``reset`` takes host ids, checks them and updates that copy; it stages them through buffers allocated with the
     state, so neither ``push`` nor ``reset`` allocates device memory or waits for the device.  A copy made by pickling
-    holds no device state and starts every stream afresh."""
+    holds no device state and starts every stream afresh.
+
+    ``push_ragged(samples, lengths)`` lets every stream bring its own number of samples, and returns only the windows
+    the push completes, compacted, with the stream and window index of each (see ``ragged_push_plan``)."""
 
     def __init__(self, audio_processor, n_streams, window_size=16000, shift_size=160, max_push=1600, device=None):
         self.audio_processor = audio_processor   # owns the front-end tables the state reads
@@ -121,6 +144,7 @@ class LiveStreams(object):
         self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
         self.n_frames = audio_processor.n_frames(self.window_size)
         self._handle = None
+        self._ragged_ws = None   # device workspace of push_ragged, allocated by the first ragged push
         self._seen = np.zeros(self.n_streams, dtype=np.int64)
         self._state()
 
@@ -154,13 +178,22 @@ class LiveStreams(object):
     def push(self, chunk, model=None, out=None):
         """chunk: CUDA [S, n] float32 or int16 PCM.  Returns (features [S, K, T, n_mels], valid [S, K] CPU bool); with
         a model, (logits [S, K, n_labels], valid) where the logits are model(features.view(S * K, T, n_mels)) on the
-        current stream.  ``out``: optional preallocated features buffer."""
+        current stream.  ``out``: optional preallocated features buffer.
+
+        Every stream's sample count must be a multiple of 160 (the hop).  Only ``push_ragged`` can break that; after a
+        ragged push that leaves a count unaligned, ``push`` raises ValueError and changes nothing, until ragged pushes
+        (or a reset) realign the counts."""
         if not (isinstance(chunk, torch.Tensor) and chunk.is_cuda):
             raise _native.NativeError("LiveStreams.push needs a CUDA tensor: there is no CPU path")
         if chunk.dim() != 2 or chunk.shape[0] != self.n_streams:
             raise ValueError(f"expected a chunk shaped [{self.n_streams}, n], got {tuple(chunk.shape)}")
         if chunk.device != self.device:
             raise ValueError(f"the chunk is on {chunk.device}, the live state on {self.device}")
+        misaligned = np.flatnonzero(self._seen % 160)
+        if misaligned.size:
+            s = int(misaligned[0])
+            raise ValueError(f"stream {s} has seen {int(self._seen[s])} samples, not a multiple of the 160-sample hop "
+                             "(a ragged push left it so); push needs aligned counts: use push_ragged")
         pcm16 = chunk.dtype == torch.int16
         if not pcm16 and chunk.dtype != torch.float32:
             chunk = chunk.float()
@@ -187,6 +220,69 @@ class LiveStreams(object):
             return out, valid
         logits = model(out.view(self.n_streams * K, self.n_frames, self.audio_processor.n_mels))
         return logits.view(self.n_streams, K, -1), valid
+
+    def push_ragged(self, samples, lengths, model=None, out=None):
+        """Stream s brings ``lengths[s]`` new samples, any number in ``[0, max_push]``.
+
+        samples: 1-D CUDA float32 or int16 PCM tensor, all streams' new samples back to back in stream order
+        (``sum(lengths)`` of them).  lengths: host sequence of S ints.  Returns ``(features [M, T, n_mels],
+        stream_ids [M], window_ids [M])`` for the M windows the push completes, ordered by stream, then window; the ids
+        are CPU int64 from the host's copy of the counters (``ragged_push_plan``), so nothing waits for the device.
+        With a model, ``(logits [M, n_labels], stream_ids, window_ids)``, the logits being ``model(features)`` on the
+        current stream; when M = 0 the samples are still pushed, the model is not called and the tensors are empty.
+        ``out``: optional preallocated contiguous float32 features buffer of at least ``sum(ceil(n / shift_size))``
+        rows (which bounds M); the features are its first M rows."""
+        if not (isinstance(samples, torch.Tensor) and samples.is_cuda):
+            raise _native.NativeError("LiveStreams.push_ragged needs a CUDA tensor: there is no CPU path")
+        if samples.dim() != 1:
+            raise ValueError(f"expected 1-D samples, got shape {tuple(samples.shape)}")
+        if samples.device != self.device:
+            raise ValueError(f"the samples are on {samples.device}, the live state on {self.device}")
+        if samples.dtype not in (torch.float32, torch.int16):
+            raise ValueError(f"samples must be float32 or int16 PCM, got {samples.dtype}")
+        if isinstance(lengths, torch.Tensor) and lengths.is_cuda:
+            raise ValueError("push_ragged takes host lengths: the host checks them and keeps samples_seen")
+        n = np.asarray(lengths).reshape(-1)
+        if n.size != self.n_streams or not np.issubdtype(n.dtype, np.integer):
+            raise ValueError(f"expected {self.n_streams} integer lengths, got {n.size} of {n.dtype}")
+        n = n.astype(np.int64)
+        if ((n < 0) | (n > self.max_push)).any():
+            s = int(np.flatnonzero((n < 0) | (n > self.max_push))[0])
+            raise ValueError(f"stream {s} brings {int(n[s])} samples; a push takes 0 to max_push = {self.max_push}")
+        if int(n.sum()) != samples.numel():
+            raise ValueError(f"the lengths add up to {int(n.sum())} samples, the tensor holds {samples.numel()}")
+        plan = ragged_push_plan(self._seen, n, self.window_size, self.shift_size)
+        shape = (plan.window_bound, self.n_frames, self.audio_processor.n_mels)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        elif out.dim() != 3 or out.shape[0] < shape[0] or out.shape[1:] != shape[1:] or out.dtype != torch.float32 \
+                or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 [>= {shape[0]}, {shape[1]}, {shape[2]}] tensor on "
+                             f"{self.device}")
+        lib = _native.load()
+        handle = self._state()
+        if self._ragged_ws is None:
+            self._ragged_ws = torch.empty(max(1, int(lib.kws_live_ragged_workspace_bytes(handle))), dtype=torch.uint8,
+                                          device=self.device)
+        lengths32 = np.ascontiguousarray(n, dtype=np.int32)
+        samples = samples.contiguous()
+        pcm16 = samples.dtype == torch.int16
+        fn = lib.kws_live_push_ragged_pcm16 if pcm16 else lib.kws_live_push_ragged
+        with torch.cuda.device(self.device):
+            _native.check(fn(handle, C.c_void_p(samples.data_ptr()), C.c_void_p(lengths32.ctypes.data),
+                             C.c_void_p(out.data_ptr()), None, None, out.shape[0], None,
+                             C.c_void_p(self._ragged_ws.data_ptr()), self._ragged_ws.numel(),
+                             C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
+                          "kws_live_push_ragged_pcm16" if pcm16 else "kws_live_push_ragged")
+        self._seen += n
+        M = plan.stream_ids.size
+        ids = torch.from_numpy(plan.stream_ids), torch.from_numpy(plan.window_ids)
+        feats = out[:M]
+        if model is None:
+            return (feats,) + ids
+        if M == 0:
+            return (torch.empty((0, model.n_labels), dtype=torch.float32, device=self.device),) + ids
+        return (model(feats),) + ids
 
     def reset(self, stream_ids):
         """Restart the given streams at sample 0; the others are not affected.  stream_ids: host integers (a list, a
@@ -223,6 +319,7 @@ class LiveStreams(object):
     def __getstate__(self):  # device state never crosses a process boundary
         d = dict(self.__dict__)
         d["_handle"] = None
+        d["_ragged_ws"] = None
         d["_seen"] = np.zeros_like(self._seen)
         for k in ("_ids_host", "_ids_dev", "_ids_copied"):
             d.pop(k, None)

@@ -98,11 +98,34 @@ int kws_mfcc_stream_forward_pcm16(const kws_frontend_t* fe, const int16_t* wav, 
  *                         bit-identical to kws_mfcc_forward on the materialised windows; slots with k < 0 (the warm-up
  *                         of a fresh stream) are all zeros.  Only the n / 160 new frame-table rows per stream and the
  *                         four reflect-padded edge frames per window are computed.
+ *                         Precondition: every c_s is a multiple of 160 (the hop), which holds unless a ragged push
+ *                         left it otherwise.  The counters live on the device, so the library cannot check it; a
+ *                         caller that mixes the two pushes checks its own copy (LiveStreams.push raises ValueError).
  *   kws_live_push_pcm16   the same on int16 PCM (see kws_mfcc_forward_pcm16): bit-identical to a float push of s/32768.
  *   kws_live_reset        stream_ids: DEVICE int64[count]; those streams restart at sample 0 (ids outside [0, S) are
  *                         ignored).  Other streams are unaffected.
  * Push and reset allocate nothing and do not synchronise the host; counters live on the device, so a caller that
- * needs the validity of each slot keeps its own copy of c_s (honk2_b200.LiveStreams does). */
+ * needs the validity of each slot keeps its own copy of c_s (honk2_b200.LiveStreams does).
+ *
+ * Ragged pushes: stream s brings its own number n_s of new samples, any n_s in [0, max_push] (not necessarily a multiple
+ * of the shift or of 160), and only the windows the push completes come back, compacted.  With c_s' = c_s + n_s, the
+ * push completes windows k with max(0, floor((c_s - window)/shift) + 1) <= k <= floor((c_s' - window)/shift).
+ *   kws_live_ragged_workspace_bytes  device scratch a ragged push needs (0 on a null state).
+ *   kws_live_push_ragged  samples: all streams' new samples back to back in stream order, sum(n_s) floats.
+ *                         lengths: HOST int32[S], read during the call.  Row i of feat [M, T, n_mels] holds window
+ *                         win_index[i] of stream win_stream[i], rows ordered by stream, then by window; M goes to
+ *                         *n_windows.  The features are bit-identical to kws_mfcc_forward on the materialised windows,
+ *                         and across any sequence of pushes each stream emits windows 0, 1, 2, ... exactly once.  feat,
+ *                         win_stream and win_index hold `capacity` rows; win_stream, win_index and n_windows may be null
+ *                         (a caller that keeps its own copy of c_s can compute them: LiveStreams does).
+ *                         Returns KWS_ERR_INVALID, launching nothing, unless every n_s is in [0, max_push], capacity >=
+ *                         sum(ceil(n_s / shift)) (which bounds M) and the workspace is large enough.
+ *   kws_live_push_ragged_pcm16  the same on int16 PCM: bit-identical to a float ragged push of s/32768.
+ * A ragged push copies the per-stream offsets and lengths to the device through a pinned host buffer of the state,
+ * allocated by the state's first ragged push; before refilling it, a push waits for the previous ragged push's copy
+ * (not for its kernels).  Nothing else allocates and the host does not wait for the device: the device derives each
+ * stream's new rows and windows from its counter and scans them (the totals are never read back).  The two pushes
+ * and reset may be mixed on one state, with the precondition of kws_live_push. */
 typedef struct kws_live kws_live_t;
 size_t kws_live_state_bytes(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push);
 int kws_live_create(const kws_frontend_t* fe, int n_streams, int window, int shift, int max_push, kws_live_t** out);
@@ -110,6 +133,13 @@ void kws_live_destroy(kws_live_t* live);
 int kws_live_reset(kws_live_t* live, const int64_t* stream_ids, int64_t count, void* stream);
 int kws_live_push(kws_live_t* live, const float* chunk, int n, float* feat, void* stream);
 int kws_live_push_pcm16(kws_live_t* live, const int16_t* chunk, int n, float* feat, void* stream);
+size_t kws_live_ragged_workspace_bytes(const kws_live_t* live);
+int kws_live_push_ragged(kws_live_t* live, const float* samples, const int32_t* lengths, float* feat,
+                         int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                         void* workspace, size_t ws_bytes, void* stream);
+int kws_live_push_ragged_pcm16(kws_live_t* live, const int16_t* samples, const int32_t* lengths, float* feat,
+                               int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                               void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- models: replace model.ResNet / model.CNN ---------------------------------------------
  * kws_resnet_create <- ResNet.__init__ (model/resnet.py:11-36); pool_h = pool_w = 0 when the
