@@ -67,7 +67,6 @@ struct TcCnnParams {
                                 //   contiguous; the first Linear's weights are permuted to this order
   int64_t B;
   TcCnnGeom g;
-  int polls;
   long long* debug;   // optional [16] cycle counters of CTA 0 (HONK2_TC_DEBUG=1), nullptr = off
 };
 
@@ -164,12 +163,12 @@ cnn_tc_fused_kernel(const TcCnnParams p) {
 #define CNN_DBG(var) if (dbg) { const long long t_ = clock64(); var += t_ - d_t; d_t = t_; }
     for (int64_t b = blockIdx.x; b < p.B; b += gridDim.x, ++it) {
       // ---- conv_0
-      mbar_wait_lean(a_full, it & 1, p.polls);
+      mbar_wait_lean(a_full, it & 1);
       tc_fence_after();
       CNN_DBG(d_afull)
       for (int t = 0; t < g.tiles0; ++t) {
         const int buf = t & 1;
-        mbar_wait_lean(acc_empty(buf), (use[buf] & 1) ^ 1, p.polls);
+        mbar_wait_lean(acc_empty(buf), (use[buf] & 1) ^ 1);
         ++use[buf];
         tc_fence_after();
         CNN_DBG(d_aempty)
@@ -188,15 +187,15 @@ cnn_tc_fused_kernel(const TcCnnParams p) {
       if (leader) umma_commit(a_free);   // all conv_0 MMAs of this issuer have read the A_e arrays
       __syncwarp();
       // ---- conv_1: this issuer's M-tiles, every tap and K chunk
-      mbar_wait_lean(pool_full, it & 1, p.polls);
-      mbar_wait_lean(acc_empty(1), (use[1] & 1) ^ 1, p.polls);   // conv_1's tiles 0-2 are buffer 1's columns
+      mbar_wait_lean(pool_full, it & 1);
+      mbar_wait_lean(acc_empty(1), (use[1] & 1) ^ 1);   // conv_1's tiles 0-2 are buffer 1's columns
       ++use[1];
       tc_fence_after();
       CNN_DBG(d_pool)
       int kw = 0;
       uint32_t tap = 0;                                           // (kh * WP + kw) rows
       for (int u = 0; u < g.units1; ++u) {
-        mbar_wait_lean(s_full(stage), sphase, p.polls);
+        mbar_wait_lean(s_full(stage), sphase);
         tc_fence_after();
         CNN_DBG(d_sfull)
         if (leader) {
@@ -289,7 +288,7 @@ cnn_tc_fused_kernel(const TcCnnParams p) {
       // ---- conv_0 tiles: max over the pool members + bias + ReLU -> pooled rows in shared memory
       for (int t = 0; t < g.tiles0; ++t) {
         const int buf = t & 1;
-        mbar_wait_lean(acc_full(buf), fullp[buf], p.polls);
+        mbar_wait_lean(acc_full(buf), fullp[buf]);
         fullp[buf] ^= 1;
         tc_fence_after();
         CNN_DBG(d_accfull)
@@ -324,12 +323,12 @@ cnn_tc_fused_kernel(const TcCnnParams p) {
       if (lane == 0) mbar_arrive(pool_full);
       // ---- the next utterance's A_e arrays (this utterance's conv_0 MMAs have retired: a_free)
       if (b + gridDim.x < p.B) {
-        mbar_wait_lean(a_free, it & 1, p.polls);
+        mbar_wait_lean(a_free, it & 1);
         build(b + gridDim.x);
       }
       CNN_DBG(d_bld)
       // ---- conv_1 tiles: bias + ReLU -> bf16 activations [position][64] in global memory
-      mbar_wait_lean(c1_done, it & 1, p.polls);
+      mbar_wait_lean(c1_done, it & 1);
       tc_fence_after();
       CNN_DBG(d_c1)
       __nv_bfloat16* act = p.act + b * (int64_t)(g.H1 * 8 * kCnnC) + (int64_t)cg * (g.H1 * 8 * 16);
@@ -531,7 +530,6 @@ struct TcCnn {
   float *b0 = nullptr, *b1 = nullptr;
   float* lin_w[4] = {nullptr, nullptr, nullptr, nullptr};
   float* lin_b[4] = {nullptr, nullptr, nullptr, nullptr};
-  int polls = 48;
   long long* debug = nullptr;   // HONK2_TC_DEBUG=1: device counters printed after every launch (synchronises)
 };
 
@@ -597,7 +595,6 @@ int tc_cnn_create(const kws_cnn_config& cfg, TcCnn** out) {
   p->supported = cnn_tc_plan(p);
   *out = p;
   if (!p->supported) return KWS_OK;
-  if (const char* e = getenv("HONK2_TC_WAIT_POLLS")) p->polls = std::max(0, atoi(e));
   const char* dbg_env = getenv("HONK2_TC_DEBUG");
   const bool want_debug = dbg_env != nullptr && atoi(dbg_env) != 0;
   const TcCnnGeom& g = p->g;
@@ -713,7 +710,7 @@ int tc_cnn_forward(TcCnn* p, const float* feat, int64_t B, int T, int F, float* 
     TcCnnParams prm;
     prm.feat = feat + b0 * (int64_t)T * F;
     prm.w0 = p->w0; prm.w1 = p->w1; prm.b0 = p->b0; prm.b1 = p->b1;
-    prm.act = act; prm.B = nb; prm.g = g; prm.polls = p->polls; prm.debug = p->debug;
+    prm.act = act; prm.B = nb; prm.g = g; prm.debug = p->debug;
     if (p->debug) cudaMemsetAsync(p->debug, 0, 16 * sizeof(long long), st);
     if (prof) prof->tick(0, st);
     const unsigned grid = (unsigned)std::min<int64_t>(nb, kNumSMs);

@@ -53,6 +53,17 @@ constexpr int kNumSMs = 148;  // B200
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
+// ResNet geometry shared by the fp32 and tensor-core paths: the dilation of C -> C layer i (1-based, resnet.py:21-23),
+// the AvgPool window after conv_0 (pool 0, 0 = absent, resnet.py:40-44), and the map it leaves of a T x F input.
+inline int resnet_dilation(const kws_resnet_config& c, int i) { return c.use_dilation ? 1 << ((i - 1) / 3) : 1; }
+struct PoolWindow { int h, w; };
+inline PoolWindow resnet_pool(const kws_resnet_config& c) { return {c.pool_h > 0 ? c.pool_h : 1, c.pool_w > 0 ? c.pool_w : 1}; }
+inline void resnet_map(const kws_resnet_config& c, int T, int F, int* H, int* W) {
+  const PoolWindow pool = resnet_pool(c);
+  *H = T / pool.h;
+  *W = F / pool.w;
+}
+
 // bump allocator over a caller-provided workspace
 struct Arena {
   char* base;

@@ -23,7 +23,7 @@ constexpr int kTcIssuers = 3;      // MMA-issuing warps (M-tiles dealt round-rob
 // 16-channel group e / 4 (two planar-8 planes) of EVERY M-tile
 __host__ __device__ constexpr int tc_epi_warps(int NKC) { return 4 * NKC; }
 __host__ __device__ constexpr int tc_threads(int NKC) { return 32 * (1 + kTcIssuers + tc_epi_warps(NKC)); }
-constexpr int kTcMaxMt = 8;       // upper bound of M-tiles per tile (min(8, kAccCols / CP) at run time)
+constexpr int kTcMaxMt = 8;       // upper bound of M-tiles per tile (tc_max_mt)
 constexpr int kAccCols = 256;     // TMEM columns per accumulator buffer
 constexpr int kMaxStages = 8;
 // ---------------------------------------------------------------------------------------------
@@ -177,19 +177,14 @@ struct TcResNet {
   TcFusedParams fused_prm{};
   int fused_smem = 0;
   // column-sweep whole-network kernel (resnet_sweep.cuh), preferred when the map is tall enough
+  // (HONK2_TC_SWEEP=0: the position-major kernel instead; the tests use it as the reference for sweep shapes)
   bool sweep_enabled = true;
-  bool sweep_k32 = true;       // HONK2_TC_SWEEP_K32=0: single-strip maps use the planar layout of the multi-strip maps too
-  int l2_policy = 1, wait_polls = 48, sweep_max_stages = 0, sweep_min_pct = 60;
-  bool sweep_discard = true;
-  bool sweep_pack = true;      // HONK2_TC_SWEEP_PACK=0: short / pooled maps stay on the position-major kernel
 };
 
 static int tc_max_mt(int CP) {
-  // M-tiles per tile, bounded by the TMEM accumulator buffer (HONK2_TC_MAXMT lowers it, for experiments:
-  // measured on B200, larger tiles win even though 5 M-tiles do not divide evenly over 3 issuer warps)
-  static const int env = [] { const char* e = std::getenv("HONK2_TC_MAXMT"); return e ? std::atoi(e) : 0; }();
-  const int cap = std::min(kTcMaxMt, kAccCols / CP);
-  return env > 0 ? std::max(1, std::min(cap, env)) : cap;
+  // M-tiles per tile, as many as the TMEM accumulator buffer holds (measured on B200: larger tiles win even though
+  // 5 M-tiles do not divide evenly over 3 issuer warps)
+  return std::min(kTcMaxMt, kAccCols / CP);
 }
 
 // Phase tiling pays when the dilation is large: a tile of R consecutive rows needs R + 2d (or 3R) input
@@ -200,7 +195,7 @@ static bool tc_use_phase(int H, int d) { return d >= 8 && d <= 32 && 2 * d <= H;
 static int tc_hpad(const kws_resnet_config& c, int H) {
   int m = 1;
   for (int i = 1; i <= c.n_layers; ++i) {
-    const int d = c.use_dilation ? (1 << ((i - 1) / 3)) : 1;
+    const int d = resnet_dilation(c, i);
     if (tc_use_phase(H, d)) m = std::max(m, d);
   }
   return round_up(H, m);
@@ -326,16 +321,9 @@ int tc_resnet_create(const kws_resnet_config& cfg, TcResNet** out) {
     p->conv0_w = reinterpret_cast<float*>(b); b += round_up<size_t>(C * 9 * 4, 256);
     p->out_w = reinterpret_cast<float*>(b); b += round_up<size_t>((size_t)cfg.n_labels * C * 4, 256);
     p->out_b = reinterpret_cast<float*>(b);
-    // every knob is read HERE, once per model handle (DESIGN.md section 4 lists them)
-    auto env_int = [](const char* name, int dflt) { const char* e = std::getenv(name); return e ? std::atoi(e) : dflt; };
-    p->sweep_enabled = env_int("HONK2_TC_SWEEP", 1) != 0;
-    p->sweep_k32 = env_int("HONK2_TC_SWEEP_K32", 1) != 0;
-    p->sweep_discard = env_int("HONK2_TC_SWEEP_DISCARD", 1) != 0;
-    p->sweep_pack = env_int("HONK2_TC_SWEEP_PACK", 1) != 0;
-    p->sweep_max_stages = env_int("HONK2_TC_SWEEP_STAGES", kSwMaxStages);
-    p->sweep_min_pct = env_int("HONK2_TC_SWEEP_MINPCT", 60);
-    p->l2_policy = env_int("HONK2_TC_L2POLICY", 1);
-    p->wait_polls = env_int("HONK2_TC_WAIT_POLLS", 48);
+    // read once per model handle (DESIGN.md section 4)
+    const char* e = std::getenv("HONK2_TC_SWEEP");
+    p->sweep_enabled = !e || std::atoi(e) != 0;
   }
   *out = p;
   return KWS_OK;
@@ -375,17 +363,11 @@ int tc_resnet_set_weights(TcResNet* p, const kws_resnet_weights& w, float* const
   return KWS_OK;
 }
 
-static void tc_map_hw(const kws_resnet_config& c, int T, int F, int* H, int* W) {
-  const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
-  *H = T / ph;
-  *W = F / pw;
-}
-
 static bool tc_layers_ok(const TcResNet* p, int H, int W) {
   TcGeom g;
   const int Hpad = tc_hpad(p->cfg, H);
   for (int i = 1; i <= p->cfg.n_layers; ++i) {
-    const int d = p->cfg.use_dilation ? (1 << ((i - 1) / 3)) : 1;
+    const int d = resnet_dilation(p->cfg, i);
     if (!tc_geom(p->NKC, H, Hpad, W, d, &g)) return false;
   }
   return true;
@@ -439,7 +421,7 @@ static TcFusedPlan tc_fused_plan(const TcResNet* p, int H, int W, bool split) {
   f.ring_off = round_up(f.w_off[1] + w_bytes, 1024);
   for (int i = 1; i <= c.n_layers; ++i) {
     TcGeom g;
-    const int d = c.use_dilation ? (1 << ((i - 1) / 3)) : 1;
+    const int d = resnet_dilation(c, i);
     // (tc_geom picks the tile rows against a budget of one resident weight set; this kernel's ring is sized below)
     if (!tc_geom(p->NKC, H, f.Hpad, W, d, &g)) return f;
     f.slot_bytes = std::max(f.slot_bytes, round_up(g.stage_bytes, 128));
@@ -511,11 +493,11 @@ static int tc_fused_forward(TcResNet* p, const TcFusedPlan& f, const float* feat
     q.out_b = p->out_b;
     q.P = P; q.Q = Q;
     q.n_layers = n; q.C = c.n_maps; q.n_labels = c.n_labels; q.T = T; q.F = F;
-    q.ph = c.pool_h > 0 ? c.pool_h : 1; q.pw = c.pool_w > 0 ? c.pool_w : 1;
+    const auto [ph, pw] = resnet_pool(c);
+    q.ph = ph; q.pw = pw;
     q.H = H; q.W = W; q.Hpad = f.Hpad;
     q.smem_w_off[0] = f.w_off[0]; q.smem_w_off[1] = f.w_off[1];
     q.smem_ring_off = f.ring_off; q.ring_slot_bytes = f.slot_bytes; q.n_stages = f.n_stages;
-    q.l2_policy = p->l2_policy;
     p->fused_smem = f.smem_total;
     p->fused_key = key;
   }
@@ -574,6 +556,10 @@ struct TcSweepPlan {
 // (PH, PW) pooling windows the pre-pass kernel of the packed-strip mode is instantiated for
 static bool tc_pack_pool_ok(int ph, int pw) { return (ph == 1 && pw == 1) || (ph == 2 && pw == 2) || (ph == 4 && pw == 3); }
 
+// An unpooled map that fills less than this share (%) of its 128-row strips is packed; a single packed map that still
+// fills less than it stays on the position-major kernel.
+constexpr int kSwMinStripPct = 60;
+
 static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
   TcSweepPlan f;
   const int H_map = H;
@@ -586,34 +572,34 @@ static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
   if ((1 + c.n_layers) * p->CP * 4 > kSwKcBytes) return f;   // per-layer epilogue constants live in shared memory
   int dmax = 1;
   for (int i = 1; i <= c.n_layers; ++i) {
-    const int d = c.use_dilation ? (1 << ((i - 1) / 3)) : 1;
+    const int d = resnet_dilation(c, i);
     if (d > 64) return f;   // (a staged column of 128 + 2d rows per plane would no longer leave room for three stages)
     dmax = std::max(dmax, d);
   }
-  const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
+  const auto [ph, pw] = resnet_pool(c);
   const bool pooled = ph > 1 || pw > 1;
   // The 128 lanes of an MMA are 128 rows of one column.  Short maps (res8 / res26 after pooling, short clips) are
   // PACKED: several utterances share a strip, stacked along the rows with dmax zero rows between them, and conv_0
   // (+ ReLU + AvgPool) is computed by a CUDA-core pre-pass (the sweep's own conv_0 pseudo-layer works on the unpooled map).
-  const bool is_short = H * 100 < ceil_div(H, 128) * 128 * p->sweep_min_pct;
+  const bool is_short = H * 100 < ceil_div(H, 128) * 128 * kSwMinStripPct;
   if (pooled || is_short) {
     const int pitch = H + dmax;
     const int n = (128 + dmax) / pitch;
-    if (!p->sweep_pack || n < 1 || !tc_pack_pool_ok(ph, pw) || !(p->sweep_k32 || split)) return f;
+    if (n < 1 || !tc_pack_pool_ok(ph, pw)) return f;
     f.packed = true;
     f.pack_n = n;
     f.pack_pitch = pitch;
     f.Hst = n * pitch - dmax;
-    if (f.Hst * 100 < 128 * p->sweep_min_pct && n == 1) return f;   // a single short map gains nothing here
+    if (f.Hst * 100 < 128 * kSwMinStripPct && n == 1) return f;   // a single short map gains nothing here
   }
   if (f.packed) H = f.Hst;   // from here on the "map" is the stack
   f.n_strips = ceil_div(H, 128);
   f.n_slots = p->n_sms;
   f.dmax = dmax;
   f.split = split;
-  // 16 channels per row: [w][K chunk][h][32 B] in HBM, swizzle-32B operand in shared memory, one bulk copy per step
-  // (single-strip maps; HONK2_TC_SWEEP_K32=0 keeps them on the planar layout of the multi-strip maps)
-  f.k32 = f.n_strips == 1 && (p->sweep_k32 || split);
+  // single-strip maps: 16 channels per row, [w][K chunk][h][32 B] in HBM, swizzle-32B operand in shared memory, one bulk
+  // copy per step; taller maps: the planar layout
+  f.k32 = f.n_strips == 1;
   if (split && !f.k32) return f;   // the split-bf16 mode is built on the 32-byte-row layout
   const int set_bytes = 9 * p->NKC * 2 * p->CP * 16;           // one weight set
   const int w_bytes = (split ? 2 : 1) * set_bytes;
@@ -640,8 +626,7 @@ static TcSweepPlan tc_sweep_plan(const TcResNet* p, int H, int W, bool split) {
     f.slot_bytes = p->NP * f.chunk_rows * 16;
     f.slack_bytes = 0;
   }
-  const int max_stages = std::min(kSwMaxStages, p->sweep_max_stages > 0 ? p->sweep_max_stages : kSwMaxStages);
-  f.n_stages = std::min(max_stages, (227 * 1024 - f.slack_bytes - f.ring_off) / f.slot_bytes);
+  f.n_stages = std::min(kSwMaxStages, (227 * 1024 - f.slack_bytes - f.ring_off) / f.slot_bytes);
   if (f.n_stages < 3) return f;
   f.smem_total = f.ring_off + f.n_stages * f.slot_bytes + f.slack_bytes;
   f.ok = true;
@@ -781,14 +766,14 @@ static int tc_launch_sweep_v(const SwParams& prm, int grid, int smem, cudaStream
 }
 
 template <int NKC>
-static int tc_launch_sweep(const SwParams& prm, bool split, int grid, int smem, cudaStream_t st) {
+static int tc_launch_sweep(const SwParams& prm, bool k32, bool split, int grid, int smem, cudaStream_t st) {
   if (prm.ext_in != nullptr)   // packed strips (always the 32-byte-row layout; no cycle-accounting build)
     return split ? tc_launch_sweep_v<NKC, false, true, true, true>(prm, grid, smem, st)
                  : tc_launch_sweep_v<NKC, false, true, false, true>(prm, grid, smem, st);
   if (split) return tc_launch_sweep_v<NKC, false, true, true, false>(prm, grid, smem, st);
   if (prm.debug != nullptr)
-    return prm.k32 ? tc_launch_sweep_v<NKC, true, true, false, false>(prm, grid, smem, st) : tc_launch_sweep_v<NKC, true, false, false, false>(prm, grid, smem, st);
-  return prm.k32 ? tc_launch_sweep_v<NKC, false, true, false, false>(prm, grid, smem, st) : tc_launch_sweep_v<NKC, false, false, false, false>(prm, grid, smem, st);
+    return k32 ? tc_launch_sweep_v<NKC, true, true, false, false>(prm, grid, smem, st) : tc_launch_sweep_v<NKC, true, false, false, false>(prm, grid, smem, st);
+  return k32 ? tc_launch_sweep_v<NKC, false, true, false, false>(prm, grid, smem, st) : tc_launch_sweep_v<NKC, false, false, false, false>(prm, grid, smem, st);
 }
 
 static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat, int64_t B, int64_t B_utt, int T, int F, int H,
@@ -806,7 +791,7 @@ static int tc_sweep_forward(TcResNet* p, const TcSweepPlan& f, const float* feat
     // one launch pair per sub-batch.  The rows between stacked utterances are never stored: zero both buffers once.
     KWS_CUDA(cudaMemsetAsync(ws, 0, 2 * buf, st));
     const int64_t chunk = tc_pack_chunk(f, B, chunk_cfg);
-    const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
+    const auto [ph, pw] = resnet_pool(c);
     uint4* ext = reinterpret_cast<uint4*>(static_cast<char*>(ws) + 2 * buf);
     for (int64_t b0 = 0; b0 < B; b0 += chunk) {
       const int64_t nb = std::min(chunk, B - b0);
@@ -848,16 +833,13 @@ static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat,
   prm.dmax = f.dmax;
   prm.chunk_rows = f.chunk_rows;
   prm.ring_slack_bytes = f.slack_bytes;
-  prm.k32 = f.k32 ? 1 : 0;
-  prm.discard_q = p->sweep_discard && f.n_strips == 1 && !f.split && !f.packed;   // (packed: the zero rows inside a column must survive)
+  prm.discard_q = f.n_strips == 1 && !f.split && !f.packed;   // (packed: the zero rows inside a column must survive)
   prm.ext_in = ext; prm.ext_stride = ext_stride;
   prm.pack_n = f.packed ? f.pack_n : 1; prm.pack_h = sub_h; prm.pack_pitch = f.packed ? f.pack_pitch : H;
   prm.smem_pool_off = f.pool_off;
   prm.B_utt = B_utt;
   prm.smem_w_off[0] = f.w_off[0]; prm.smem_w_off[1] = f.w_off[1];
   prm.smem_ring_off = f.ring_off; prm.ring_slot_bytes = f.slot_bytes; prm.n_stages = f.n_stages;
-  prm.l2_policy = p->l2_policy;
-  prm.wait_polls = p->wait_polls;
   prm.feat = feat;
   prm.logits = logits;
   prm.B = B;
@@ -868,8 +850,6 @@ static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat,
   if (dbg_on && !f.split && !f.packed) {
     if (!dbg_buf) cudaMalloc(&dbg_buf, 16 * sizeof(long long));
     prm.debug = dbg_buf;
-    const char* e = std::getenv("HONK2_TC_DIAG");
-    prm.diag = e ? std::atoi(e) : 0;
   }
   static const bool trace_on = [] { const char* e = std::getenv("HONK2_TC_TRACE"); return e && std::atoi(e) != 0; }();
   static long long* trace_buf = nullptr;
@@ -917,9 +897,9 @@ static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat,
     }
   } dbg_print{prm.debug, st, prm.trace};
   switch (p->NKC) {
-    case 1: return tc_launch_sweep<1>(prm, f.split, grid, f.smem_total, st);
-    case 2: return tc_launch_sweep<2>(prm, f.split, grid, f.smem_total, st);
-    default: return tc_launch_sweep<3>(prm, f.split, grid, f.smem_total, st);
+    case 1: return tc_launch_sweep<1>(prm, f.k32, f.split, grid, f.smem_total, st);
+    case 2: return tc_launch_sweep<2>(prm, f.k32, f.split, grid, f.smem_total, st);
+    default: return tc_launch_sweep<3>(prm, f.k32, f.split, grid, f.smem_total, st);
   }
 }
 
@@ -928,7 +908,7 @@ static int tc_sweep_launch(TcResNet* p, const TcSweepPlan& f, const float* feat,
 size_t tc_resnet_workspace_bytes(const TcResNet* p, int64_t B, int T, int F, int chunk, bool split) {
   if (!p || !p->supported) return 0;
   int H, W;
-  tc_map_hw(p->cfg, T, F, &H, &W);
+  resnet_map(p->cfg, T, F, &H, &W);
   if (H < 1 || W < 1 || W > 256 || !tc_layers_ok(p, H, W)) return 0;
   const TcSweepPlan sp = tc_sweep_plan(p, H, W, split);
   if (sp.ok) return tc_sweep_ws_bytes(p, sp, H, W, B, chunk, nullptr);
@@ -939,7 +919,7 @@ size_t tc_resnet_workspace_bytes(const TcResNet* p, int64_t B, int T, int F, int
 const char* tc_resnet_kernel_path(const TcResNet* p, int T, int F, bool split) {
   if (!p || !p->supported) return "unsupported";
   int H, W;
-  tc_map_hw(p->cfg, T, F, &H, &W);
+  resnet_map(p->cfg, T, F, &H, &W);
   if (H < 1 || W < 1 || W > 256 || !tc_layers_ok(p, H, W)) return "unsupported";
   if (tc_sweep_plan(p, H, W, split).ok) return "resnet_tc_sweep_kernel";
   if (tc_fused_plan(p, H, W, split).ok) return "resnet_tc_fused_kernel";
@@ -954,7 +934,7 @@ int tc_resnet_forward(TcResNet* p, const float* feat, int64_t B, int T, int F, f
     return KWS_ERR_UNSUPPORTED;
   }
   int H, W;
-  tc_map_hw(p->cfg, T, F, &H, &W);
+  resnet_map(p->cfg, T, F, &H, &W);
   KWS_REQUIRE(H >= 1 && W >= 1, "ResNet: input %dx%d is smaller than the pooling window", T, F);
   const size_t need = tc_resnet_workspace_bytes(p, B, T, F, chunk_cfg, split);
   if (need == 0) {

@@ -42,10 +42,6 @@ struct Model {
   int c_h0 = 0, c_w0 = 0, c_hp0 = 0, c_wp0 = 0, c_h1 = 0, c_w1 = 0, c_hp1 = 0, c_wp1 = 0, c_flat = 0;
 };
 
-static int resnet_dilation(const kws_resnet_config& c, int i) {
-  return c.use_dilation ? (1 << ((i - 1) / 3)) : 1;  // resnet.py:21-23
-}
-
 // ---------------------------------------------------------------------------------------------
 // packing kernels (run once per load_state_dict)
 
@@ -188,12 +184,6 @@ extern "C" int kws_resnet_set_weights(kws_model_t* m, const kws_resnet_weights* 
 
 namespace kws {
 
-static void resnet_map(const kws_resnet_config& c, int T, int F, int* H, int* W) {
-  const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
-  *H = T / ph;
-  *W = F / pw;
-}
-
 static int64_t default_chunk(const Model* m, int precision, int64_t per_utt_bytes) {
   if (m->chunk[precision] > 0) return m->chunk[precision];
   // The fp32 CUDA-core path is FMA-bound (a layer moves ~2.2 MB per utterance through DRAM at < 10 % of the HBM
@@ -233,7 +223,7 @@ static int resnet_forward_f32(Model* m, const float* feat, int64_t B, int T, int
   float* P = reinterpret_cast<float*>(static_cast<char*>(ws));            // skip tensor / conv_0 output
   float* A0 = reinterpret_cast<float*>(static_cast<char*>(ws) + buf);
   float* A1 = reinterpret_cast<float*>(static_cast<char*>(ws) + 2 * buf);
-  const int ph = c.pool_h > 0 ? c.pool_h : 1, pw = c.pool_w > 0 ? c.pool_w : 1;
+  const auto [ph, pw] = resnet_pool(c);
   // equal sub-batches (2048 utterances = 3 x 683, not 985 + 985 + 78): the persistent kernels' last wave stays full
   if (B > chunk) chunk = ceil_div<int64_t>(B, ceil_div<int64_t>(B, chunk));
   for (int64_t b0 = 0; b0 < B; b0 += chunk) {

@@ -58,15 +58,15 @@ __device__ __forceinline__ void mbar_wait_sleepy(uint32_t bar, uint32_t parity) 
 // Wait with few instructions per poll (for the MMA issuers, whose instruction count is the bottleneck): the
 // hardware suspends the thread until the phase completes or the hint elapses; the watchdog is read every 256 polls.
 // The hinted try_wait compiles to TRYWAIT + NANOSLEEP.SYNCS: the thread leaves the issue slots to other warps, but waking
-// up is slow; waits that are usually short poll a few times first (`polls`, a kernel parameter: HONK2_TC_WAIT_POLLS,
-// default 48; measured +2-4 %).
-__device__ __forceinline__ void mbar_wait_lean(uint32_t bar, uint32_t parity, int polls) {
+// up is slow; waits that are usually short poll 48 times first (measured +2-4 % against suspending at once).
+__device__ __forceinline__ void mbar_wait_lean(uint32_t bar, uint32_t parity) {
+  constexpr int kPolls = 48;
   if (mbar_try_wait(bar, parity)) return;
 #pragma unroll 1
-  for (int i = 0; i < polls; ++i)
+  for (int i = 0; i < kPolls; ++i)
     if (mbar_try_wait(bar, parity)) return;
   long long t0 = 0;
-  for (uint32_t it = 1; !mbar_try_wait_hint(bar, parity, polls > 0 ? 1000u : 100000u); ++it) {
+  for (uint32_t it = 1; !mbar_try_wait_hint(bar, parity, 1000u); ++it) {
     if ((it & 255u) == 0u) {
       if (t0 == 0) t0 = clock64();
       else if (clock64() - t0 > kSpinLimitCycles) __trap();
@@ -109,14 +109,6 @@ __device__ __forceinline__ bool elect_one() {
       : "=r"(pred));
   return pred != 0;
 }
-__device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1,
-                                            int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6, %7}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
 // ---- L2 eviction-priority policies (createpolicy) and hinted accesses
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t pol;
@@ -126,11 +118,6 @@ __device__ __forceinline__ uint64_t l2_policy_evict_last() {
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_normal() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
   return pol;
 }
 __device__ __forceinline__ uint4 ld_hint(const uint4* ptr, uint64_t pol) {

@@ -75,7 +75,6 @@ struct TcFusedParams {
   int smem_w_off[2], smem_ring_off, ring_slot_bytes;
   int n_stages;       // ring slots in use (2 .. kFusedStages)
   long long* debug;   // optional [16] cycle counters written by CTA 0's first issuer thread (nullptr = off)
-  int l2_policy;   // 1: buffer P (read twice, rewritten in place) evict_last, buffer Q (write once, read once) evict_first
 };
 
 template <int NKC, bool SPLIT>
@@ -150,10 +149,8 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
 
   // The two slot buffers of all CTAs together are about as large as the L2, so plain LRU thrashes.  P is
   // kept (evict_last): it is read as the odd layers' input, read again as the skip tensor and rewritten in
-  // place.  Q streams (evict_first): written once, read once.
-  const bool use_pol = p.l2_policy != 0;
-  const uint64_t pol_keep = l2_policy_evict_last();
-  const uint64_t pol_stream = l2_policy_evict_first();
+  // place.  Q streams (evict_first): written once, read once.  Each policy is created where it is used: one
+  // instruction, and no register pair held for the whole kernel.
 
   // pipeline state (persists across layers and utterances; every role walks the same tile sequence)
   int stage = 0, acc = 0;
@@ -219,7 +216,7 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
 #pragma unroll
                 for (int e = 0; e < 4; ++e) ob[e] = __floats2bfloat162_rn(a4[px][2 * e], a4[px][2 * e + 1]);
                 uint4* dst = bufP + pl * plane_stride + (int64_t)h * p.W + w0 + px;
-                if (use_pol) st_hint(dst, o, pol_keep); else *dst = o;
+                st_hint(dst, o, l2_policy_evict_last());
                 if constexpr (SPLIT) {   // lo part: x - float(hi)
                   uint4 o2;
                   __nv_bfloat162* ob2 = reinterpret_cast<__nv_bfloat162*>(&o2);
@@ -228,7 +225,7 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
                     const float2 fh = __bfloat1622float2(ob[e]);
                     ob2[e] = __floats2bfloat162_rn(a4[px][2 * e] - fh.x, a4[px][2 * e + 1] - fh.y);
                   }
-                  if (use_pol) st_hint(dst + NP * plane_stride, o2, pol_keep); else dst[NP * plane_stride] = o2;
+                  st_hint(dst + NP * plane_stride, o2, l2_policy_evict_last());
                 }
               }
             }
@@ -333,13 +330,9 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
               const uint32_t sbase = smem_u32(s_ring + (size_t)stage * p.ring_slot_bytes);
               for (int half = 0; half < 2; ++half)
                 for (int bx = 0; bx < g.n_boxes; ++bx)
-                  if (use_pol)
-                    tma_load_5d_hint(sbase + half * g.slab_bytes + bx * g.box_stride, map, full_bar(stage), 0, -g.dpad,
-                                     r0 + g.h_start[bx], ph, (int)blockIdx.x * NPX + 2 * kc + half,
-                                     L.in_buf ? pol_stream : pol_keep);
-                  else
-                    tma_load_5d(sbase + half * g.slab_bytes + bx * g.box_stride, map, full_bar(stage), 0, -g.dpad,
-                                r0 + g.h_start[bx], ph, (int)blockIdx.x * NPX + 2 * kc + half);
+                  tma_load_5d_hint(sbase + half * g.slab_bytes + bx * g.box_stride, map, full_bar(stage), 0, -g.dpad,
+                                   r0 + g.h_start[bx], ph, (int)blockIdx.x * NPX + 2 * kc + half,
+                                   L.in_buf ? l2_policy_evict_first() : l2_policy_evict_last());
               if (++stage == p.n_stages) { stage = 0; phase ^= 1; }
             }
           }
@@ -446,11 +439,11 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
           };
           constexpr int NSK = SPLIT ? 4 : 2;   // skip registers: planes 2j, 2j+1 (SPLIT: and their lo planes)
           auto load_skip = [&](int64_t b0, uint4 (&dst)[NSK]) {
-            dst[0] = use_pol ? ld_hint(skip_in + b0, pol_keep) : skip_in[b0];
-            dst[1] = use_pol ? ld_hint(skip_in + b0 + plane_stride, pol_keep) : skip_in[b0 + plane_stride];
+            dst[0] = ld_hint(skip_in + b0, l2_policy_evict_last());
+            dst[1] = ld_hint(skip_in + b0 + plane_stride, l2_policy_evict_last());
             if constexpr (SPLIT) {
-              dst[2] = use_pol ? ld_hint(skip_in + b0 + NP * plane_stride, pol_keep) : skip_in[b0 + NP * plane_stride];
-              dst[3] = use_pol ? ld_hint(skip_in + b0 + (NP + 1) * plane_stride, pol_keep) : skip_in[b0 + (NP + 1) * plane_stride];
+              dst[2] = ld_hint(skip_in + b0 + NP * plane_stride, l2_policy_evict_last());
+              dst[3] = ld_hint(skip_in + b0 + (NP + 1) * plane_stride, l2_policy_evict_last());
             }
           };
           uint4 pv_next[NSK];
@@ -507,8 +500,7 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
                   __nv_bfloat162* yb = reinterpret_cast<__nv_bfloat162*>(&yo);
 #pragma unroll
                   for (int e = 0; e < 4; ++e) yb[e] = __floats2bfloat162_rn(x[2 * e], x[2 * e + 1]);
-                  if (use_pol) st_hint(y_out + base + hf * plane_stride, yo, has_skip ? pol_keep : pol_stream);
-                  else y_out[base + hf * plane_stride] = yo;
+                  st_hint(y_out + base + hf * plane_stride, yo, has_skip ? l2_policy_evict_last() : l2_policy_evict_first());
                   if constexpr (SPLIT) {   // lo part: x - float(hi)
                     uint4 yl;
                     __nv_bfloat162* lb = reinterpret_cast<__nv_bfloat162*>(&yl);
@@ -517,8 +509,7 @@ resnet_tc_fused_kernel(const TcFusedParams p) {
                       const float2 fh = __bfloat1622float2(yb[e]);
                       lb[e] = __floats2bfloat162_rn(x[2 * e] - fh.x, x[2 * e + 1] - fh.y);
                     }
-                    if (use_pol) st_hint(y_out + base + (NP + hf) * plane_stride, yl, has_skip ? pol_keep : pol_stream);
-                    else y_out[base + (NP + hf) * plane_stride] = yl;
+                    st_hint(y_out + base + (NP + hf) * plane_stride, yl, has_skip ? l2_policy_evict_last() : l2_policy_evict_first());
                   }
                 }
               }

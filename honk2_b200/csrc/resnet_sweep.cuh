@@ -116,19 +116,13 @@ struct SwParams {
   int smem_w_off[2], smem_ring_off, ring_slot_bytes, n_stages;
   int smem_skip_off;            // skip staging: one slot of NP * 2048 bytes per epilogue warp group (unused by SPLIT)
   int ring_slack_bytes;         // bytes behind the last stage that its lanes past the map read (planar: zeroed)
-  int l2_policy;
   int chunk_rows;               // planar: rows per plane of a staged column (a multiple of 8): data row h of the strip sits at
-                                //   slot row dmax + h, the pad rows above and below are zero (single strip: zeroed once and
-                                //   never written; several strips: re-zeroed by the producer for the strips that touch the
-                                //   map's top / bottom), 128 + 2 dmax.  (k32: the chunk pitch is H)
+                                //   slot row dmax + h, the pad rows above and below are zero (zeroed once, and re-zeroed by
+                                //   the producer for the strips that touch the map's top / bottom), 128 + 2 dmax.  (k32: the
+                                //   chunk pitch is H)
   int dmax;                     // largest dilation of the network = the guard rows in front of a k32 stage's first chunk
-  int k32;                      // 1 = activations as [w][K chunk][h][16 channels = 32 B] (single strip): one copy per step,
-                                //     swizzle-32B A operand, edge lanes masked; the two 16-byte halves of row h of chunk kc are
-                                //     stored swapped where ((dmax + kc H + h) >> 2) & 1, i.e. exactly as the linear copy must
-                                //     land them in the stage (stages are 256-byte aligned: the swizzle works on absolute addresses)
-  int wait_polls;               // barrier polls before a wait falls back to the suspending try_wait (HONK2_TC_WAIT_POLLS)
-  int discard_q;                // 1 = Q columns are discarded from L2 (no write-back) once the layer that reads them has consumed them
-  int diag;                     // diagnostics (wrong results!): 1 = epilogue skips math and stores, 2 = skips the skip-tensor loads
+  int discard_q;                // 1 = Q columns are discarded from L2 (no write-back) once the layer that reads them has consumed
+                                //     them (single-strip maps, so the 32-byte-row layout only)
   long long* debug;             // optional cycle counters of CTA 0 (HONK2_TC_DEBUG=1)
   long long* trace;             // optional [8][kSwTraceLen] event timestamps of CTA 0 (HONK2_TC_TRACE=1, needs DEBUG)
   // Packed strips (short maps: res8 / res26 after pooling, short clips): `pack_n` utterances share ONE strip, stacked along
@@ -143,6 +137,9 @@ struct SwParams {
   int64_t B_utt;                // utterances (packed mode: the last group may be partly empty)
 };
 
+// K32: the 32-byte-row layout of single-strip maps (above), else the planar one.  The two 16-byte halves of row h of
+// chunk kc are stored swapped where ((dmax + kc H + h) >> 2) & 1, i.e. exactly as the linear copy must land them in the
+// stage (stages are 256-byte aligned: the swizzle works on absolute addresses).
 template <int NKC, bool DBG, bool K32, bool SPLIT, bool PACK>
 __global__ void __launch_bounds__(sw_threads(NKC), 1)
 resnet_tc_sweep_kernel(const SwParams p) {
@@ -194,7 +191,6 @@ resnet_tc_sweep_kernel(const SwParams p) {
   const int64_t col_stride = (int64_t)NA * H * 2;  // k32: 16-byte units between columns
   const int64_t plane_stride = (int64_t)W * H;    // planar: 16-byte units between planes
   const int64_t slot_base = (int64_t)blockIdx.x * ((int64_t)(SPLIT ? 2 : 1) * NP * W * H);   // this CTA's utterance slot
-  auto wait_lean = [&](uint32_t bar, uint32_t parity) { mbar_wait_lean(bar, parity, p.wait_polls); };
   uint4* bufP = reinterpret_cast<uint4*>(p.P) + slot_base;
   uint4* bufQ = reinterpret_cast<uint4*>(p.Q) + slot_base;
 
@@ -247,10 +243,9 @@ resnet_tc_sweep_kernel(const SwParams p) {
   __syncthreads();
   tc_fence_after();
 
-  const bool use_pol = p.l2_policy != 0;
-  // l2_policy: 1 = P evict_last / Q evict_first (default), 2 = P evict_last / Q evict_normal, 3 = P normal / Q evict_first
-  const uint64_t pol_keep = p.l2_policy == 3 ? l2_policy_evict_normal() : l2_policy_evict_last();
-  const uint64_t pol_stream = p.l2_policy == 2 ? l2_policy_evict_normal() : l2_policy_evict_first();
+  // L2 policies: P (read as the odd layers' input and as the skip tensor, rewritten in place) evict_last, Q (written once,
+  // read once) evict_first.  Each is created where it is used: one instruction, and no register pair held for the
+  // whole kernel.
 
   auto layer_dil = [&](int l) { return p.use_dilation ? (1 << (l / 3)) : 1; };
   // rows per plane / chunk of a staged column = its pitch in shared memory (a multiple of 8 rows)
@@ -288,7 +283,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
           const int d = is_c0 ? 1 : layer_dil(l);
           const int n_runs = d < W ? d : W;
           const bool in_q = !is_c0 && (l & 1) != 0;
-          const uint64_t pol = in_q ? pol_stream : pol_keep;
+          const uint64_t pol = in_q ? l2_policy_evict_first() : l2_policy_evict_last();
           bool w_pending = !is_c0 && wq + 1 < n_wq;
           auto request_weights = [&]() {
             if constexpr (SPLIT) {
@@ -338,7 +333,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
 #pragma unroll
                     for (int c = 0; c < 4; ++c) { st[c] = t; ph[c] = q2; if (++t == p.n_stages) { t = 0; q2 ^= 1u; } } }
 #pragma unroll
-                  for (int c = 0; c < 4; ++c) if (c < cnt) wait_lean(empty_bar(st[c]), ph[c] ^ 1u);
+                  for (int c = 0; c < 4; ++c) if (c < cnt) mbar_wait_lean(empty_bar(st[c]), ph[c] ^ 1u);
                   pstamp(pd_empty);
                   float4 fr[5];
 #pragma unroll
@@ -402,9 +397,9 @@ resnet_tc_sweep_kernel(const SwParams p) {
               for (int w = r; w < W; w += d, ++step) {
                 if (!SPLIT && w_pending && step == kSwWeightStep) request_weights();
                 pstamp(pd_issue);
-                if (!is_c0 && !(ext && l == 0)) wait_lean(col_bar(prev_par, w), prev_phase);   // column w of the previous pseudo-layer is stored
+                if (!is_c0 && !(ext && l == 0)) mbar_wait_lean(col_bar(prev_par, w), prev_phase);   // column w of the previous pseudo-layer is stored
                 pstamp(pd_col);
-                wait_lean(empty_bar(stage), sphase ^ 1);
+                mbar_wait_lean(empty_bar(stage), sphase ^ 1);
                 pstamp(pd_empty);
                 const uint32_t dst = sbase + p.smem_ring_off + (uint32_t)stage * p.ring_slot_bytes;
                 if (k32) {
@@ -548,7 +543,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
             else umma_f16_lohi2<true>(dt, a, a_hi, b, desc_hi, id);
           };
           stamp(dbg_other);
-          if (!is_c0) wait_lean(wfull_bar((int)(wq & 1)), (uint32_t)((wq >> 1) & 1));
+          if (!is_c0) mbar_wait_lean(wfull_bar((int)(wq & 1)), (uint32_t)((wq >> 1) & 1));
           stamp(dbg_w);
           for (int s = 0; s < n_strips; ++s)
             for (int r = 0; r < n_runs; ++r) {
@@ -566,12 +561,12 @@ resnet_tc_sweep_kernel(const SwParams p) {
                   stamp(dbg_other);
                   tr(1);
                   // the epilogue must have drained and re-zeroed the previous use of every slot of the window
-                  if (lo) wait_lean(tempty_bar(s_lo), par_lo ^ 1u);
-                  wait_lean(tempty_bar(sl), pr ^ 1u);
-                  if (hi_) wait_lean(tempty_bar(s_hi), par_hi ^ 1u);
+                  if (lo) mbar_wait_lean(tempty_bar(s_lo), par_lo ^ 1u);
+                  mbar_wait_lean(tempty_bar(sl), pr ^ 1u);
+                  if (hi_) mbar_wait_lean(tempty_bar(s_hi), par_hi ^ 1u);
                   stamp(dbg_tempty);
                   tr(2);
-                  wait_lean(full_bar(stage), sphase);
+                  mbar_wait_lean(full_bar(stage), sphase);
                   tc_fence_after();
                   tr(3);
                   if constexpr (DBG) { if (is_c0 && s == 0 && r == 0 && i < kSwIssuers) stamp(dbg_utt); else stamp(dbg_full); }
@@ -593,7 +588,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                   // together, then all three do their commits / bookkeeping / operand preparation at the same time and
                   // the tensor pipe idles ~600 cycles per round (event trace).  With it, everything above this line
                   // and the commits below overlap the other two issuers' bursts.
-                  wait_lean(turn_bar(me), turn_par);
+                  mbar_wait_lean(turn_bar(me), turn_par);
                   turn_par ^= 1u;
                   if (!leader) {
                     // (only the elected lane issues)
@@ -718,7 +713,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
           constexpr bool LAST = decltype(last_c)::value;       // pooled instead of stored
           const bool to_p = HAS_SKIP || is_c0;   // conv_0 and the skip layers write P, the others Q
           uint4* y_out = to_p ? bufP : bufQ;
-          const uint64_t pol_out = to_p ? pol_keep : pol_stream;
+          const uint64_t pol_out = to_p ? l2_policy_evict_last() : l2_policy_evict_first();
           float psum[LAST ? CP : 1];
 #pragma unroll
           for (int c = 0; c < (LAST ? CP : 1); ++c) psum[c] = 0.f;
@@ -785,9 +780,9 @@ resnet_tc_sweep_kernel(const SwParams p) {
               // This layer READS Q (the previous layer's output), one column per step, and the MMAs of this block were
               // the last consumers of Q column w.  Nothing reads that column again before the next even layer rewrites
               // it, so its dirty lines need not ever reach HBM: discard the 128-byte lines that lie wholly inside the
-              // column (lines shared with the neighbouring columns stay).  One line per lane (k32: the column is
-              // contiguous, NKC * H * 32 B <= 96 lines), planes 16 lanes apart.
-              if (p.discard_q && k32) {
+              // column (lines shared with the neighbouring columns stay).  One line per lane: the column is contiguous,
+              // NKC * H * 32 B <= 96 lines.
+              if (k32 && p.discard_q) {
                 const char* qb = reinterpret_cast<const char*>(bufQ);
                 const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(qb) & 127u);
                 const uint32_t col_bytes = (uint32_t)(NKC * H) * 32u;
@@ -795,17 +790,6 @@ resnet_tc_sweep_kernel(const SwParams p) {
                 const uint32_t a = ((o0 + 127u) & ~127u) + (uint32_t)(q * 32 + lane) * 128u;
                 if (a + 128u <= o0 + col_bytes)
                   asm volatile("discard.global.L2 [%0], 128;" ::"l"(qb + (a - mis)) : "memory");
-              } else if (p.discard_q) {
-                const int t = q * 32 + lane, pl = t >> 4, j = t & 15;
-                if (pl < NP) {
-                  // (single strip: H <= 128 rows = at most 16 lines per plane, one per lane)
-                  const char* qb = reinterpret_cast<const char*>(bufQ);
-                  const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(qb) & 127u);
-                  const uint32_t o0 = ((uint32_t)pl * (uint32_t)plane_stride + (uint32_t)(ob.w * H)) * 16u + mis;
-                  const uint32_t a = ((o0 + 127u) & ~127u) + (uint32_t)j * 128u;
-                  if (a + 128u <= o0 + (uint32_t)H * 16u)
-                    asm volatile("discard.global.L2 [%0], 128;" ::"l"(qb + (a - mis)) : "memory");
-                }
               }
               if constexpr (!SPLIT) { mbar_wait_sleepy(skfull_bar(g), eskpar); eskpar ^= 1u; }
             }
@@ -836,7 +820,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                 __syncwarp();
                 if (lane == 0) mbar_arrive(tempty_bar(ob.slot));   // all channels are in registers / stored, the slot is zero again
               }
-              if (valid && !(DBG && (p.diag & 1))) {
+              if (valid) {
                 uint4 ykeep = make_uint4(0u, 0u, 0u, 0u), ykeep_lo = make_uint4(0u, 0u, 0u, 0u);
                 const uint32_t swl = swl_of(jj), swl_lo = SPLIT ? swl_of(NKC + jj) : 0u;   // (SPLIT: the lo chunk's rows)
 #pragma unroll
@@ -899,9 +883,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                       if (hf == 0) ykeep = yo;
                       else st_hint256(y_out + jj * kc_stride + ob.off, swl ? yo : ykeep, swl ? ykeep : yo, pol_out);
                     } else {
-                      uint4* dst = y_out + (int64_t)(2 * jj + hf) * plane_stride + ob.off;
-                      if (use_pol) st_hint(dst, yo, pol_out);
-                      else *dst = yo;
+                      st_hint(y_out + (int64_t)(2 * jj + hf) * plane_stride + ob.off, yo, pol_out);
                     }
                   }
                 }
@@ -926,7 +908,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                   const uint32_t bytes = (uint32_t)(NKC * H) * 32u;
                   mbar_expect_tx(skfull_bar(g), bytes);
                   bulk_load_hint(sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT, skipP + (ob.w * NKC) * H * 2, bytes,
-                                 skfull_bar(g), pol_keep);
+                                 skfull_bar(g), l2_policy_evict_last());
                 }
               } else if (q == 0 && ob.exists && elect_one()) {
                 const int rows = H - ob.s * 128 < 128 ? H - ob.s * 128 : 128;
@@ -935,7 +917,7 @@ resnet_tc_sweep_kernel(const SwParams p) {
                 const uint32_t d0 = sbase + p.smem_skip_off + (uint32_t)g * SKIP_SLOT;
 #pragma unroll
                 for (int pl = 0; pl < NP; ++pl)
-                  bulk_load_hint(d0 + (uint32_t)pl * 2048u, src + (int64_t)pl * plane_stride, (uint32_t)(rows * 16), skfull_bar(g), pol_keep);
+                  bulk_load_hint(d0 + (uint32_t)pl * 2048u, src + (int64_t)pl * plane_stride, (uint32_t)(rows * 16), skfull_bar(g), l2_policy_evict_last());
               }
             }
           };

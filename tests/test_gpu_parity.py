@@ -714,27 +714,6 @@ def test_bf16_column_sweep_kernel_matches_position_major_kernel_at_full_batch(de
 
 
 @pytest.mark.parametrize("name", ["res15", "res15_narrow"])
-def test_bf16_sweep_kernel_planar_layout_matches_16_channel_row_layout(dev, monkeypatch, model_golden, name):
-    """The default activation layout for single-strip maps is [K chunk][w][h][16 channels] (swizzle-32B operand, one
-    bulk copy per K chunk, 32-byte stores); HONK2_TC_SWEEP_K32=0 selects the planar [8-channel plane][w][h] layout
-    that multi-strip maps use.  Same arithmetic: logits agree to accumulation-order noise, both with the golden."""
-    feats = torch.from_numpy(model_golden["feats"]).to(dev)
-    with torch.no_grad():
-        monkeypatch.setenv("HONK2_TC_SWEEP_K32", "0")
-        m_planar, _ = gpu_model(name, "hardened", dev, precision="bf16")
-        y_planar = m_planar(feats)
-        monkeypatch.setenv("HONK2_TC_SWEEP_K32", "1")
-        m_k32, _ = gpu_model(name, "hardened", dev, precision="bf16")
-        y_k32 = m_k32(feats)
-        y_again = m_k32(feats)
-    scale = float(y_planar.abs().max())
-    assert float((y_k32 - y_planar).abs().max()) <= 2e-3 * scale
-    assert float((y_k32 - y_again).abs().max()) <= 2e-3 * scale
-    assert logit_err(y_k32.cpu().numpy(), model_golden[f"{name}/hardened/logits"]) <= BF16_TOL
-    assert logit_err(y_planar.cpu().numpy(), model_golden[f"{name}/hardened/logits"]) <= BF16_TOL
-
-
-@pytest.mark.parametrize("name", ["res15", "res15_narrow"])
 def test_bf16_resnet_other_time_lengths(dev, name, model_golden):
     """T = 301 frames: the column-sweep kernel runs three 128-row strips per column (planar layout, one bulk copy per
     8-channel plane, pad rows re-zeroed at the map's top and bottom); checked against the reference golden."""
@@ -965,17 +944,35 @@ def test_packed_strips_ragged_batches_vs_oracle(dev, name, precision, tol):
 
 
 @pytest.mark.parametrize("name", ["res8", "res26"])
-def test_packed_strips_match_position_major_kernel(dev, monkeypatch, name):
+def test_packed_strips_match_position_major_reference(dev, monkeypatch, name):
+    """Pooled maps run as packed strips on the sweep kernel; HONK2_TC_SWEEP=0 runs them on the position-major kernel,
+    which has to agree within 1e-2 of the logit scale."""
     feats = torch.from_numpy(mfcc_ref.compute_mfccs_batch(synth.broadband(300, seed=13))).to(dev)
     with torch.no_grad():
         m_pack, _ = gpu_model(name, "hardened", dev, precision="bf16")
         y_pack = m_pack(feats)
         assert _kernel_path(m_pack, dev) == "resnet_tc_sweep_kernel"
-        monkeypatch.setenv("HONK2_TC_SWEEP_PACK", "0")
+        monkeypatch.setenv("HONK2_TC_SWEEP", "0")
         m_pos, _ = gpu_model(name, "hardened", dev, precision="bf16")
         y_pos = m_pos(feats)
         assert _kernel_path(m_pos, dev) == "resnet_tc_fused_kernel"
     assert float((y_pack - y_pos).abs().max()) <= 1e-2 * float(y_pos.abs().max())
+
+
+@pytest.mark.parametrize("name", ["res15", "res8"])
+def test_retired_tensor_core_variables_change_nothing(dev, monkeypatch, name):
+    """The layout, packing, L2 policy, barrier polling and stage count of the tensor-core kernels are decided by their
+    plans alone: variables that once overrode them are ignored, so the kernel and every logit bit stay the same."""
+    feats = torch.from_numpy(mfcc_ref.compute_mfccs_batch(synth.broadband(300, seed=17))).to(dev)
+    with torch.no_grad():
+        m, _ = gpu_model(name, "hardened", dev, precision="bf16")
+        path, y = _kernel_path(m, dev), m(feats)
+        for var, value in (("HONK2_TC_SWEEP_K32", "0"), ("HONK2_TC_SWEEP_PACK", "0"), ("HONK2_TC_L2POLICY", "0"),
+                           ("HONK2_TC_WAIT_POLLS", "0"), ("HONK2_TC_SWEEP_STAGES", "3")):
+            monkeypatch.setenv(var, value)
+        m_env, _ = gpu_model(name, "hardened", dev, precision="bf16")
+        assert _kernel_path(m_env, dev) == path == "resnet_tc_sweep_kernel"
+        assert torch.equal(m_env(feats), y)
 
 
 SHORT_CLIP_PATHS = {("res15", 50): "resnet_tc_sweep_kernel", ("res15", 33): "resnet_tc_sweep_kernel",

@@ -138,7 +138,7 @@ def _variant(row, precision):
     ph, pw = row.pool or (1, 1)
     H = row.T // ph
     strips = -(-H // 128)
-    packed = row.pool is not None or H * 100 < strips * 128 * 60
+    packed = row.pool is not None or H * 100 < strips * 128 * 60   # 60: kSwMinStripPct in conv_tc.cu
     layout = "packed" if packed else "32B" if strips == 1 else "planar"
     if precision == "bf16x3":
         assert layout != "planar", row.id
