@@ -14,7 +14,7 @@ from .zoo import MODEL_ZOO, model_config  # noqa: F401
 from ._native import NativeError  # noqa: F401
 from .profile import profile_layers  # noqa: F401
 from .workspace import load_checkpoint, strip_data_parallel_prefix  # noqa: F401
-from .streaming import n_stream_windows, stream_window_targets, evaluate_stream, LiveStreams  # noqa: F401
+from .streaming import n_stream_windows, stream_window_targets, evaluate_stream, LiveStreams, LiveCNN  # noqa: F401
 from .data_loader import AudioDataLoader  # noqa: F401
 from . import metric  # noqa: F401  (registers metric.Acc, metric.PerClassAcc, loss_fn.ce_loss)
 

@@ -12,8 +12,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libhonk2_b200.so")
-SOURCES = ["api.cu", "mfcc.cu", "resnet_fp32.cu", "cnn_fp32.cu", "cnn_tc.cu", "conv_tc.cu", "model.cu"]
-HEADERS = ["common.cuh", "kernels.cuh", "tc.cuh", "ptx.cuh", "resnet_fused.cuh", "resnet_sweep.cuh", os.path.join("..", "..", "include", "honk2_b200.h")]
+SOURCES = ["api.cu", "mfcc.cu", "resnet_fp32.cu", "cnn_fp32.cu", "cnn_tc.cu", "conv_tc.cu", "model.cu", "live_cnn.cu"]
+HEADERS = ["common.cuh", "kernels.cuh", "live.cuh", "tc.cuh", "ptx.cuh", "resnet_fused.cuh", "resnet_sweep.cuh", os.path.join("..", "..", "include", "honk2_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wno-stringop-overflow"]
 

@@ -41,21 +41,9 @@ constexpr int kCnnWorkers = 16;          // worker warps: A_e builder + epilogue
 constexpr int kCnnThreads = 32 * (4 + kCnnWorkers);   // warps 0, 1, 3 issue, warp 2 streams conv_1's weights
 constexpr int kCnnRingUnit = 4 * 2 * kCnnC * 16;   // one (kh, kw) tap of conv_1: 4 K chunks x 2 halves x 64 x 16 B = 8 KB
 constexpr int kCnnMaxRing = 8;
-constexpr int kLin0Split = 8;         // split-K factor of the first Linear
+constexpr int kLin0Split = kTcCnnLin0Split;   // split-K factor of the first Linear
 constexpr int kLin0Warps = 4;         // warps (16 utterances each) per CTA of the first Linear
 constexpr int kLin0N = 32;            // padded outputs of the first Linear
-
-struct TcCnnGeom {
-  int T, F, KH0, KW0, H0, WP, KH1, KW1, H1;
-  int n0;        // pooled rows = H0 * WP
-  int tiles0;    // conv_0 M-tiles per pool member
-  int ks0;       // conv_0 K steps (two kernel rows each)
-  int tiles1;    // conv_1 M-tiles (16 output rows each)
-  int units1;    // KH1 * KW1 weight units
-  int a_rows;    // rows of an A_e array (T*WP + WP zero rows)
-  int off_w0, off_a, a_bytes, off_pool, plane_bytes, off_ring, n_ring;
-  int smem_bytes;
-};
 
 struct TcCnnParams {
   const float* feat;            // [B][T][F]
@@ -386,8 +374,10 @@ __device__ __forceinline__ void mma_bf16_16816(float (&c)[4], uint32_t a0, uint3
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
+// ROWS says where row r's activations are (DenseActRows, LiveActRows: tc.cuh).
+template <typename ROWS>
 __global__ void __launch_bounds__(32 * kLin0Warps)
-cnn_lin0_kernel(const __nv_bfloat16* __restrict__ act, const __nv_bfloat16* __restrict__ w, float* __restrict__ partial,
+cnn_lin0_kernel(const ROWS rows, const __nv_bfloat16* __restrict__ w, float* __restrict__ partial,
                 int64_t B, int K, int k_per_split) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int gq = lane >> 2, tq = lane & 3;
@@ -396,8 +386,7 @@ cnn_lin0_kernel(const __nv_bfloat16* __restrict__ act, const __nv_bfloat16* __re
   const int split = blockIdx.y;
   const int k0 = split * k_per_split, k1 = min(K, k0 + k_per_split);
   const int64_t ra = min(row0 + gq, B - 1), rb = min(row0 + gq + 8, B - 1);
-  const uint4* pa = reinterpret_cast<const uint4*>(act + ra * K) + tq;
-  const uint4* pb = reinterpret_cast<const uint4*>(act + rb * K) + tq;
+  const typename ROWS::Cursor pa = rows.row(ra, K, tq), pb = rows.row(rb, K, tq);
   const uint4* pw[4];
 #pragma unroll
   for (int nt = 0; nt < 4; ++nt) pw[nt] = reinterpret_cast<const uint4*>(w + (int64_t)(8 * nt + gq) * K) + tq;
@@ -409,7 +398,7 @@ cnn_lin0_kernel(const __nv_bfloat16* __restrict__ act, const __nv_bfloat16* __re
 #pragma unroll 4
   for (int k = k0; k < k1; k += 32) {
     const int o = k >> 3;
-    const uint4 a = __ldcs(pa + o), bq = __ldcs(pb + o);
+    const uint4 a = __ldcs(pa.at(o)), bq = __ldcs(pb.at(o));
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt) {
       const uint4 wv = __ldg(pw[nt] + o);
@@ -526,6 +515,7 @@ struct TcCnn {
   int first = -1;              // index (0 lin_0, 1 dnn_0, 2 dnn_1, 3 lin_1) of the first Linear
   int lin_in[4] = {0, 0, 0, 0}, lin_out[4] = {0, 0, 0, 0};
   unsigned char* blob = nullptr;
+  size_t blob_bytes = 0;
   __nv_bfloat16 *w0 = nullptr, *w1 = nullptr, *wl = nullptr;
   float *b0 = nullptr, *b1 = nullptr;
   float* lin_w[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -608,6 +598,7 @@ int tc_cnn_create(const kws_cnn_config& cfg, TcCnn** out) {
       o_lb[i] = take(sizeof(float) * p->lin_out[i]);
       if (i != p->first) o_lw[i] = take(sizeof(float) * (size_t)p->lin_out[i] * p->lin_in[i]);
     }
+  p->blob_bytes = off;
   cudaError_t e = cudaMalloc(&p->blob, off);
   if (e != cudaSuccess) {
     set_error("tc_cnn_create: cudaMalloc(%zu) failed: %s", off, cudaGetErrorString(e));
@@ -728,7 +719,8 @@ int tc_cnn_forward(TcCnn* p, const float* feat, int64_t B, int T, int F, float* 
     }
     if (prof) prof->tick(1, st);
     const int k_per = round_up(ceil_div(K, kLin0Split), 32);
-    cnn_lin0_kernel<<<dim3((unsigned)ceil_div<int64_t>(nb, 16 * kLin0Warps), kLin0Split), 32 * kLin0Warps, 0, st>>>(act, p->wl, partial, nb, K, k_per);
+    cnn_lin0_kernel<<<dim3((unsigned)ceil_div<int64_t>(nb, 16 * kLin0Warps), kLin0Split), 32 * kLin0Warps, 0, st>>>(
+        DenseActRows{act}, p->wl, partial, nb, K, k_per);
     KWS_CHECK_LAUNCH();
     MlpParams mp{};
     mp.partial = partial;
@@ -743,6 +735,58 @@ int tc_cnn_forward(TcCnn* p, const float* feat, int64_t B, int T, int F, float* 
     cnn_mlp_kernel<<<(unsigned)ceil_div<int64_t>(nb, kMlpUtt), 256, 0, st>>>(mp);
     KWS_CHECK_LAUNCH();
   }
+  return KWS_OK;
+}
+
+bool tc_cnn_view(const TcCnn* p, TcCnnView* v) {
+  if (!p || !p->supported) return false;
+  v->g = p->g;
+  v->w0 = p->w0; v->w1 = p->w1; v->b0 = p->b0; v->b1 = p->b1;
+  v->blob_bytes = p->blob_bytes;
+  v->n_labels = 0;
+  for (int i = 0; i < 4; ++i) if (p->lin_out[i] > 0) v->n_labels = p->lin_out[i];
+  return true;
+}
+
+int tc_cnn_copy(const TcCnn* src, TcCnn** out, cudaStream_t st) {
+  *out = nullptr;
+  KWS_REQUIRE(src != nullptr && src->supported, "CNN: no tensor-core path for this configuration");
+  TcCnn* p = nullptr;
+  KWS_TRY(tc_cnn_create(src->cfg, &p));
+  if (p->blob_bytes != src->blob_bytes) {
+    tc_cnn_destroy(p);
+    set_error("tc_cnn_copy: plans of one configuration differ in size");
+    return KWS_ERR_INVALID;
+  }
+  const cudaError_t e = cudaMemcpyAsync(p->blob, src->blob, src->blob_bytes, cudaMemcpyDeviceToDevice, st);
+  if (e != cudaSuccess) {
+    tc_cnn_destroy(p);
+    set_error("tc_cnn_copy: %s", cudaGetErrorString(e));
+    return KWS_ERR_CUDA;
+  }
+  *out = p;
+  return KWS_OK;
+}
+
+int tc_cnn_live_linear(const TcCnn* p, const LiveActRows& rows, int64_t B, float* partial, float* logits,
+                       cudaStream_t st) {
+  KWS_REQUIRE(p != nullptr && p->supported, "CNN: no tensor-core path for this configuration");
+  const int K = p->g.H1 * 8 * kCnnC;
+  const int k_per = round_up(ceil_div(K, kLin0Split), 32);   // the batch path's split-K slices
+  cnn_lin0_kernel<<<dim3((unsigned)ceil_div<int64_t>(B, 16 * kLin0Warps), kLin0Split), 32 * kLin0Warps, 0, st>>>(
+      rows, p->wl, partial, B, K, k_per);
+  KWS_CHECK_LAUNCH();
+  MlpParams mp{};
+  mp.partial = partial;
+  mp.bias_first = p->lin_b[p->first];
+  mp.first_out = p->lin_out[p->first];
+  mp.n_layers = 0;
+  for (int i = p->first + 1; i < 4; ++i)
+    if (p->lin_out[i] > 0) mp.layer[mp.n_layers++] = MlpLayer{p->lin_w[i], p->lin_b[i], p->lin_in[i], p->lin_out[i]};
+  mp.logits = logits;
+  mp.B = B;
+  cnn_mlp_kernel<<<(unsigned)ceil_div<int64_t>(B, kMlpUtt), 256, 0, st>>>(mp);
+  KWS_CHECK_LAUNCH();
   return KWS_OK;
 }
 

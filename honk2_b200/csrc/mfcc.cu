@@ -12,6 +12,7 @@
 // A warp works on two frames at a time (one per half-warp); a CTA stages the 2880 samples its
 // 16 frames cover once (coalesced loads, reflect indexing at the clip edges).
 #include "common.cuh"
+#include "live.cuh"
 #include <cub/device/device_scan.cuh>
 #include <cmath>
 #include <vector>
@@ -229,6 +230,14 @@ struct RingSource {
       const int64_t r = (count[b] - n) / kHop - 1 + t;
       return feat + (b * (int64_t)fcap + pos_mod(r, fcap)) * n_mels;
     }
+  }
+};
+
+// EdgeRingSource (kws_live_cnn): RingSource<true>'s window slots, but only the four edge frames of a slot are stored,
+// dense [S K][4][n_mels] (frames t = 0, 1, T-2, T-1 in that order).
+struct EdgeRingSource : RingSource<true> {
+  __device__ __forceinline__ float* out_row(float* feat, int64_t b, int T, int t, int n_mels) const {
+    return feat + (b * 4 + (t < 2 ? t : t - T + 4)) * n_mels;
   }
 };
 
@@ -772,6 +781,9 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
     e = cudaFuncSetAttribute(mfcc_kernel<true, float, RingSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)fe->smem_bytes_edges);
   if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(mfcc_kernel<true, float, EdgeRingSource>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)fe->smem_bytes_edges);
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(mfcc_kernel<false, float, RaggedSource<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)fe->smem_bytes_edges);
   if (e == cudaSuccess)
@@ -904,17 +916,7 @@ extern "C" int kws_mfcc_stream_forward_pcm16(const kws_frontend_t* fe, const int
 // One device allocation per state: sample rings [S][cap] f32, frame rings [S][fcap][n_mels] f32, counters [S] i64,
 // first-window ring positions [S] i32.  Ragged pushes add a pinned host staging buffer for their per-stream sample
 // offsets and lengths and the event that marks its last copy done; both are created by the first ragged push.
-struct kws_live {
-  const kws_frontend* fe;
-  int S, window, shift, max_push, T, cap, fcap;
-  void* dev;
-  float* ring;
-  float* frames;
-  int64_t* count;
-  int* wpos;
-  void* ragged_host = nullptr;
-  cudaEvent_t ragged_copied = nullptr;
-};
+// (struct kws_live: live.cuh)
 
 namespace {
 struct LiveLayout {
@@ -992,15 +994,15 @@ extern "C" int kws_live_reset(kws_live_t* live, const int64_t* stream_ids, int64
   return KWS_OK;
 }
 
+namespace kws {
 template <typename SMP>
-static int live_push_any(const char* who, kws_live_t* L, const SMP* chunk, int n, float* feat, void* stream) {
+int live_append_rows(const char* who, kws_live_t* L, const SMP* chunk, int n, cudaStream_t st) {
   KWS_REQUIRE(L != nullptr, "%s: live state is null", who);
   KWS_REQUIRE(n >= 1 && n <= L->max_push && n % L->shift == 0,
               "%s: a push of %d samples per stream: need a multiple of the shift %d in [%d, %d]", who, n, L->shift,
               L->shift, L->max_push);
-  KWS_REQUIRE(chunk != nullptr && feat != nullptr, "%s: null buffer", who);
+  KWS_REQUIRE(chunk != nullptr, "%s: null buffer", who);
   const kws_frontend* fe = L->fe;
-  cudaStream_t st = as_stream(stream);
   const int K = n / L->shift;
   const int64_t slots = (int64_t)L->S * K;
   const int rows = n / kHop;
@@ -1017,6 +1019,31 @@ static int live_push_any(const char* who, kws_live_t* L, const SMP* chunk, int n
       fe->t, RingSource<false>{L->ring, L->count, L->wpos, L->cap, n, L->fcap, L->shift, K, (int)slots}, (int64_t)L->S, 0,
       rows, tiles, L->frames);
   KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+template int live_append_rows<float>(const char*, kws_live_t*, const float*, int, cudaStream_t);
+template int live_append_rows<int16_t>(const char*, kws_live_t*, const int16_t*, int, cudaStream_t);
+
+int live_edge_frames(kws_live_t* L, int n, float* edges, cudaStream_t st) {
+  const int K = n / L->shift;
+  const int64_t slots = (int64_t)L->S * K;
+  mfcc_kernel<true, float, EdgeRingSource><<<(unsigned)ceil_div<int64_t>(slots, 4), kMfccThreads,
+                                             L->fe->smem_bytes_edges, st>>>(
+      L->fe->t, EdgeRingSource{{L->ring, L->count, L->wpos, L->cap, n, L->fcap, L->shift, K, (int)slots}}, slots,
+      L->window, L->T, 1, edges);
+  KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+}  // namespace kws
+
+template <typename SMP>
+static int live_push_any(const char* who, kws_live_t* L, const SMP* chunk, int n, float* feat, void* stream) {
+  KWS_REQUIRE(feat != nullptr || L == nullptr, "%s: null buffer", who);
+  cudaStream_t st = as_stream(stream);
+  KWS_TRY(live_append_rows(who, L, chunk, n, st));
+  const kws_frontend* fe = L->fe;
+  const int K = n / L->shift;
+  const int64_t slots = (int64_t)L->S * K;
   // 3) the four reflect-padded edge frames of each of the S K new windows
   mfcc_kernel<true, float, RingSource<true>><<<(unsigned)ceil_div<int64_t>(slots, 4), kMfccThreads, fe->smem_bytes_edges,
                                                st>>>(

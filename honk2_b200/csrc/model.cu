@@ -100,6 +100,11 @@ using namespace kws;
 
 struct kws_model : kws::Model {};
 
+const TcCnn* kws::model_tc_cnn(const kws_model_t* m, bool* weights_set) {
+  *weights_set = m && m->weights_set;
+  return m && m->kind == KIND_CNN ? m->tcc : nullptr;
+}
+
 // =============================================================================================
 // ResNet
 

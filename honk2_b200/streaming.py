@@ -110,7 +110,114 @@ def ragged_push_plan(seen, lengths, window_size, shift_size):
     return RaggedPlan(stream_ids, window_ids, int((-(-n // 160)).sum()), int((-(-n // shift_size)).sum()))
 
 
-class LiveStreams(object):
+class _LiveState(object):
+    """What the live states share: device selection, the host's copy of the sample counters, the checks of a uniform
+    push's chunk, the validity mask of its slots, reset and pickling.  Subclasses name their C functions
+    (``_create``, ``_reset_fn``, ``_destroy_fn``) and add their own device buffers."""
+    _kind = "live state"
+
+    def __init__(self, audio_processor, n_streams, window_size, shift_size, max_push, device):
+        self.audio_processor = audio_processor   # owns the front-end tables the state reads
+        self.n_streams = int(n_streams)
+        self.window_size = int(window_size)
+        self.shift_size = int(shift_size)
+        self.max_push = int(max_push)
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev.type != "cuda":
+            raise _native.NativeError(f"{type(self).__name__} needs a CUDA device: there is no CPU path")
+        self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
+        self.n_frames = audio_processor.n_frames(self.window_size)
+        self._handle = None
+        self._seen = np.zeros(self.n_streams, dtype=np.int64)
+
+    def _state(self):
+        if self._handle is None:
+            self._handle = self._create(_native.load())
+            self._seen[:] = 0
+            # reset's stream ids: pinned staging buffer, device copy, and the event that marks the staging buffer free
+            self._ids_host = torch.empty(self.n_streams, dtype=torch.int64, pin_memory=True)
+            self._ids_dev = torch.empty(self.n_streams, dtype=torch.int64, device=self.device)
+            self._ids_copied = torch.cuda.Event()
+        return self._handle
+
+    @property
+    def samples_seen(self):
+        """Samples pushed into each stream since its last reset: CPU int64 [S]."""
+        return torch.from_numpy(self._seen.copy())
+
+    def _check_chunk(self, chunk):
+        """A uniform push's chunk as the C call takes it: (contiguous chunk, pcm16?)."""
+        name = type(self).__name__
+        if not (isinstance(chunk, torch.Tensor) and chunk.is_cuda):
+            raise _native.NativeError(f"{name}.push needs a CUDA tensor: there is no CPU path")
+        if chunk.dim() != 2 or chunk.shape[0] != self.n_streams:
+            raise ValueError(f"expected a chunk shaped [{self.n_streams}, n], got {tuple(chunk.shape)}")
+        if chunk.device != self.device:
+            raise ValueError(f"the chunk is on {chunk.device}, the live state on {self.device}")
+        misaligned = np.flatnonzero(self._seen % 160)
+        if misaligned.size:
+            s = int(misaligned[0])
+            raise ValueError(f"stream {s} has seen {int(self._seen[s])} samples, not a multiple of the 160-sample hop "
+                             "(a ragged push left it so); push needs aligned counts: use push_ragged")
+        pcm16 = chunk.dtype == torch.int16
+        if not pcm16 and chunk.dtype != torch.float32:
+            chunk = chunk.float()
+        return chunk.contiguous(), pcm16
+
+    def _advance(self, n):
+        """After a uniform push of n samples: the host-side validity mask [S, K] of its slots; counters advance."""
+        # window index of slot j: floor((c - W) / H) + 1 + j, c = samples before this push
+        first = (self._seen - self.window_size) // self.shift_size + 1
+        valid = torch.from_numpy(first[:, None] + np.arange(n // self.shift_size)[None, :] >= 0)
+        self._seen += n
+        return valid
+
+    def reset(self, stream_ids):
+        """Restart the given streams at sample 0; the others are not affected.  stream_ids: host integers (a list, a
+        numpy array or a CPU tensor) in [0, S); repeats are allowed."""
+        if isinstance(stream_ids, torch.Tensor) and stream_ids.is_cuda:
+            raise ValueError("reset takes host stream ids: the host checks them and keeps samples_seen")
+        ids = np.unique(np.asarray(stream_ids, dtype=np.int64).reshape(-1))
+        if ((ids < 0) | (ids >= self.n_streams)).any():
+            raise ValueError(f"stream ids must lie in [0, {self.n_streams})")
+        if ids.size == 0:
+            return
+        lib = _native.load()
+        handle = self._state()
+        m = ids.size
+        st = torch.cuda.current_stream(self.device)
+        self._ids_copied.synchronize()   # the previous reset's copy out of the staging buffer (long done, in practice)
+        self._ids_host[:m].copy_(torch.from_numpy(ids))
+        with torch.cuda.device(self.device):
+            self._ids_dev[:m].copy_(self._ids_host[:m], non_blocking=True)
+            self._ids_copied.record(st)
+            _native.check(getattr(lib, self._reset_fn)(handle, C.c_void_p(self._ids_dev.data_ptr()), m,
+                                                       C.c_void_p(st.cuda_stream)), self._reset_fn)
+        self._seen[ids] = 0
+
+    def __del__(self):
+        try:
+            lib = _native.loaded()   # (never dlopen from a destructor)
+            if lib is not None and self._handle is not None:
+                getattr(lib, self._destroy_fn)(self._handle)
+                self._handle = None
+        except Exception:
+            pass
+
+    _device_buffers = ()
+
+    def __getstate__(self):  # device state never crosses a process boundary
+        d = dict(self.__dict__)
+        d["_handle"] = None
+        for k in self._device_buffers:
+            d[k] = None
+        d["_seen"] = np.zeros_like(self._seen)
+        for k in ("_ids_host", "_ids_dev", "_ids_copied"):
+            d.pop(k, None)
+        return d
+
+
+class LiveStreams(_LiveState):
     """Live keyword-spotting front-end for ``n_streams`` microphones, fed a chunk at a time (``kws_live_*``).
 
     Each stream keeps a device-resident sample ring, frame ring and sample counter.  ``push(chunk)`` hands every stream
@@ -131,43 +238,21 @@ class LiveStreams(object):
 
     ``push_ragged(samples, lengths)`` lets every stream bring its own number of samples, and returns only the windows
     the push completes, compacted, with the stream and window index of each (see ``ragged_push_plan``)."""
+    _reset_fn, _destroy_fn = "kws_live_reset", "kws_live_destroy"
+    _device_buffers = ("_ragged_ws",)
 
     def __init__(self, audio_processor, n_streams, window_size=16000, shift_size=160, max_push=1600, device=None):
-        self.audio_processor = audio_processor   # owns the front-end tables the state reads
-        self.n_streams = int(n_streams)
-        self.window_size = int(window_size)
-        self.shift_size = int(shift_size)
-        self.max_push = int(max_push)
-        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if dev.type != "cuda":
-            raise _native.NativeError("LiveStreams needs a CUDA device: there is no CPU path")
-        self.device = torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
-        self.n_frames = audio_processor.n_frames(self.window_size)
-        self._handle = None
+        super().__init__(audio_processor, n_streams, window_size, shift_size, max_push, device)
         self._ragged_ws = None   # device workspace of push_ragged, allocated by the first ragged push
-        self._seen = np.zeros(self.n_streams, dtype=np.int64)
         self._state()
 
-    def _state(self):
-        if self._handle is None:
-            lib = _native.load()
-            fe = self.audio_processor._frontend(self.device)
-            out = C.c_void_p()
-            with torch.cuda.device(self.device):
-                _native.check(lib.kws_live_create(fe, self.n_streams, self.window_size, self.shift_size, self.max_push,
-                                                  C.byref(out)), "kws_live_create")
-            self._handle = out
-            self._seen[:] = 0
-            # reset's stream ids: pinned staging buffer, device copy, and the event that marks the staging buffer free
-            self._ids_host = torch.empty(self.n_streams, dtype=torch.int64, pin_memory=True)
-            self._ids_dev = torch.empty(self.n_streams, dtype=torch.int64, device=self.device)
-            self._ids_copied = torch.cuda.Event()
-        return self._handle
-
-    @property
-    def samples_seen(self):
-        """Samples pushed into each stream since its last reset: CPU int64 [S]."""
-        return torch.from_numpy(self._seen.copy())
+    def _create(self, lib):
+        fe = self.audio_processor._frontend(self.device)
+        out = C.c_void_p()
+        with torch.cuda.device(self.device):
+            _native.check(lib.kws_live_create(fe, self.n_streams, self.window_size, self.shift_size, self.max_push,
+                                              C.byref(out)), "kws_live_create")
+        return out
 
     def state_bytes(self):
         """Device bytes the state holds (kws_live_state_bytes)."""
@@ -183,21 +268,7 @@ class LiveStreams(object):
         Every stream's sample count must be a multiple of 160 (the hop).  Only ``push_ragged`` can break that; after a
         ragged push that leaves a count unaligned, ``push`` raises ValueError and changes nothing, until ragged pushes
         (or a reset) realign the counts."""
-        if not (isinstance(chunk, torch.Tensor) and chunk.is_cuda):
-            raise _native.NativeError("LiveStreams.push needs a CUDA tensor: there is no CPU path")
-        if chunk.dim() != 2 or chunk.shape[0] != self.n_streams:
-            raise ValueError(f"expected a chunk shaped [{self.n_streams}, n], got {tuple(chunk.shape)}")
-        if chunk.device != self.device:
-            raise ValueError(f"the chunk is on {chunk.device}, the live state on {self.device}")
-        misaligned = np.flatnonzero(self._seen % 160)
-        if misaligned.size:
-            s = int(misaligned[0])
-            raise ValueError(f"stream {s} has seen {int(self._seen[s])} samples, not a multiple of the 160-sample hop "
-                             "(a ragged push left it so); push needs aligned counts: use push_ragged")
-        pcm16 = chunk.dtype == torch.int16
-        if not pcm16 and chunk.dtype != torch.float32:
-            chunk = chunk.float()
-        chunk = chunk.contiguous()
+        chunk, pcm16 = self._check_chunk(chunk)
         n = chunk.shape[1]
         K = n // self.shift_size
         shape = (self.n_streams, K, self.n_frames, self.audio_processor.n_mels)
@@ -212,10 +283,7 @@ class LiveStreams(object):
             _native.check(fn(handle, C.c_void_p(chunk.data_ptr()), n, C.c_void_p(out.data_ptr()),
                              C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
                           "kws_live_push_pcm16" if pcm16 else "kws_live_push")
-        # window index of slot j: floor((c - W) / H) + 1 + j, c = samples before this push
-        first = (self._seen - self.window_size) // self.shift_size + 1
-        valid = torch.from_numpy(first[:, None] + np.arange(K)[None, :] >= 0)
-        self._seen += n
+        valid = self._advance(n)
         if model is None:
             return out, valid
         logits = model(out.view(self.n_streams * K, self.n_frames, self.audio_processor.n_mels))
@@ -284,43 +352,79 @@ class LiveStreams(object):
             return (torch.empty((0, model.n_labels), dtype=torch.float32, device=self.device),) + ids
         return (model(feats),) + ids
 
-    def reset(self, stream_ids):
-        """Restart the given streams at sample 0; the others are not affected.  stream_ids: host integers (a list, a
-        numpy array or a CPU tensor) in [0, S); repeats are allowed."""
-        if isinstance(stream_ids, torch.Tensor) and stream_ids.is_cuda:
-            raise ValueError("reset takes host stream ids: the host checks them and keeps samples_seen")
-        ids = np.unique(np.asarray(stream_ids, dtype=np.int64).reshape(-1))
-        if ((ids < 0) | (ids >= self.n_streams)).any():
-            raise ValueError(f"stream ids must lie in [0, {self.n_streams})")
-        if ids.size == 0:
-            return
+
+
+class LiveCNN(_LiveState):
+    """Live keyword spotting with a CNN for ``n_streams`` microphones (``kws_live_cnn_*``): a live front-end and the
+    bf16 tensor-core CNN in one state, where each push returns the logits of the windows it completes.
+
+    The slots, the validity mask, ``samples_seen`` and ``reset`` are those of ``LiveStreams``.  The CNN's convolutions
+    do not pad in time, so a window's convolution rows are its stream's rows except the four of each convolution that
+    read the window's reflect-padded edge frames: a push computes n / 160 new rows of each convolution per stream and
+    those four per window, instead of the whole network per window.  The logits are bit-identical to
+    ``LiveStreams.push(chunk, model)`` on the same audio.
+
+    ``model`` must be a ``honk2_b200.CNN`` with ``precision == "bf16"`` whose shape has the tensor-core path, and
+    ``1 + window_size / 160`` must be its ``time``.  The state copies the model's weights when it is created: later
+    changes to the model do not reach it.  ``max_push`` defaults to 10 shifts."""
+    _reset_fn, _destroy_fn = "kws_live_cnn_reset", "kws_live_cnn_destroy"
+
+    def __init__(self, model, n_streams, window_size=16000, shift_size=160, max_push=None, audio_processor=None,
+                 device=None):
+        from .model import CNN
+        if not isinstance(model, CNN):
+            raise ValueError(f"LiveCNN runs a honk2_b200.CNN, got {type(model).__name__}")
+        if model.precision != "bf16":
+            raise ValueError(f"LiveCNN runs the bf16 tensor-core CNN; the model's precision is {model.precision!r}")
+        if max_push is None:
+            max_push = 10 * int(shift_size)
+        super().__init__(audio_processor if audio_processor is not None else AudioProcessor(), n_streams, window_size,
+                         shift_size, max_push, device)
+        self.n_labels = model.n_labels
+        self._model = model   # held until the state exists; the state keeps its own copy of the weights
+        self._state()
+        self._model = None
+
+    def _model_handle(self, lib):
+        model = self._model
+        if model is None:
+            raise _native.NativeError("a LiveCNN restored from a pickle has no model to copy the weights from")
+        _, st = model._state(self.device)   # packs the current weights
+        return st["handle"]
+
+    def _create(self, lib):
+        fe = self.audio_processor._frontend(self.device)
+        out = C.c_void_p()
+        with torch.cuda.device(self.device):
+            handle = self._model_handle(lib)
+            _native.check(lib.kws_live_cnn_create(handle, fe, self.n_streams, self.window_size, self.shift_size,
+                                                  self.max_push, C.byref(out)), "kws_live_cnn_create")
+            self._state_bytes = int(lib.kws_live_cnn_state_bytes(handle, fe, self.n_streams, self.window_size,
+                                                                 self.shift_size, self.max_push))
+        return out
+
+    def state_bytes(self):
+        """Device bytes the state holds (kws_live_cnn_state_bytes)."""
+        if self._handle is None:
+            raise _native.NativeError("the state holds no device memory")
+        return self._state_bytes
+
+    def push(self, chunk, out=None):
+        """chunk: CUDA [S, n] float32 or int16 PCM, n a multiple of ``shift_size`` in ``[shift_size, max_push]``.
+        Returns (logits [S, K, n_labels], valid [S, K] CPU bool), K = n / shift_size; invalid slots are all zeros.
+        ``out``: optional preallocated logits buffer."""
+        chunk, pcm16 = self._check_chunk(chunk)
+        n = chunk.shape[1]
+        shape = (self.n_streams, n // self.shift_size, self.n_labels)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.float32, device=self.device)
+        elif out.shape != shape or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 {list(shape)} tensor on {self.device}")
         lib = _native.load()
         handle = self._state()
-        m = ids.size
-        st = torch.cuda.current_stream(self.device)
-        self._ids_copied.synchronize()   # the previous reset's copy out of the staging buffer (long done, in practice)
-        self._ids_host[:m].copy_(torch.from_numpy(ids))
+        fn = lib.kws_live_cnn_push_pcm16 if pcm16 else lib.kws_live_cnn_push
         with torch.cuda.device(self.device):
-            self._ids_dev[:m].copy_(self._ids_host[:m], non_blocking=True)
-            self._ids_copied.record(st)
-            _native.check(lib.kws_live_reset(handle, C.c_void_p(self._ids_dev.data_ptr()), m,
-                                             C.c_void_p(st.cuda_stream)), "kws_live_reset")
-        self._seen[ids] = 0
-
-    def __del__(self):
-        try:
-            lib = _native.loaded()   # (never dlopen from a destructor)
-            if lib is not None and self._handle is not None:
-                lib.kws_live_destroy(self._handle)
-                self._handle = None
-        except Exception:
-            pass
-
-    def __getstate__(self):  # device state never crosses a process boundary
-        d = dict(self.__dict__)
-        d["_handle"] = None
-        d["_ragged_ws"] = None
-        d["_seen"] = np.zeros_like(self._seen)
-        for k in ("_ids_host", "_ids_dev", "_ids_copied"):
-            d.pop(k, None)
-        return d
+            _native.check(fn(handle, C.c_void_p(chunk.data_ptr()), n, C.c_void_p(out.data_ptr()),
+                             C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
+                          "kws_live_cnn_push_pcm16" if pcm16 else "kws_live_cnn_push")
+        return out, self._advance(n)

@@ -141,6 +141,35 @@ int kws_live_push_ragged_pcm16(kws_live_t* live, const int16_t* samples, const i
                                int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
                                void* workspace, size_t ws_bytes, void* stream);
 
+/* Live CNN streams: a live front-end (above) feeding a CNN of the bf16 tensor-core family (cnn-trad-fpool3 and the
+ * shapes kws_cnn_create gives that path), where each push returns the logits of the windows it completes.  Neither
+ * convolution pads in time, so a window's convolution rows are the stream's rows except the four of each convolution
+ * that read its reflect-padded edge frames: a push computes n / 160 new rows of each convolution per stream plus those
+ * four per window, not the whole network per window (DESIGN.md section 7).
+ *   kws_live_cnn_state_bytes  device bytes kws_live_cnn_create allocates (0 on invalid or unsupported arguments).
+ *   kws_live_cnn_create   copies the model's packed bf16 weights: the state runs the weights the model had then, and
+ *                         the model may change or go away afterwards.  Refuses with KWS_ERR_UNSUPPORTED a ResNet, a CNN
+ *                         without the bf16 tensor-core path, and a window whose 1 + window / 160 frames differ from
+ *                         the CNN's time; with KWS_ERR_INVALID whatever kws_live_create refuses and a model whose
+ *                         weights were never set.  The front-end must outlive the state.
+ *   kws_live_cnn_push     chunk [S, n] f32, n a multiple of the shift in [shift, max_push], as kws_live_push; logits
+ *                         [S, K, n_labels] (K = n / shift) receive the logits of slot j = window
+ *                         floor((c_s - window) / shift) + 1 + j of each stream; warm-up slots (k < 0) are all zeros.
+ *                         Same precondition as kws_live_push.  The logits are bit-identical to the bf16 model
+ *                         (kws_model_forward) on the materialised windows' features.
+ *   kws_live_cnn_push_pcm16  the same on int16 PCM: bit-identical to a float push of s/32768.
+ *   kws_live_cnn_reset    as kws_live_reset.
+ * Push and reset allocate nothing and do not synchronise the host. */
+typedef struct kws_live_cnn kws_live_cnn_t;
+size_t kws_live_cnn_state_bytes(const kws_model_t* m, const kws_frontend_t* fe, int n_streams, int window, int shift,
+                                int max_push);
+int kws_live_cnn_create(const kws_model_t* m, const kws_frontend_t* fe, int n_streams, int window, int shift,
+                        int max_push, kws_live_cnn_t** out);
+void kws_live_cnn_destroy(kws_live_cnn_t* lc);
+int kws_live_cnn_reset(kws_live_cnn_t* lc, const int64_t* stream_ids, int64_t count, void* stream);
+int kws_live_cnn_push(kws_live_cnn_t* lc, const float* chunk, int n, float* logits, void* stream);
+int kws_live_cnn_push_pcm16(kws_live_cnn_t* lc, const int16_t* chunk, int n, float* logits, void* stream);
+
 /* ---- models: replace model.ResNet / model.CNN ---------------------------------------------
  * kws_resnet_create <- ResNet.__init__ (model/resnet.py:11-36); pool_h = pool_w = 0 when the
  *                      config has no "pool" key.

@@ -32,6 +32,16 @@ paths run on two states fed the same audio and are timed alternately in the same
   model     push_ragged(x, model) against push(x, model), bf16, at --model-streams streams: during the warm-up of fresh
             streams (the 99 pushes of 160 samples before the first window completes: the uniform push runs the model on
             S all-zero slots, the ragged push on none) and in the steady state (both run it on S windows)
+
+    python tools/live_bench.py --cnn [--streams 148,1024,8192] [--push-ms 10,100] [--dtypes float32,int16]
+                                     [--kernel-only] [--seconds 2] [--reps 3] [--profile-calls 20] [--out FILE]
+
+runs the live CNN leg instead: LiveCNN.push(chunk) against LiveStreams.push(chunk, model) on cnn-trad-fpool3 in bf16
+(1 s windows, 10 ms shift), two states fed the same chunk past the warm-up, timed alternately in the same loop of
+repetitions (cnn_ms, streams_model_ms, their spreads and ratio).  With --kernel-only it reports instead, from
+torch.profiler in a loop of --profile-calls calls per path, the summed kernel time per push of each path
+(cnn_kernel_ms, streams_model_kernel_ms); run it as a separate invocation so that tracing does not slow the timed
+loops.
 """
 import argparse
 import json
@@ -46,7 +56,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 import honk2_b200  # noqa: E402
-from honk2_b200 import AudioProcessor, LiveStreams  # noqa: E402
+from honk2_b200 import AudioProcessor, LiveCNN, LiveStreams  # noqa: E402
 from honk2_b200.streaming import ragged_push_plan  # noqa: E402
 
 W, H = 16000, 160
@@ -227,6 +237,62 @@ def ragged_leg(args, dev, ap, models):
     return lines
 
 
+def cnn_leg(args, dev, ap):
+    """The --cnn leg (see the module doc); returns its JSON lines."""
+    lines = []
+    gen = torch.Generator(device=dev).manual_seed(0)
+    m = honk2_b200.build_model("cnn-trad-fpool3", precision="bf16").to(dev)
+    for S in [int(s) for s in args.streams.split(",")]:
+        for push_ms in [int(p) for p in args.push_ms.split(",")]:
+            n = 16 * push_ms
+            K = n // H
+            for dtype in args.dtypes.split(","):
+                x = torch.rand((S, n), generator=gen, device=dev) * 2 - 1
+                chunk = (x * 32767).to(torch.int16) if dtype == "int16" else x
+                lc = LiveCNN(m, S, W, H, max_push=n, audio_processor=ap, device=dev)
+                ls = LiveStreams(ap, S, W, H, max_push=n, device=dev)
+                out_c = torch.empty((S, K, 12), device=dev)
+                feats = torch.empty((S, K, 101, 40), device=dev)
+                fc = lambda: lc.push(chunk, out=out_c)            # noqa: E731
+                fs = lambda: ls.push(chunk, m, out=feats)         # noqa: E731
+                with torch.no_grad():
+                    for _ in range(W // n + 2):                   # past the warm-up: every slot valid
+                        fc()
+                        fs()
+                    row = {"leg": "cnn", "model": "cnn-trad-fpool3", "precision": "bf16", "S": S, "push_ms": push_ms,
+                           "K": K, "dtype": dtype, "windows_per_push": S * K}
+                    if args.kernel_only:
+                        row["cnn_kernel_ms"] = kernel_ms(fc, args.profile_calls)
+                        row["streams_model_kernel_ms"] = kernel_ms(fs, args.profile_calls)
+                    else:
+                        (c_ms, c_sp), (s_ms, s_sp) = timed_pair(fc, fs, args.seconds, args.reps)
+                        row.update({"cnn_ms": c_ms, "cnn_spread": c_sp, "streams_model_ms": s_ms,
+                                    "streams_model_spread": s_sp, "speedup": s_ms / c_ms})
+                print(json.dumps(row), flush=True)
+                lines.append(row)
+                del lc, ls, out_c, feats
+                torch.cuda.empty_cache()
+    return lines
+
+
+def cnn_table(lines):
+    """The --cnn leg's lines as a text table."""
+    rows = [r for r in lines if r.get("leg") == "cnn"]
+    out = ["cnn-trad-fpool3 bf16, ms per push: LiveCNN.push against LiveStreams.push(chunk, model)"]
+    if rows and "cnn_ms" in rows[0]:
+        out.append(f"{'S':>6} {'push':>6} {'dtype':>8} {'LiveCNN':>18} {'LiveStreams+model':>20} {'speedup':>8}")
+        for r in rows:
+            out.append(f"{r['S']:>6} {r['push_ms']:>4}ms {r['dtype']:>8} {r['cnn_ms']:>9.3f} "
+                       f"({100 * r['cnn_spread']:.1f}%) {r['streams_model_ms']:>11.3f} "
+                       f"({100 * r['streams_model_spread']:.1f}%) {r['speedup']:>8.2f}")
+    elif rows:
+        out.append(f"{'S':>6} {'push':>6} {'dtype':>8} {'LiveCNN kernels':>16} {'LiveStreams+model kernels':>26}")
+        for r in rows:
+            out.append(f"{r['S']:>6} {r['push_ms']:>4}ms {r['dtype']:>8} {r['cnn_kernel_ms']:>16.3f} "
+                       f"{r['streams_model_kernel_ms']:>26.3f}")
+    return "\n".join(out)
+
+
 def ragged_table(lines):
     """The --ragged leg's lines as text tables."""
     out = []
@@ -263,6 +329,8 @@ def ragged_table(lines):
 def main():
     ap_ = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     ap_.add_argument("--ragged", action="store_true", help="run the ragged-push leg instead")
+    ap_.add_argument("--cnn", action="store_true", help="run the live CNN leg instead")
+    ap_.add_argument("--kernel-only", action="store_true", help="--cnn: kernel times from torch.profiler only")
     ap_.add_argument("--model-streams", type=int, default=8192, help="streams of the ragged leg's model runs")
     ap_.add_argument("--streams", default=None, help="default 1,148,1024,8192 (--ragged: 148,1024,8192)")
     ap_.add_argument("--push-ms", default="10,100")
@@ -281,6 +349,20 @@ def main():
     print(json.dumps(header), flush=True)
     lines = [header]
     ap = AudioProcessor()
+    if args.cnn:
+        args.streams = args.streams or "148,1024,8192"
+        lines += cnn_leg(args, dev, ap)
+        lines.append({"device": device_line()})
+        print(json.dumps(lines[-1]), flush=True)
+        table = cnn_table(lines)
+        print(table, flush=True)
+        if args.out:
+            with open(args.out, "a") as f:
+                f.write(f"# tools/live_bench.py {' '.join(sys.argv[1:])}\n# device: {header['device']}\n")
+                f.write("\n".join("# " + ln for ln in table.splitlines()) + "\n")
+                for ln in lines:
+                    f.write(json.dumps(ln) + "\n")
+        return
     models = {}
     for name in [m for m in args.models.split(",") if m]:
         models[name] = honk2_b200.build_model(name, precision="bf16").to(dev)
