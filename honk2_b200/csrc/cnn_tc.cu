@@ -617,9 +617,9 @@ int tc_cnn_create(const kws_cnn_config& cfg, TcCnn** out) {
       p->lin_b[i] = reinterpret_cast<float*>(p->blob + o_lb[i]);
       if (i != p->first) p->lin_w[i] = reinterpret_cast<float*>(p->blob + o_lw[i]);
     }
-  e = cudaFuncSetAttribute(cnn_tc_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem_bytes);
+  e = raise_dynamic_smem(cnn_tc_fused_kernel, g.smem_bytes);
   if (e != cudaSuccess) {
-    set_error("tc_cnn_create: cudaFuncSetAttribute(%d) failed: %s", g.smem_bytes, cudaGetErrorString(e));
+    set_error("tc_cnn_create: raising the shared memory limit to %d failed: %s", g.smem_bytes, cudaGetErrorString(e));
     cudaFree(p->blob);
     delete p;
     *out = nullptr;

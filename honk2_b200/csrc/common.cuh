@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstdarg>
+#include <mutex>
 #include <string>
 #include <vector>
 #include "../../include/honk2_b200.h"
@@ -52,6 +53,20 @@ __host__ __device__ constexpr T round_up(T a, T b) { return ceil_div(a, b) * b; 
 constexpr int kNumSMs = 148;  // B200
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// A kernel's dynamic shared memory limit belongs to the kernel, not to the object that launches it.  Objects that plan
+// their own shared memory when they are created (front-ends, CNN plans, live CNN states) only ever raise it: lowering it
+// for a smaller object would make every larger one that already exists fail its launches with "invalid argument".
+template <typename K>
+cudaError_t raise_dynamic_smem(K* kernel, size_t bytes) {
+  static std::mutex mu;
+  std::lock_guard<std::mutex> lock(mu);
+  cudaFuncAttributes a;
+  cudaError_t e = cudaFuncGetAttributes(&a, reinterpret_cast<const void*>(kernel));
+  if (e != cudaSuccess || (size_t)a.maxDynamicSharedSizeBytes >= bytes) return e;
+  return cudaFuncSetAttribute(reinterpret_cast<const void*>(kernel), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              (int)bytes);
+}
 
 // ResNet geometry shared by the fp32 and tensor-core paths: the dilation of C -> C layer i (1-based, resnet.py:21-23),
 // the AvgPool window after conv_0 (pool 0, 0 = absent, resnet.py:40-44), and the map it leaves of a T x F input.

@@ -422,9 +422,9 @@ extern "C" int kws_live_cnn_create(const kws_model_t* m, const kws_frontend_t* f
     lc->smem0 = (size_t)g.ks0 * 2048 + (size_t)kLc0Warps * 3 * 2 * g.ks0 * 256;
     lc->smem1 = (size_t)kLc1Jobs * g.WP * 128 + (size_t)g.KW1 * 8192 + kLc1Jobs * sizeof(void*);
     if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(live_cnn_conv0_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc->smem0);
+      e = raise_dynamic_smem(live_cnn_conv0_kernel, lc->smem0);
     if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(live_cnn_conv1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lc->smem1);
+      e = raise_dynamic_smem(live_cnn_conv1_kernel, lc->smem1);
     if (e != cudaSuccess) {
       set_error("kws_live_cnn_create: %zu bytes of device state: %s", L.total, cudaGetErrorString(e));
       st = KWS_ERR_CUDA;

@@ -688,11 +688,14 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
   KWS_TRY(kws_device_info(&major, &minor, &sms));
 
   const int n_bins = 1 + n_fft / 2;
-  // librosa.filters.mel(htk=False, norm='slaney'), float32 storage like numpy
+  // librosa.filters.mel(htk=False, norm='slaney'), float32 storage like numpy.  The band edges follow np.linspace:
+  // m_lo + i * step, the last one exactly m_hi.  (m_lo + (m_hi - m_lo) * i / (n_mels + 1) can round the last edge above
+  // f_max, which gives the last filter a weight at bin f_max; at f_max = sr/2 that is the Nyquist bin.)
   std::vector<double> mel_f(n_mels + 2);
   const double m_lo = hz_to_mel_slaney(f_min), m_hi = hz_to_mel_slaney(f_max);
-  for (int i = 0; i < n_mels + 2; ++i)
-    mel_f[i] = mel_to_hz_slaney(m_lo + (m_hi - m_lo) * i / (n_mels + 1));
+  const double step = (m_hi - m_lo) / (n_mels + 1);
+  for (int i = 0; i < n_mels + 1; ++i) mel_f[i] = mel_to_hz_slaney(m_lo + i * step);
+  mel_f[n_mels + 1] = mel_to_hz_slaney(m_hi);
   std::vector<int> lo(n_mels), cnt(n_mels), off(n_mels);
   std::vector<float> wts;
   int max_bin = 0;
@@ -767,30 +770,17 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
                    sizeof(float) * (kStageSamples + kNfft) + sizeof(int) * 3 * kMaxMels +
                    sizeof(float) * (nnz + 1);
   fe->smem_bytes_edges = fe->smem_bytes + sizeof(float) * (kEdgeStageSamples - kStageSamples);
-  e = cudaFuncSetAttribute(mfcc_kernel<false, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<false, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<true, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes_edges);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<true, int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fe->smem_bytes_edges);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<false, float, RingSource<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fe->smem_bytes);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<true, float, RingSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fe->smem_bytes_edges);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<true, float, EdgeRingSource>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fe->smem_bytes_edges);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<false, float, RaggedSource<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fe->smem_bytes_edges);
-  if (e == cudaSuccess)
-    e = cudaFuncSetAttribute(mfcc_kernel<true, float, RaggedSource<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)fe->smem_bytes_edges);
+  e = raise_dynamic_smem(mfcc_kernel<false, float>, fe->smem_bytes);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<false, int16_t>, fe->smem_bytes);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, int16_t>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<false, float, RingSource<false>>, fe->smem_bytes);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, RingSource<true>>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, EdgeRingSource>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<false, float, RaggedSource<false>>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, RaggedSource<true>>, fe->smem_bytes_edges);
   if (e != cudaSuccess) {
-    set_error("kws_frontend_create: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
+    set_error("kws_frontend_create: raising the shared memory limit failed: %s", cudaGetErrorString(e));
     cudaFree(fe->dev_blob);
     delete fe;
     return KWS_ERR_CUDA;

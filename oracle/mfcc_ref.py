@@ -120,5 +120,6 @@ def compute_mfccs(y, **kw):
 
 def compute_mfccs_batch(waves, **kw):
     """The collate loop of data_loader/audio_data_loader.py:26-29: per-sample compute_mfccs,
-    reshape(1, -1, 40), concatenate on dim 0 -> float32 [B, T, 40]."""
-    return np.concatenate([compute_mfccs(w, **kw).reshape(1, -1, 40) for w in waves], 0)
+    reshape(1, -1, n_mels), concatenate on dim 0 -> float32 [B, T, n_mels] (n_mels = 40 by default)."""
+    n_mels = kw.get("n_mels", N_MELS)
+    return np.concatenate([compute_mfccs(w, **kw).reshape(1, -1, n_mels) for w in waves], 0)
