@@ -68,6 +68,12 @@ SIGNATURES = {
     "kws_live_cnn_reset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "kws_live_cnn_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "kws_live_cnn_push_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "kws_live_cnn_ragged_workspace_bytes": (C.c_size_t, [C.c_void_p]),
+    "kws_live_cnn_push_ragged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "kws_live_cnn_push_ragged_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                 C.c_void_p]),
     "kws_live_ragged_workspace_bytes": (C.c_size_t, [C.c_void_p]),
     "kws_live_push_ragged": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

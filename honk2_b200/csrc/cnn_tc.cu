@@ -374,7 +374,7 @@ __device__ __forceinline__ void mma_bf16_16816(float (&c)[4], uint32_t a0, uint3
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-// ROWS says where row r's activations are (DenseActRows, LiveActRows: tc.cuh).
+// ROWS says where row r's activations are (DenseActRows, LiveActRows, RaggedActRows: tc.cuh).
 template <typename ROWS>
 __global__ void __launch_bounds__(32 * kLin0Warps)
 cnn_lin0_kernel(const ROWS rows, const __nv_bfloat16* __restrict__ w, float* __restrict__ partial,
@@ -768,8 +768,8 @@ int tc_cnn_copy(const TcCnn* src, TcCnn** out, cudaStream_t st) {
   return KWS_OK;
 }
 
-int tc_cnn_live_linear(const TcCnn* p, const LiveActRows& rows, int64_t B, float* partial, float* logits,
-                       cudaStream_t st) {
+template <typename ROWS>
+static int live_linear(const TcCnn* p, const ROWS& rows, int64_t B, float* partial, float* logits, cudaStream_t st) {
   KWS_REQUIRE(p != nullptr && p->supported, "CNN: no tensor-core path for this configuration");
   const int K = p->g.H1 * 8 * kCnnC;
   const int k_per = round_up(ceil_div(K, kLin0Split), 32);   // the batch path's split-K slices
@@ -788,6 +788,16 @@ int tc_cnn_live_linear(const TcCnn* p, const LiveActRows& rows, int64_t B, float
   cnn_mlp_kernel<<<(unsigned)ceil_div<int64_t>(B, kMlpUtt), 256, 0, st>>>(mp);
   KWS_CHECK_LAUNCH();
   return KWS_OK;
+}
+
+int tc_cnn_live_linear(const TcCnn* p, const LiveActRows& rows, int64_t B, float* partial, float* logits,
+                       cudaStream_t st) {
+  return live_linear(p, rows, B, partial, logits, st);
+}
+
+int tc_cnn_live_linear(const TcCnn* p, const RaggedActRows& rows, int64_t B, float* partial, float* logits,
+                       cudaStream_t st) {
+  return live_linear(p, rows, B, partial, logits, st);
 }
 
 }  // namespace kws

@@ -28,8 +28,17 @@
 // layout.  They keep cnn_tc_fused_kernel's MMA shape (K = 16 per product), K order and rounding points (features and
 // pooled rows to bf16, max + bias + ReLU on the fp32 accumulators), and the first Linear keeps its split-K slices: on
 // the B200 the logits are bit-identical to the batch path's on the materialised windows (tests/test_live_cnn.py).
+//
+// Ragged pushes (kws_live_cnn_push_ragged): stream s goes from count c to c' = c + n_s, any n_s in [0, max_push].  The
+// stream rows of a convolution are a function of the counter alone: with top(c) = floor((c - W) / H) m + Hc - 3 (Hc =
+// H0 or H1, the floor not clamped at 0), a push computes rows (top(c), top(c')], which for aligned counts are the rows
+// the uniform push computes, so the two pushes may be mixed on one state.  During a stream's warm-up a push computes
+// rows although it completes no window; window 0 reads them.  The windows the push completes are compacted as the
+// front-end's ragged push lists them (window i of the push: stream s, window k), and their window-specific rows go to
+// slot i of the edge buffers.  Ring capacity: DESIGN.md section 7, "Ragged pushes".
 #include "live.cuh"
 #include "tc.cuh"
+#include <cub/device/device_scan.cuh>
 #include <algorithm>
 
 namespace kws {
@@ -68,6 +77,7 @@ __device__ __forceinline__ uint32_t lc_pack_relu(float a, float b) {
 // Row jobs of a push, shared by both convolutions: jobs [0, S P) are stream rows (stream j / P, row
 // (k0 - 1) m + H - 2 + j % P); jobs [S P, S P + 4 S K) are window rows (slot w / 4, row 0, 1, H-2, H-1 for w % 4).
 struct LcPush {
+  static constexpr bool kRagged = false;
   const int64_t* count;
   int S, n, window, shift, K, m, P;
   int64_t jobs;
@@ -99,14 +109,68 @@ __device__ __forceinline__ LcJob lc_job(const LcPush& p, int64_t j, int H) {
   }
   return J;
 }
+__device__ __forceinline__ int64_t lc_total(const LcPush& p) { return p.jobs; }
+
+// Row jobs of a ragged push: jobs [0, R) are stream rows, rows (top(c), top(c')] of each stream in stream order
+// (rows[s]: exclusive scan of the per-stream counts, rows[S] = R); jobs [R, R + 4 M) are window rows (window w / 4 of the
+// push's compacted list, row 0, 1, H-2, H-1 for w % 4; wins: the front-end's plan, windows in the low 32 bits, wins[S]
+// = M).  R and M live on the device and the launch covers the host's bounds: CTAs past R + 4 M exit.  conv_0 also writes
+// each window's stream and index and M (each pointer may be null).
+struct LcRagged {
+  static constexpr bool kRagged = true;
+  const int64_t* count;   // this push included
+  const int* len;
+  const int64_t* rows;
+  const int64_t* wins;
+  int S, window, shift, m;
+  int64_t *win_stream, *win_index, *n_windows;
+};
+__device__ __forceinline__ int64_t lc_total(const LcRagged& p) {
+  return __ldg(p.rows + p.S) + 4 * (__ldg(p.wins + p.S) & 0xffffffffll);
+}
+// stream of entry e of a compacted list (plan & mask: exclusive scan of the per-stream counts) and the entries before it
+__device__ __forceinline__ int lc_stream_of(const int64_t* plan, int S, int64_t mask, int64_t e, int64_t* before) {
+  int lo = 0, hi = S;   // (plan[lo] <= e < plan[hi])
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if ((__ldg(plan + mid) & mask) <= e) lo = mid;
+    else hi = mid;
+  }
+  *before = __ldg(plan + lo) & mask;
+  return lo;
+}
+__device__ __forceinline__ LcJob lc_job(const LcRagged& p, int64_t j, int H) {
+  LcJob J;
+  const int64_t R = __ldg(p.rows + p.S);
+  int64_t before;
+  if (j < R) {
+    J.s = lc_stream_of(p.rows, p.S, ~0ll, j, &before);
+    J.stream = true;
+    const int64_t c_old = __ldg(p.count + J.s) - __ldg(p.len + J.s);
+    J.row = lc_floor_div(c_old - p.window, p.shift) * p.m + H - 2 + (j - before);   // top(c) + 1 + ...
+    J.slot = 0; J.e = 0;
+  } else {
+    const int64_t w = j - R;
+    J.slot = w >> 2; J.e = (int)(w & 3);
+    J.s = lc_stream_of(p.wins, p.S, 0xffffffffll, J.slot, &before);
+    J.stream = false;
+    const int64_t c_old = __ldg(p.count + J.s) - __ldg(p.len + J.s);
+    const int64_t k0 = lc_floor_div(c_old - p.window, p.shift) + 1;
+    J.row = (k0 > 0 ? k0 : 0) + (J.slot - before);
+  }
+  return J;
+}
+
 // window row of job J (window job) for kernel row kh, and whether it is one of the window's own rows
 __device__ __forceinline__ int lc_win_row(const LcJob& J, int H) { return J.e < 2 ? J.e : H - 4 + J.e; }
 
 // ---------------------------------------------------------------------------------------------
 // conv_0 + max pool (1, 3) + bias + ReLU.  One warp computes one pooled row: M = 3 pool members x 16 pooled columns
 // (column 3j + e is row j of m-tile e), N = 64, K = ks0 steps of two kernel rows x 8 taps (conv_0's packed weights).
+// JOBS: LcPush (uniform pushes) or LcRagged.
+template <typename JOBS>
 struct Lc0Params {
-  LcPush p;
+  JOBS p;
   const float* frames; int fcap;      // live frame rings [S][fcap][F]
   const float* edges;                 // [S K][4][F]
   const __nv_bfloat16* w0;            // [ks0][2][64][8]
@@ -116,18 +180,30 @@ struct Lc0Params {
   int T, F, KH0, H0, WP, ks0;
 };
 
+template <typename JOBS>
 __global__ void __launch_bounds__(32 * kLc0Warps)
-live_cnn_conv0_kernel(const Lc0Params q) {
+live_cnn_conv0_kernel(const Lc0Params<JOBS> q) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int64_t jobs = lc_total(q.p);
+  if constexpr (JOBS::kRagged) {
+    if (blockIdx.x == 0 && threadIdx.x == 0 && q.p.n_windows) *q.p.n_windows = __ldg(q.p.wins + q.p.S) & 0xffffffffll;
+    if ((int64_t)blockIdx.x * kLc0Warps >= jobs) return;
+  }
   const int kh2 = 2 * q.ks0;
   unsigned char* s_w = smem;                                          // ks0 * 2048 B
   unsigned char* s_a = smem + q.ks0 * 2048 + warp * (3 * kh2 * 256);  // [3][kh2][16 columns][16 B]
   for (int i = threadIdx.x; i < q.ks0 * 128; i += blockDim.x)
     reinterpret_cast<uint4*>(s_w)[i] = reinterpret_cast<const uint4*>(q.w0)[i];
   const int64_t job = (int64_t)blockIdx.x * kLc0Warps + warp;
-  const bool live = job < q.p.jobs;
-  const LcJob J = lc_job(q.p, live ? job : q.p.jobs - 1, q.H0);
+  const bool live = job < jobs;
+  const LcJob J = lc_job(q.p, live ? job : jobs - 1, q.H0);
+  if constexpr (JOBS::kRagged) {
+    if (live && lane == 0 && !J.stream && J.e == 0) {
+      if (q.p.win_stream) q.p.win_stream[J.slot] = J.s;
+      if (q.p.win_index) q.p.win_index[J.slot] = J.row;
+    }
+  }
   const int r = J.stream ? 0 : lc_win_row(J, q.H0);
   const int64_t slot4 = J.slot * 4;
   const float* frames_s = q.frames + (int64_t)J.s * q.fcap * q.F;
@@ -206,8 +282,9 @@ live_cnn_conv0_kernel(const Lc0Params q) {
 // N = 64, K = KH1 x KW1 x 64 in the batch kernel's order ((kh, kw) units outer, 16-channel chunks inner).  Per kernel row
 // kh the CTA stages that input row of its 32 rows (WP x 128 B each, 16-byte chunks XOR-swizzled by position so that
 // ldmatrix's eight rows hit distinct banks) and the KW1 weight units of kh.
+template <typename JOBS>
 struct Lc1Params {
-  LcPush p;
+  JOBS p;
   const __nv_bfloat16* ring0; int cap0;   // [S][cap0][WP][64]
   const __nv_bfloat16* edge0;             // [S K][4][WP][64]
   const __nv_bfloat16* w1;                // [KH1*KW1][4][2][64][8]
@@ -217,7 +294,8 @@ struct Lc1Params {
   int H0, WP, KH1, KW1, H1;
 };
 
-__device__ __forceinline__ const __nv_bfloat16* lc1_in(const Lc1Params& q, const LcJob& J, int kh) {
+template <typename JOBS>
+__device__ __forceinline__ const __nv_bfloat16* lc1_in(const Lc1Params<JOBS>& q, const LcJob& J, int kh) {
   const __nv_bfloat16* ring = q.ring0 + (int64_t)J.s * q.cap0 * q.WP * 64;
   if (J.stream) return ring + (int64_t)lc_mod(J.row + kh, q.cap0) * q.WP * 64;
   const int t = lc_win_row(J, q.H1) + kh;
@@ -226,10 +304,14 @@ __device__ __forceinline__ const __nv_bfloat16* lc1_in(const Lc1Params& q, const
   return ring + (int64_t)lc_mod(J.row * q.p.m + t, q.cap0) * q.WP * 64;
 }
 
+template <typename JOBS>
 __global__ void __launch_bounds__(kLc1Threads)
-live_cnn_conv1_kernel(const Lc1Params q) {
+live_cnn_conv1_kernel(const Lc1Params<JOBS> q) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if constexpr (JOBS::kRagged) {
+    if ((int64_t)blockIdx.x * kLc1Jobs >= lc_total(q.p)) return;
+  }
   const int row_bytes = q.WP * 128;
   unsigned char* s_a = smem;                                   // [32][WP][128 B]
   unsigned char* s_w = smem + kLc1Jobs * row_bytes;            // [KW1][4][2][64][16 B]
@@ -246,7 +328,7 @@ live_cnn_conv1_kernel(const Lc1Params q) {
   const uint32_t a_s = lc_smem(s_a), w_s = lc_smem(s_w);
   const uint32_t b_base = w_s + (uint32_t)((((mi & 1) * 64) + (mi >> 1) * 8 + l8) * 16);
   LcJob mine{};   // threads 0..31: the row this thread stages pointers for
-  if (tid < kLc1Jobs) mine = lc_job(q.p, job0 + tid < q.p.jobs ? job0 + tid : q.p.jobs - 1, q.H1);
+  if (tid < kLc1Jobs) mine = lc_job(q.p, job0 + tid < lc_total(q.p) ? job0 + tid : lc_total(q.p) - 1, q.H1);
   for (int kh = 0; kh < q.KH1; ++kh) {
     __syncthreads();   // the previous kernel row's operands are consumed
     if (tid < kLc1Jobs) s_ptr[tid] = lc1_in(q, mine, kh);
@@ -286,7 +368,7 @@ live_cnn_conv1_kernel(const Lc1Params q) {
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
       const int64_t job = job0 + 4 * warp + 2 * mt + h;
-      if (job >= q.p.jobs) continue;
+      if (job >= lc_total(q.p)) continue;
       const LcJob J = lc_job(q.p, job, q.H1);
       __nv_bfloat16* out = J.stream ? q.ring1 + ((int64_t)J.s * q.cap1 + lc_mod(J.row, q.cap1)) * kLcRow1
                                     : q.edge1 + (J.slot * 4 + J.e) * kLcRow1;
@@ -297,6 +379,19 @@ live_cnn_conv1_kernel(const Lc1Params q) {
         *reinterpret_cast<uint32_t*>(out + (co >> 4) * 128 + gq * 16 + (co & 15)) = lc_pack_relu(vx, vy);
       }
     }
+}
+
+// Ragged pushes: stream s's number of new stream rows of each convolution, m (floor((c' - W) / H) - floor((c - W) / H))
+// (the row rule above), into counts[s]; counts[S] = 0, so that the exclusive scan of counts[0 .. S] ends in the total.
+__global__ void live_cnn_ragged_rows_kernel(const int64_t* __restrict__ count, const int* __restrict__ len, int S,
+                                            int window, int shift, int m, int64_t* __restrict__ counts) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s < S) {
+    const int64_t c = count[s];
+    counts[s] = m * (lc_floor_div(c - window, shift) - lc_floor_div(c - len[s] - window, shift));
+  } else if (s == S) {
+    counts[S] = 0;
+  }
 }
 
 // Warm-up slots (window index < 0) get all-zero logits.
@@ -421,10 +516,10 @@ extern "C" int kws_live_cnn_create(const kws_model_t* m, const kws_frontend_t* f
     const TcCnnGeom& g = lc->v.g;
     lc->smem0 = (size_t)g.ks0 * 2048 + (size_t)kLc0Warps * 3 * 2 * g.ks0 * 256;
     lc->smem1 = (size_t)kLc1Jobs * g.WP * 128 + (size_t)g.KW1 * 8192 + kLc1Jobs * sizeof(void*);
-    if (e == cudaSuccess)
-      e = raise_dynamic_smem(live_cnn_conv0_kernel, lc->smem0);
-    if (e == cudaSuccess)
-      e = raise_dynamic_smem(live_cnn_conv1_kernel, lc->smem1);
+    if (e == cudaSuccess) e = raise_dynamic_smem(live_cnn_conv0_kernel<LcPush>, lc->smem0);
+    if (e == cudaSuccess) e = raise_dynamic_smem(live_cnn_conv1_kernel<LcPush>, lc->smem1);
+    if (e == cudaSuccess) e = raise_dynamic_smem(live_cnn_conv0_kernel<LcRagged>, lc->smem0);
+    if (e == cudaSuccess) e = raise_dynamic_smem(live_cnn_conv1_kernel<LcRagged>, lc->smem1);
     if (e != cudaSuccess) {
       set_error("kws_live_cnn_create: %zu bytes of device state: %s", L.total, cudaGetErrorString(e));
       st = KWS_ERR_CUDA;
@@ -463,11 +558,11 @@ static int live_cnn_push_any(const char* who, kws_live_cnn_t* lc, const SMP* chu
   LcPush p{lc->live->count, lc->S, n, lc->window, lc->shift, K, lc->shift / 160, n / 160, 0};
   p.jobs = (int64_t)lc->S * p.P + 4 * slots;
   KWS_TRY(live_edge_frames(lc->live, n, lc->edges, st));
-  Lc0Params q0{p, lc->live->frames, lc->live->fcap, lc->edges, lc->v.w0, lc->v.b0, lc->ring0, lc->cap0, lc->edge0,
+  Lc0Params<LcPush> q0{p, lc->live->frames, lc->live->fcap, lc->edges, lc->v.w0, lc->v.b0, lc->ring0, lc->cap0, lc->edge0,
                g.T, g.F, g.KH0, g.H0, g.WP, g.ks0};
   live_cnn_conv0_kernel<<<(unsigned)ceil_div<int64_t>(p.jobs, kLc0Warps), 32 * kLc0Warps, lc->smem0, st>>>(q0);
   KWS_CHECK_LAUNCH();
-  Lc1Params q1{p, lc->ring0, lc->cap0, lc->edge0, lc->v.w1, lc->v.b1, lc->ring1, lc->cap1, lc->edge1,
+  Lc1Params<LcPush> q1{p, lc->ring0, lc->cap0, lc->edge0, lc->v.w1, lc->v.b1, lc->ring1, lc->cap1, lc->edge1,
                g.H0, g.WP, g.KH1, g.KW1, g.H1};
   live_cnn_conv1_kernel<<<(unsigned)ceil_div<int64_t>(p.jobs, kLc1Jobs), kLc1Threads, lc->smem1, st>>>(q1);
   KWS_CHECK_LAUNCH();
@@ -484,4 +579,97 @@ extern "C" int kws_live_cnn_push(kws_live_cnn_t* lc, const float* chunk, int n, 
 
 extern "C" int kws_live_cnn_push_pcm16(kws_live_cnn_t* lc, const int16_t* chunk, int n, float* logits, void* stream) {
   return live_cnn_push_any<int16_t>("kws_live_cnn_push_pcm16", lc, chunk, n, logits, stream);
+}
+
+// ---- ragged pushes ----------------------------------------------------------------------------
+// Workspace: the front-end's ragged workspace (offsets, lengths, its plan), then the per-stream stream-row counts
+// i64[S+1], their exclusive scan i64[S+1] and CUB's scan scratch.
+namespace {
+struct LcRaggedLayout {
+  size_t o_rows, o_temp, temp, total;
+};
+
+int lc_ragged_layout(const char* who, const kws_live_cnn* lc, LcRaggedLayout* R) {
+  const size_t plan = round_up<size_t>((size_t)(lc->S + 1) * sizeof(int64_t), 256);
+  R->o_rows = plan;
+  R->o_temp = 2 * plan;
+  R->temp = 0;
+  const cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, R->temp, static_cast<int64_t*>(nullptr),
+                                                      static_cast<int64_t*>(nullptr), lc->S + 1);
+  if (e != cudaSuccess) {
+    set_error("%s: scan size query failed: %s", who, cudaGetErrorString(e));
+    return KWS_ERR_CUDA;
+  }
+  R->total = R->o_temp + R->temp;
+  return KWS_OK;
+}
+}  // namespace
+
+extern "C" size_t kws_live_cnn_ragged_workspace_bytes(const kws_live_cnn_t* lc) {
+  const char* who = "kws_live_cnn_ragged_workspace_bytes";
+  if (lc == nullptr) {
+    set_error("%s: live CNN state is null", who);
+    return 0;
+  }
+  LcRaggedLayout R;
+  if (lc_ragged_layout(who, lc, &R) != KWS_OK) return 0;
+  return live_ragged_workspace_bytes(who, lc->live, R.total);
+}
+
+template <typename SMP>
+static int live_cnn_push_ragged_any(const char* who, kws_live_cnn_t* lc, const SMP* samples, const int32_t* lengths,
+                                    float* logits, int64_t* win_stream, int64_t* win_index, int64_t capacity,
+                                    int64_t* n_windows, void* workspace, size_t ws_bytes, void* stream) {
+  KWS_REQUIRE(lc != nullptr, "%s: live CNN state is null", who);
+  LcRaggedLayout X;
+  KWS_TRY(lc_ragged_layout(who, lc, &X));
+  cudaStream_t st = as_stream(stream);
+  kws_live_t* L = lc->live;
+  // the whole push is checked on the host first; then the samples, the front-end's plan and the new frame-table rows
+  LiveRagged P;
+  KWS_TRY(live_ragged_append_rows(who, L, samples, lengths, capacity, logits, "logits", workspace, ws_bytes, X.total, st,
+                                  &P));
+  unsigned char* x = static_cast<unsigned char*>(P.extra);
+  int64_t* counts = reinterpret_cast<int64_t*>(x);
+  int64_t* rows = reinterpret_cast<int64_t*>(x + X.o_rows);
+  const int m = lc->shift / 160;
+  // the stream-row plan: where each stream's new convolution rows start in the job list, and their total
+  live_cnn_ragged_rows_kernel<<<(unsigned)ceil_div(lc->S + 1, 256), 256, 0, st>>>(L->count, P.len, lc->S, lc->window,
+                                                                                  lc->shift, m, counts);
+  KWS_CHECK_LAUNCH();
+  size_t temp = X.temp;
+  KWS_CUDA(cub::DeviceScan::ExclusiveSum(x + X.o_temp, temp, counts, rows, lc->S + 1, st));
+  // edge frames of the completed windows; conv_0 and conv_1 rows (stream rows even when no window completes: warm-up);
+  // the Linear layers.  Launches are sized by the host's bounds, m + 4 jobs and one window per ceil(n_s / shift).
+  KWS_TRY(live_ragged_edge_frames(L, P, lc->edges, st));
+  const TcCnnGeom& g = lc->v.g;
+  const LcRagged p{L->count, P.len, rows, P.plan, lc->S, lc->window, lc->shift, m, win_stream, win_index, n_windows};
+  const int64_t job_bound = (int64_t)(m + 4) * P.win_bound;
+  Lc0Params<LcRagged> q0{p, L->frames, L->fcap, lc->edges, lc->v.w0, lc->v.b0, lc->ring0, lc->cap0, lc->edge0,
+                         g.T, g.F, g.KH0, g.H0, g.WP, g.ks0};
+  // (one CTA even when nothing is pushed: it writes *n_windows)
+  live_cnn_conv0_kernel<<<(unsigned)std::max<int64_t>(ceil_div<int64_t>(job_bound, kLc0Warps), 1), 32 * kLc0Warps,
+                          lc->smem0, st>>>(q0);
+  KWS_CHECK_LAUNCH();
+  if (P.win_bound == 0) return KWS_OK;
+  Lc1Params<LcRagged> q1{p, lc->ring0, lc->cap0, lc->edge0, lc->v.w1, lc->v.b1, lc->ring1, lc->cap1, lc->edge1,
+                         g.H0, g.WP, g.KH1, g.KW1, g.H1};
+  live_cnn_conv1_kernel<<<(unsigned)ceil_div<int64_t>(job_bound, kLc1Jobs), kLc1Threads, lc->smem1, st>>>(q1);
+  KWS_CHECK_LAUNCH();
+  const RaggedActRows act{lc->ring1, lc->edge1, L->count, P.len, P.plan, lc->S, lc->window, lc->shift, lc->cap1, g.H1};
+  return tc_cnn_live_linear(lc->plan, act, P.win_bound, lc->partial, logits, st);
+}
+
+extern "C" int kws_live_cnn_push_ragged(kws_live_cnn_t* lc, const float* samples, const int32_t* lengths, float* logits,
+                                        int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                        void* workspace, size_t ws_bytes, void* stream) {
+  return live_cnn_push_ragged_any<float>("kws_live_cnn_push_ragged", lc, samples, lengths, logits, win_stream,
+                                         win_index, capacity, n_windows, workspace, ws_bytes, stream);
+}
+
+extern "C" int kws_live_cnn_push_ragged_pcm16(kws_live_cnn_t* lc, const int16_t* samples, const int32_t* lengths,
+                                              float* logits, int64_t* win_stream, int64_t* win_index, int64_t capacity,
+                                              int64_t* n_windows, void* workspace, size_t ws_bytes, void* stream) {
+  return live_cnn_push_ragged_any<int16_t>("kws_live_cnn_push_ragged_pcm16", lc, samples, lengths, logits, win_stream,
+                                           win_index, capacity, n_windows, workspace, ws_bytes, stream);
 }

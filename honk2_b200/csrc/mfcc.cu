@@ -325,6 +325,14 @@ struct RaggedSource {
   }
 };
 
+// RaggedEdgeSource (ragged pushes of kws_live_cnn): RaggedSource<true>'s windows, but only the four edge frames of a
+// window are stored, dense [M][4][n_mels] (frames t = 0, 1, T-2, T-1 in that order).
+struct RaggedEdgeSource : RaggedSource<true> {
+  __device__ __forceinline__ float* out_row(float* feat, int64_t b, int T, int t, int n_mels) const {
+    return feat + (b * 4 + (t < 2 ? t : t - T + 4)) * n_mels;
+  }
+};
+
 template <bool EDGES, typename SMP, typename SRC = DenseSource<SMP>>
 __global__ void __launch_bounds__(kMfccThreads)
 mfcc_kernel(FrontendTables tb, SRC src, int64_t B, int N, int T, int tiles_per_utt, float* __restrict__ feat) {
@@ -779,6 +787,7 @@ extern "C" int kws_frontend_create(int sr, int n_mels, float f_min, float f_max,
   if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, EdgeRingSource>, fe->smem_bytes_edges);
   if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<false, float, RaggedSource<false>>, fe->smem_bytes_edges);
   if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, RaggedSource<true>>, fe->smem_bytes_edges);
+  if (e == cudaSuccess) e = raise_dynamic_smem(mfcc_kernel<true, float, RaggedEdgeSource>, fe->smem_bytes_edges);
   if (e != cudaSuccess) {
     set_error("kws_frontend_create: raising the shared memory limit failed: %s", cudaGetErrorString(e));
     cudaFree(fe->dev_blob);
@@ -1064,39 +1073,46 @@ extern "C" int kws_live_push_pcm16(kws_live_t* live, const int16_t* chunk, int n
 
 // ---- ragged pushes --------------------------------------------------------------------------
 // Workspace: per-stream sample offsets i64[S] and lengths i32[S] (one copy from the pinned staging buffer), the plan
-// counts i64[S+1], their exclusive scan i64[S+1], and CUB's scan scratch.
+// counts i64[S+1], their exclusive scan i64[S+1], and CUB's scan scratch; then, 256-byte aligned, the caller's own part
+// (kws_live_cnn's).
 namespace {
 struct RaggedLayout {
-  size_t o_len, o_counts, o_plan, o_temp, total;
+  size_t o_len, o_counts, o_plan, o_temp, temp, o_extra, total;
 };
 
-int ragged_layout(const char* who, const kws_live* L, RaggedLayout* R) {
+int ragged_layout(const char* who, const kws_live* L, size_t extra, RaggedLayout* R) {
   const size_t S = (size_t)L->S;
   R->o_len = S * sizeof(int64_t);
   R->o_counts = round_up<size_t>(R->o_len + S * sizeof(int32_t), 256);
   R->o_plan = R->o_counts + round_up<size_t>((S + 1) * sizeof(int64_t), 256);
   R->o_temp = R->o_plan + round_up<size_t>((S + 1) * sizeof(int64_t), 256);
-  size_t temp = 0;
-  const cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, temp, static_cast<int64_t*>(nullptr),
+  R->temp = 0;
+  const cudaError_t e = cub::DeviceScan::ExclusiveSum(nullptr, R->temp, static_cast<int64_t*>(nullptr),
                                                       static_cast<int64_t*>(nullptr), L->S + 1);
   if (e != cudaSuccess) {
     set_error("%s: scan size query failed: %s", who, cudaGetErrorString(e));
     return KWS_ERR_CUDA;
   }
-  R->total = R->o_temp + temp;
+  R->o_extra = round_up<size_t>(R->o_temp + R->temp, 256);
+  R->total = extra ? R->o_extra + extra : R->o_temp + R->temp;
   return KWS_OK;
 }
 }  // namespace
 
 extern "C" size_t kws_live_ragged_workspace_bytes(const kws_live_t* live) {
+  return live ? live_ragged_workspace_bytes("kws_live_ragged_workspace_bytes", live, 0) : 0;
+}
+
+namespace kws {
+size_t live_ragged_workspace_bytes(const char* who, const kws_live_t* L, size_t extra) {
   RaggedLayout R;
-  return live && ragged_layout("kws_live_ragged_workspace_bytes", live, &R) == KWS_OK ? R.total : 0;
+  return ragged_layout(who, L, extra, &R) == KWS_OK ? R.total : 0;
 }
 
 template <typename SMP>
-static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* samples, const int32_t* lengths, float* feat,
-                                int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
-                                void* workspace, size_t ws_bytes, void* stream) {
+int live_ragged_append_rows(const char* who, kws_live_t* L, const SMP* samples, const int32_t* lengths,
+                            int64_t capacity, const void* out, const char* out_name, void* workspace, size_t ws_bytes,
+                            size_t ws_extra, cudaStream_t st, LiveRagged* P) {
   KWS_REQUIRE(L != nullptr, "%s: live state is null", who);
   KWS_REQUIRE(lengths != nullptr, "%s: lengths is null", who);
   // the whole plan is checked on the host, before anything is staged or launched
@@ -1114,12 +1130,11 @@ static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* sampl
               "%s: the push can complete up to %lld windows (sum of ceil(length / shift)); capacity is %lld", who,
               (long long)win_bound, (long long)capacity);
   KWS_REQUIRE(n_samples == 0 || samples != nullptr, "%s: samples is null", who);
-  KWS_REQUIRE(win_bound == 0 || feat != nullptr, "%s: feat is null", who);
+  KWS_REQUIRE(win_bound == 0 || out != nullptr, "%s: %s is null", who, out_name);
   RaggedLayout R;
-  KWS_TRY(ragged_layout(who, L, &R));
+  KWS_TRY(ragged_layout(who, L, ws_extra, &R));
   KWS_REQUIRE(workspace != nullptr && ws_bytes >= R.total, "%s: needs %zu bytes of workspace, got %zu", who, R.total,
               workspace ? ws_bytes : (size_t)0);
-  cudaStream_t st = as_stream(stream);
   const size_t stage_bytes = R.o_len + (size_t)L->S * sizeof(int32_t);
   if (!L->ragged_host) {
     KWS_CUDA(cudaMallocHost(&L->ragged_host, stage_bytes));
@@ -1138,6 +1153,7 @@ static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* sampl
   const int* len = reinterpret_cast<const int*>(ws + R.o_len);
   int64_t* counts = reinterpret_cast<int64_t*>(ws + R.o_counts);
   int64_t* plan = reinterpret_cast<int64_t*>(ws + R.o_plan);
+  *P = LiveRagged{len, plan, row_bound, win_bound, ws_extra ? ws + R.o_extra : nullptr};
   KWS_CUDA(cudaMemcpyAsync(ws, L->ragged_host, stage_bytes, cudaMemcpyHostToDevice, st));
   KWS_CUDA(cudaEventRecord(L->ragged_copied, st));
   const kws_frontend* fe = L->fe;
@@ -1146,7 +1162,7 @@ static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* sampl
                                                                  L->shift, L->S, L->count, counts);
   KWS_CHECK_LAUNCH();
   // the plan: where each stream's rows and windows start in the compacted lists, and the totals
-  size_t temp = R.total - R.o_temp;
+  size_t temp = R.temp;
   KWS_CUDA(cub::DeviceScan::ExclusiveSum(ws + R.o_temp, temp, counts, plan, L->S + 1, st));
   // 2) the new frame-table rows, 16 entries of the compacted list per CTA, from any streams
   const RaggedSource<false> rows{L->ring, L->frames, L->count, len, plan, L->S, L->cap, L->fcap, fe->n_mels, L->window,
@@ -1157,6 +1173,37 @@ static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* sampl
         fe->t, rows, row_bound, 0, kFramesPerCta, 1, nullptr);
     KWS_CHECK_LAUNCH();
   }
+  return KWS_OK;
+}
+template int live_ragged_append_rows<float>(const char*, kws_live_t*, const float*, const int32_t*, int64_t,
+                                            const void*, const char*, void*, size_t, size_t, cudaStream_t, LiveRagged*);
+template int live_ragged_append_rows<int16_t>(const char*, kws_live_t*, const int16_t*, const int32_t*, int64_t,
+                                              const void*, const char*, void*, size_t, size_t, cudaStream_t,
+                                              LiveRagged*);
+
+int live_ragged_edge_frames(kws_live_t* L, const LiveRagged& P, float* edges, cudaStream_t st) {
+  if (P.win_bound == 0) return KWS_OK;
+  const RaggedEdgeSource src{{L->ring, L->frames, L->count, P.len, P.plan, L->S, L->cap, L->fcap, L->fe->n_mels,
+                              L->window, L->shift}};
+  mfcc_kernel<true, float, RaggedEdgeSource><<<(unsigned)ceil_div<int64_t>(P.win_bound, 4), kMfccThreads,
+                                               L->fe->smem_bytes_edges, st>>>(L->fe->t, src, P.win_bound, L->window,
+                                                                              L->T, 1, edges);
+  KWS_CHECK_LAUNCH();
+  return KWS_OK;
+}
+}  // namespace kws
+
+template <typename SMP>
+static int live_push_ragged_any(const char* who, kws_live_t* L, const SMP* samples, const int32_t* lengths, float* feat,
+                                int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                void* workspace, size_t ws_bytes, void* stream) {
+  cudaStream_t st = as_stream(stream);
+  LiveRagged P;
+  KWS_TRY(live_ragged_append_rows(who, L, samples, lengths, capacity, feat, "feat", workspace, ws_bytes, 0, st, &P));
+  const kws_frontend* fe = L->fe;
+  const int64_t win_bound = P.win_bound;
+  const int* len = P.len;
+  const int64_t* plan = P.plan;
   // 3) the four reflect-padded edge frames of each completed window, four windows per CTA
   if (win_bound > 0) {
     const RaggedSource<true> edges{L->ring, L->frames, L->count, len, plan, L->S, L->cap, L->fcap, fe->n_mels,

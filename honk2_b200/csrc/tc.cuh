@@ -90,6 +90,35 @@ struct LiveActRows {
   }
 };
 
+// RaggedActRows (ragged pushes of kws_live_cnn): row r is window r of the push's compacted list, the (stream s, window
+// k) of live_ragged_append_rows' plan (low 32 bits of plan[s]: the windows of the streams before s; plan[S]: M), with
+// its window-specific rows at edge[r] and the others in stream s's ring as for LiveActRows.  Rows past the device's M
+// (the launch covers the host's bound) read window min(r, M - 1), or window 0 of the last stream when M = 0: valid
+// memory, results nobody reads.
+struct RaggedActRows {
+  const __nv_bfloat16* ring;
+  const __nv_bfloat16* edge;
+  const int64_t* count;   // samples per stream, this push included
+  const int* len;         // samples per stream of this push
+  const int64_t* plan;
+  int S, window, shift, cap, H1;
+  using Cursor = LiveActRows::Cursor;
+  __device__ __forceinline__ Cursor row(int64_t r, int, int tq) const {
+    const int64_t M = __ldg(plan + S) & 0xffffffffll;
+    r = r < M ? r : (M > 0 ? M - 1 : 0);
+    int lo = 0, hi = S;   // (plan[lo] <= r < plan[hi] in the low words)
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if ((__ldg(plan + mid) & 0xffffffffll) <= r) lo = mid;
+      else hi = mid;
+    }
+    const int64_t d = __ldg(count + lo) - __ldg(len + lo) - window;   // first window = max(0, floor(d / shift) + 1)
+    int64_t k = (d >= 0 ? d / shift : -((-d + shift - 1) / shift)) + 1;
+    k = (k > 0 ? k : 0) + r - (__ldg(plan + lo) & 0xffffffffll);
+    return {ring + lo * (int64_t)cap * 512, edge + r * 2048, k * (shift / 160), cap, H1, tq};
+  }
+};
+
 // What a live CNN state needs of a plan: geometry, packed conv weights (tc_cnn_set_weights' layouts), sizes.
 struct TcCnnView {
   TcCnnGeom g;
@@ -104,6 +133,8 @@ int tc_cnn_copy(const TcCnn* src, TcCnn** out, cudaStream_t st);
 // The first Linear over rows addressed by `rows` (the batch path's split-K slices), then the remaining layers, for B
 // windows.  partial: kTcCnnLin0Split * B * 32 floats; logits [B][n_labels].
 int tc_cnn_live_linear(const TcCnn* p, const LiveActRows& rows, int64_t B, float* partial, float* logits,
+                       cudaStream_t st);
+int tc_cnn_live_linear(const TcCnn* p, const RaggedActRows& rows, int64_t B, float* partial, float* logits,
                        cudaStream_t st);
 // The tensor-core plan of a CNN model handle (model.cu): nullptr for a ResNet; *weights_set: kws_cnn_set_weights ran.
 const TcCnn* model_tc_cnn(const kws_model_t* m, bool* weights_set);

@@ -112,8 +112,9 @@ def ragged_push_plan(seen, lengths, window_size, shift_size):
 
 class _LiveState(object):
     """What the live states share: device selection, the host's copy of the sample counters, the checks of a uniform
-    push's chunk, the validity mask of its slots, reset and pickling.  Subclasses name their C functions
-    (``_create``, ``_reset_fn``, ``_destroy_fn``) and add their own device buffers."""
+    push's chunk and of a ragged push's samples and lengths, the validity mask of a uniform push's slots, reset and
+    pickling.  Subclasses name their C functions (``_create``, ``_reset_fn``, ``_destroy_fn``) and add their own device
+    buffers."""
     _kind = "live state"
 
     def __init__(self, audio_processor, n_streams, window_size, shift_size, max_push, device):
@@ -163,6 +164,30 @@ class _LiveState(object):
         if not pcm16 and chunk.dtype != torch.float32:
             chunk = chunk.float()
         return chunk.contiguous(), pcm16
+
+    def _check_ragged(self, samples, lengths):
+        """A ragged push's arguments as the C call takes them: (contiguous samples, lengths int64 [S], pcm16?)."""
+        name = type(self).__name__
+        if not (isinstance(samples, torch.Tensor) and samples.is_cuda):
+            raise _native.NativeError(f"{name}.push_ragged needs a CUDA tensor: there is no CPU path")
+        if samples.dim() != 1:
+            raise ValueError(f"expected 1-D samples, got shape {tuple(samples.shape)}")
+        if samples.device != self.device:
+            raise ValueError(f"the samples are on {samples.device}, the live state on {self.device}")
+        if samples.dtype not in (torch.float32, torch.int16):
+            raise ValueError(f"samples must be float32 or int16 PCM, got {samples.dtype}")
+        if isinstance(lengths, torch.Tensor) and lengths.is_cuda:
+            raise ValueError("push_ragged takes host lengths: the host checks them and keeps samples_seen")
+        n = np.asarray(lengths).reshape(-1)
+        if n.size != self.n_streams or not np.issubdtype(n.dtype, np.integer):
+            raise ValueError(f"expected {self.n_streams} integer lengths, got {n.size} of {n.dtype}")
+        n = n.astype(np.int64)
+        if ((n < 0) | (n > self.max_push)).any():
+            s = int(np.flatnonzero((n < 0) | (n > self.max_push))[0])
+            raise ValueError(f"stream {s} brings {int(n[s])} samples; a push takes 0 to max_push = {self.max_push}")
+        if int(n.sum()) != samples.numel():
+            raise ValueError(f"the lengths add up to {int(n.sum())} samples, the tensor holds {samples.numel()}")
+        return samples.contiguous(), n, samples.dtype == torch.int16
 
     def _advance(self, n):
         """After a uniform push of n samples: the host-side validity mask [S, K] of its slots; counters advance."""
@@ -300,25 +325,7 @@ class LiveStreams(_LiveState):
         current stream; when M = 0 the samples are still pushed, the model is not called and the tensors are empty.
         ``out``: optional preallocated contiguous float32 features buffer of at least ``sum(ceil(n / shift_size))``
         rows (which bounds M); the features are its first M rows."""
-        if not (isinstance(samples, torch.Tensor) and samples.is_cuda):
-            raise _native.NativeError("LiveStreams.push_ragged needs a CUDA tensor: there is no CPU path")
-        if samples.dim() != 1:
-            raise ValueError(f"expected 1-D samples, got shape {tuple(samples.shape)}")
-        if samples.device != self.device:
-            raise ValueError(f"the samples are on {samples.device}, the live state on {self.device}")
-        if samples.dtype not in (torch.float32, torch.int16):
-            raise ValueError(f"samples must be float32 or int16 PCM, got {samples.dtype}")
-        if isinstance(lengths, torch.Tensor) and lengths.is_cuda:
-            raise ValueError("push_ragged takes host lengths: the host checks them and keeps samples_seen")
-        n = np.asarray(lengths).reshape(-1)
-        if n.size != self.n_streams or not np.issubdtype(n.dtype, np.integer):
-            raise ValueError(f"expected {self.n_streams} integer lengths, got {n.size} of {n.dtype}")
-        n = n.astype(np.int64)
-        if ((n < 0) | (n > self.max_push)).any():
-            s = int(np.flatnonzero((n < 0) | (n > self.max_push))[0])
-            raise ValueError(f"stream {s} brings {int(n[s])} samples; a push takes 0 to max_push = {self.max_push}")
-        if int(n.sum()) != samples.numel():
-            raise ValueError(f"the lengths add up to {int(n.sum())} samples, the tensor holds {samples.numel()}")
+        samples, n, pcm16 = self._check_ragged(samples, lengths)
         plan = ragged_push_plan(self._seen, n, self.window_size, self.shift_size)
         shape = (plan.window_bound, self.n_frames, self.audio_processor.n_mels)
         if out is None:
@@ -333,8 +340,6 @@ class LiveStreams(_LiveState):
             self._ragged_ws = torch.empty(max(1, int(lib.kws_live_ragged_workspace_bytes(handle))), dtype=torch.uint8,
                                           device=self.device)
         lengths32 = np.ascontiguousarray(n, dtype=np.int32)
-        samples = samples.contiguous()
-        pcm16 = samples.dtype == torch.int16
         fn = lib.kws_live_push_ragged_pcm16 if pcm16 else lib.kws_live_push_ragged
         with torch.cuda.device(self.device):
             _native.check(fn(handle, C.c_void_p(samples.data_ptr()), C.c_void_p(lengths32.ctypes.data),
@@ -364,10 +369,16 @@ class LiveCNN(_LiveState):
     those four per window, instead of the whole network per window.  The logits are bit-identical to
     ``LiveStreams.push(chunk, model)`` on the same audio.
 
+    ``push_ragged(samples, lengths)`` lets every stream bring its own number of samples and returns the logits of only
+    the windows the push completes, compacted, as ``LiveStreams.push_ragged(samples, lengths, model)`` does and
+    bit-identical to it; it too computes each convolution row of a stream once.  The two pushes may be mixed on one
+    state while every stream's sample count is a multiple of 160.
+
     ``model`` must be a ``honk2_b200.CNN`` with ``precision == "bf16"`` whose shape has the tensor-core path, and
     ``1 + window_size / 160`` must be its ``time``.  The state copies the model's weights when it is created: later
     changes to the model do not reach it.  ``max_push`` defaults to 10 shifts."""
     _reset_fn, _destroy_fn = "kws_live_cnn_reset", "kws_live_cnn_destroy"
+    _device_buffers = ("_ragged_ws",)
 
     def __init__(self, model, n_streams, window_size=16000, shift_size=160, max_push=None, audio_processor=None,
                  device=None):
@@ -381,6 +392,7 @@ class LiveCNN(_LiveState):
         super().__init__(audio_processor if audio_processor is not None else AudioProcessor(), n_streams, window_size,
                          shift_size, max_push, device)
         self.n_labels = model.n_labels
+        self._ragged_ws = None   # device workspace of push_ragged, allocated by the first ragged push
         self._model = model   # held until the state exists; the state keeps its own copy of the weights
         self._state()
         self._model = None
@@ -428,3 +440,34 @@ class LiveCNN(_LiveState):
                              C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
                           "kws_live_cnn_push_pcm16" if pcm16 else "kws_live_cnn_push")
         return out, self._advance(n)
+
+    def push_ragged(self, samples, lengths, out=None):
+        """Stream s brings ``lengths[s]`` new samples, any number in ``[0, max_push]``; samples and lengths as for
+        ``LiveStreams.push_ragged``.  Returns ``(logits [M, n_labels], stream_ids [M], window_ids [M])`` for the M windows
+        the push completes, ordered by stream, then window; the ids are CPU int64 from the host's copy of the counters
+        (``ragged_push_plan``), so nothing waits for the device.  When M = 0 the push still runs: it computes the
+        convolution rows the streams' next windows read.  ``out``: optional preallocated contiguous float32 logits
+        buffer of at least ``sum(ceil(n / shift_size))`` rows (which bounds M); the logits are its first M rows."""
+        samples, n, pcm16 = self._check_ragged(samples, lengths)
+        plan = ragged_push_plan(self._seen, n, self.window_size, self.shift_size)
+        if out is None:
+            out = torch.empty((plan.window_bound, self.n_labels), dtype=torch.float32, device=self.device)
+        elif out.dim() != 2 or out.shape[0] < plan.window_bound or out.shape[1] != self.n_labels \
+                or out.dtype != torch.float32 or not out.is_contiguous() or out.device != self.device:
+            raise ValueError(f"out must be a contiguous float32 [>= {plan.window_bound}, {self.n_labels}] tensor on "
+                             f"{self.device}")
+        lib = _native.load()
+        handle = self._state()
+        if self._ragged_ws is None:
+            self._ragged_ws = torch.empty(max(1, int(lib.kws_live_cnn_ragged_workspace_bytes(handle))),
+                                          dtype=torch.uint8, device=self.device)
+        lengths32 = np.ascontiguousarray(n, dtype=np.int32)
+        name = "kws_live_cnn_push_ragged_pcm16" if pcm16 else "kws_live_cnn_push_ragged"
+        with torch.cuda.device(self.device):
+            _native.check(getattr(lib, name)(handle, C.c_void_p(samples.data_ptr()), C.c_void_p(lengths32.ctypes.data),
+                                             C.c_void_p(out.data_ptr()), None, None, out.shape[0], None,
+                                             C.c_void_p(self._ragged_ws.data_ptr()), self._ragged_ws.numel(),
+                                             C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), name)
+        self._seen += n
+        M = plan.stream_ids.size
+        return out[:M], torch.from_numpy(plan.stream_ids), torch.from_numpy(plan.window_ids)

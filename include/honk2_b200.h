@@ -159,7 +159,24 @@ int kws_live_push_ragged_pcm16(kws_live_t* live, const int16_t* samples, const i
  *                         (kws_model_forward) on the materialised windows' features.
  *   kws_live_cnn_push_pcm16  the same on int16 PCM: bit-identical to a float push of s/32768.
  *   kws_live_cnn_reset    as kws_live_reset.
- * Push and reset allocate nothing and do not synchronise the host. */
+ * Push and reset allocate nothing and do not synchronise the host.
+ *
+ * Ragged pushes, as kws_live_push_ragged: stream s brings any n_s in [0, max_push] samples, and only the windows the push
+ * completes come back, compacted, ordered by stream, then by window.
+ *   kws_live_cnn_ragged_workspace_bytes  device scratch a ragged push needs (0, with a message, on a null state).
+ *   kws_live_cnn_push_ragged  samples, lengths (HOST int32[S]), win_stream, win_index, capacity, n_windows and the
+ *                         workspace as kws_live_push_ragged; row i of logits [capacity][n_labels] receives the logits of
+ *                         window win_index[i] of stream win_stream[i], i < M = *n_windows; rows past M are unspecified.
+ *                         The logits are bit-identical to the bf16 model on the materialised windows' features, hence to
+ *                         kws_live_cnn_push on the same windows.  Returns KWS_ERR_INVALID, launching nothing, as
+ *                         kws_live_push_ragged does (logits may be null only when every n_s is 0).
+ *   kws_live_cnn_push_ragged_pcm16  the same on int16 PCM: bit-identical to a float ragged push of s/32768.
+ * Row rule: with top(c) = floor((c - window) / shift) * shift / 160 + H - 3 for a convolution of H rows per window (the
+ * floor not clamped at 0), a push from count c to c' computes that stream's convolution rows (top(c), top(c')], even when
+ * it completes no window (window 0 of a fresh stream reads rows computed during its warm-up).  For counts that are
+ * multiples of 160 these are the rows kws_live_cnn_push computes, so the two pushes and reset may be mixed on one state
+ * with the precondition of kws_live_cnn_push: every c_s a multiple of 160 when kws_live_cnn_push is called.  As for the
+ * front-end, a ragged push waits only for the previous ragged push's copy out of the state's pinned staging buffer. */
 typedef struct kws_live_cnn kws_live_cnn_t;
 size_t kws_live_cnn_state_bytes(const kws_model_t* m, const kws_frontend_t* fe, int n_streams, int window, int shift,
                                 int max_push);
@@ -169,6 +186,13 @@ void kws_live_cnn_destroy(kws_live_cnn_t* lc);
 int kws_live_cnn_reset(kws_live_cnn_t* lc, const int64_t* stream_ids, int64_t count, void* stream);
 int kws_live_cnn_push(kws_live_cnn_t* lc, const float* chunk, int n, float* logits, void* stream);
 int kws_live_cnn_push_pcm16(kws_live_cnn_t* lc, const int16_t* chunk, int n, float* logits, void* stream);
+size_t kws_live_cnn_ragged_workspace_bytes(const kws_live_cnn_t* lc);
+int kws_live_cnn_push_ragged(kws_live_cnn_t* lc, const float* samples, const int32_t* lengths, float* logits,
+                             int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                             void* workspace, size_t ws_bytes, void* stream);
+int kws_live_cnn_push_ragged_pcm16(kws_live_cnn_t* lc, const int16_t* samples, const int32_t* lengths, float* logits,
+                                   int64_t* win_stream, int64_t* win_index, int64_t capacity, int64_t* n_windows,
+                                   void* workspace, size_t ws_bytes, void* stream);
 
 /* ---- models: replace model.ResNet / model.CNN ---------------------------------------------
  * kws_resnet_create <- ResNet.__init__ (model/resnet.py:11-36); pool_h = pool_w = 0 when the

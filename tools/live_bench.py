@@ -42,6 +42,17 @@ repetitions (cnn_ms, streams_model_ms, their spreads and ratio).  With --kernel-
 torch.profiler in a loop of --profile-calls calls per path, the summed kernel time per push of each path
 (cnn_kernel_ms, streams_model_kernel_ms); run it as a separate invocation so that tracing does not slow the timed
 loops.
+
+    python tools/live_bench.py --cnn --ragged [--streams 148,1024,8192] [--push-ms 10,100] [--kernel-only]
+                                              [--seconds 2] [--reps 3] [--profile-calls 20] [--out FILE]
+
+runs the live CNN's ragged-push leg: cnn-trad-fpool3 in bf16 (1 s windows, 10 ms shift), float32 samples, states fed
+the same audio past the warm-up and timed alternately in the same loop of repetitions.
+  aligned   every stream brings the push's n samples: LiveCNN.push_ragged (cnn_ragged_ms), LiveStreams.push_ragged(x,
+            lengths, model) (streams_model_ms, the route without LiveCNN's row sharing) and LiveCNN.push (cnn_uniform_ms)
+  jitter    the --ragged leg's jittered lengths (10 ms only), which LiveCNN.push cannot take: cnn_ragged_ms against
+            streams_model_ms, and the windows per push
+With --kernel-only the same rows report the summed kernel time per push of each path (torch.profiler, *_kernel_ms).
 """
 import argparse
 import json
@@ -111,8 +122,13 @@ def kernel_ms(fn, calls):
 
 def timed_pair(fa, fb, seconds, reps):
     """timed() of two calls, their repetitions alternating: (median_a, spread_a), (median_b, spread_b)."""
+    return timed_group((fa, fb), seconds, reps)
+
+
+def timed_group(fns, seconds, reps):
+    """timed() of several calls, their repetitions alternating: ((median, spread) of each)."""
     loops = []
-    for fn in (fa, fb):
+    for fn in fns:
         for _ in range(3):
             fn()
         torch.cuda.synchronize()
@@ -121,9 +137,9 @@ def timed_pair(fa, fb, seconds, reps):
             fn()
         torch.cuda.synchronize()
         loops.append(max(10, int(seconds / max((time.perf_counter() - t) / 10, 1e-6))))
-    ms = ([], [])
+    ms = tuple([] for _ in fns)
     for _ in range(reps):
-        for i, fn in enumerate((fa, fb)):
+        for i, fn in enumerate(fns):
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
             for _ in range(loops[i]):
@@ -168,8 +184,7 @@ def ragged_leg(args, dev, ap, models):
             del uni, rag
             torch.cuda.empty_cache()
         # jittered lengths: a fixed cycle of 64 pushes, the same for every repetition
-        choices = np.array([0, 160, 320, 1024])
-        cycle = [rng.choice(choices, size=S, p=[0.5, 0.3, 0.13, 0.07]).astype(np.int64) for _ in range(64)]
+        cycle = jitter_cycle(S, rng)
         pool = torch.rand(S * max_push, generator=gen, device=dev) * 2 - 1
         x = torch.rand((S, H), generator=gen, device=dev) * 2 - 1
         uni = LiveStreams(ap, S, W, H, max_push, device=dev)
@@ -275,6 +290,117 @@ def cnn_leg(args, dev, ap):
     return lines
 
 
+def jitter_cycle(S, rng):
+    """The --ragged leg's jittered lengths: a fixed cycle of 64 pushes, lengths from {0, 160, 320, 1024}."""
+    choices = np.array([0, 160, 320, 1024])
+    return [rng.choice(choices, size=S, p=[0.5, 0.3, 0.13, 0.07]).astype(np.int64) for _ in range(64)]
+
+
+def cnn_ragged_leg(args, dev, ap):
+    """The --cnn --ragged leg (see the module doc); returns its JSON lines."""
+    lines = []
+    rng = np.random.default_rng(0)
+    gen = torch.Generator(device=dev).manual_seed(0)
+    m = honk2_b200.build_model("cnn-trad-fpool3", precision="bf16").to(dev)
+
+    def measure(row, paths):
+        names = list(paths)
+        if args.kernel_only:
+            for k in names:
+                row[f"{k}_kernel_ms"] = kernel_ms(paths[k], args.profile_calls)
+        else:
+            for k, (ms, sp) in zip(names, timed_group([paths[k] for k in names], args.seconds, args.reps)):
+                row[f"{k}_ms"], row[f"{k}_spread"] = ms, sp
+        print(json.dumps(row), flush=True)
+        lines.append(row)
+
+    with torch.no_grad():
+        for S in [int(s) for s in args.streams.split(",")]:
+            for push_ms in [int(p) for p in args.push_ms.split(",")]:
+                n = 16 * push_ms
+                K = n // H
+                x = torch.rand((S, n), generator=gen, device=dev) * 2 - 1
+                flat = x.reshape(-1)
+                lengths = np.full(S, n, dtype=np.int64)
+                rag = LiveCNN(m, S, W, H, max_push=n, audio_processor=ap, device=dev)
+                uni = LiveCNN(m, S, W, H, max_push=n, audio_processor=ap, device=dev)
+                ls = LiveStreams(ap, S, W, H, max_push=n, device=dev)
+                out_r = torch.empty((S * K, 12), device=dev)
+                out_u = torch.empty((S, K, 12), device=dev)
+                feats = torch.empty((S * K, 101, 40), device=dev)
+                paths = {"cnn_ragged": lambda: rag.push_ragged(flat, lengths, out=out_r),
+                         "streams_model": lambda: ls.push_ragged(flat, lengths, m, out=feats),
+                         "cnn_uniform": lambda: uni.push(x, out=out_u)}
+                for _ in range(W // n + 2):                   # past the warm-up: every stream completes K windows
+                    for f in paths.values():
+                        f()
+                measure({"leg": "cnn_aligned", "model": "cnn-trad-fpool3", "precision": "bf16", "S": S,
+                         "push_ms": push_ms, "dtype": "float32", "windows_per_push": S * K}, paths)
+                del rag, uni, ls, out_r, out_u, feats, paths
+                torch.cuda.empty_cache()
+            if 10 not in [int(p) for p in args.push_ms.split(",")]:
+                continue
+            cycle = jitter_cycle(S, rng)
+            max_push = 1600
+            pool = torch.rand(S * max_push, generator=gen, device=dev) * 2 - 1
+            rag = LiveCNN(m, S, W, H, max_push=max_push, audio_processor=ap, device=dev)
+            ls = LiveStreams(ap, S, W, H, max_push=max_push, device=dev)
+            out_r = torch.empty((S * 7, 12), device=dev)       # >= sum(ceil(n / 160)) for n <= 1024
+            feats = torch.empty((S * 7, 101, 40), device=dev)
+            state = {"r": 0, "s": 0}
+
+            def step(key, fn):
+                def call():
+                    nn = cycle[state[key] % 64]
+                    state[key] += 1
+                    fn(pool[:int(nn.sum())], nn)
+                return call
+            paths = {"cnn_ragged": step("r", lambda v, nn: rag.push_ragged(v, nn, out=out_r)),
+                     "streams_model": step("s", lambda v, nn: ls.push_ragged(v, nn, m, out=feats))}
+            for _ in range(2 * W // 160):
+                for f in paths.values():
+                    f()
+            seen = rag.samples_seen.numpy()
+            wins = []
+            for nn in cycle:
+                wins.append(len(ragged_push_plan(seen, nn, W, H).stream_ids))
+                seen = seen + nn
+            measure({"leg": "cnn_jitter", "model": "cnn-trad-fpool3", "precision": "bf16", "S": S, "dtype": "float32",
+                     "mean_samples": float(np.mean([c.mean() for c in cycle])),
+                     "mean_windows_per_push": float(np.mean(wins))}, paths)
+            del rag, ls, out_r, feats, pool, paths
+            torch.cuda.empty_cache()
+    return lines
+
+
+def cnn_ragged_table(lines):
+    """The --cnn --ragged leg's lines as text tables."""
+    kern = any("cnn_ragged_kernel_ms" in r for r in lines)
+    suf = "_kernel_ms" if kern else "_ms"
+    out = [f"cnn-trad-fpool3 bf16, {'kernel ' if kern else ''}ms per push" + ("" if kern else " (spread)")]
+
+    def cell(r, k):
+        return f"{r[k + suf]:>9.3f}" + ("" if kern else f" ({100 * r[k + '_spread']:4.1f}%)")
+    rows = [r for r in lines if r.get("leg") == "cnn_aligned"]
+    if rows:
+        out.append("aligned pushes: LiveCNN.push_ragged, LiveStreams.push_ragged(x, lengths, model), LiveCNN.push")
+        out.append(f"{'S':>6} {'push':>6} {'cnn_ragged':>18} {'streams+model':>18} {'cnn_uniform':>18} "
+                   f"{'model/ragged':>13} {'ragged/uniform':>15}")
+        for r in rows:
+            out.append(f"{r['S']:>6} {r['push_ms']:>4}ms {cell(r, 'cnn_ragged'):>18} {cell(r, 'streams_model'):>18} "
+                       f"{cell(r, 'cnn_uniform'):>18} {r['streams_model' + suf] / r['cnn_ragged' + suf]:>13.2f} "
+                       f"{r['cnn_ragged' + suf] / r['cnn_uniform' + suf]:>15.2f}")
+    rows = [r for r in lines if r.get("leg") == "cnn_jitter"]
+    if rows:
+        out.append("jittered pushes (lengths from {0, 160, 320, 1024}), which LiveCNN.push cannot take")
+        out.append(f"{'S':>6} {'samples':>8} {'windows':>8} {'cnn_ragged':>18} {'streams+model':>18} {'model/ragged':>13}")
+        for r in rows:
+            out.append(f"{r['S']:>6} {r['mean_samples']:>8.1f} {r['mean_windows_per_push']:>8.1f} "
+                       f"{cell(r, 'cnn_ragged'):>18} {cell(r, 'streams_model'):>18} "
+                       f"{r['streams_model' + suf] / r['cnn_ragged' + suf]:>13.2f}")
+    return "\n".join(out)
+
+
 def cnn_table(lines):
     """The --cnn leg's lines as a text table."""
     rows = [r for r in lines if r.get("leg") == "cnn"]
@@ -349,6 +475,20 @@ def main():
     print(json.dumps(header), flush=True)
     lines = [header]
     ap = AudioProcessor()
+    if args.cnn and args.ragged:
+        args.streams = args.streams or "148,1024,8192"
+        lines += cnn_ragged_leg(args, dev, ap)
+        lines.append({"device": device_line()})
+        print(json.dumps(lines[-1]), flush=True)
+        table = cnn_ragged_table(lines)
+        print(table, flush=True)
+        if args.out:
+            with open(args.out, "a") as f:
+                f.write(f"# tools/live_bench.py {' '.join(sys.argv[1:])}\n# device: {header['device']}\n")
+                f.write("\n".join("# " + ln for ln in table.splitlines()) + "\n")
+                for ln in lines:
+                    f.write(json.dumps(ln) + "\n")
+        return
     if args.cnn:
         args.streams = args.streams or "148,1024,8192"
         lines += cnn_leg(args, dev, ap)
